@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the dense-factorisation hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], the one the metric is quoted on): batched Householder
 QR of 2^20 independent 32 x 32 float64 matrices per GPU; one "step" = one pass over that batch.
@@ -15,6 +15,10 @@ e2e     = the same metric through the host-pointer C-ABI call lq_householder_qr_
 roofline, cpu_baseline, clocks, gpu_launches: see DESIGN.md "Measurement".
 extras  = the other BASELINE configs (MGS, least squares, blocked 8192^2, tall-skinny TSQR / SVD)
           measured the same way, each with its own roofline fraction.
+
+--dump-outputs DIR writes Q and R of the last timed step for a fixed, seeded sample of DUMP_MATRICES matrices
+(rank 0's batch) as DIR/Q.npy and DIR/R.npy, float64.  The inputs depend on the arguments only, so two builds
+of the project can be compared output for output.
 
 --impl reference times the reference's CPU algorithm (the NumPy oracle port -- the reference is
 pure Python and cannot travel to the GPU box) on all host cores, on a bounded sample of the same
@@ -43,7 +47,7 @@ FLOPS_HH32 = 87381                               # F_QR(32, 32)
 FLOPS_MGS32 = 65536
 PER_GPU_BATCH = 1 << 20
 UNIQUE = 1 << 16                                 # distinct random matrices, tiled to the full batch
-
+DUMP_MATRICES = 2048                             # --dump-outputs sample: 2 x 2048 x 8 KiB = 32 MiB
 
 
 def _json_default(o):
@@ -263,6 +267,20 @@ def tile_to_device(ctx, block: np.ndarray, reps: int):
     return buf
 
 
+def dump_outputs(ctx, out_dir, dQ, dR, batch):
+    """Q and R of DUMP_MATRICES matrices of the batch, drawn with a fixed seed across all of it (the tiled replicas
+    included), -> out_dir/Q.npy, out_dir/R.npy as (count, 32, 32) float64 in ascending batch order."""
+    idx = np.sort(np.random.default_rng(0).choice(batch, size=min(DUMP_MATRICES, batch), replace=False))
+    per = 8 * N32 * N32
+    os.makedirs(out_dir, exist_ok=True)
+    for name, buf in (("Q", dQ), ("R", dR)):
+        out = np.empty((len(idx), N32, N32))
+        for k, i in enumerate(idx):
+            ctx.call("lq_memcpy_d2h", out[k].ctypes.data, buf.ptr + int(i) * per, per)
+        ctx.sync()
+        np.save(os.path.join(out_dir, f"{name}.npy"), out)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -273,7 +291,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--e2e-steps", type=int, default=0, help="end-to-end steps (default min(steps, 5))")
     ap.add_argument("--batch", type=int, default=PER_GPU_BATCH, help="matrices per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write Q and R of the last timed step (a fixed sample of the batch) as DIR/Q.npy, DIR/R.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -345,6 +367,8 @@ def main():
     resid = float(np.max(np.linalg.norm(block[:nchk] - Qh @ Rh, axis=(1, 2)) / np.linalg.norm(block[:nchk], axis=(1, 2))))
     if not resid < 1e-12:
         raise SystemExit(f"bench: factorisation check failed (residual {resid})")
+    if args.dump_outputs and info.rank == 0:
+        dump_outputs(ctx, args.dump_outputs, dQ, dR, batch)   # before the MGS leg below overwrites dQ, dR
 
     extras = {"hh32_residual_check": resid}
 

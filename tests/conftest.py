@@ -18,8 +18,16 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
+    """Reference outputs from the fixture file plus the seeded inputs they were computed from, regenerated."""
+    from golden.make_golden import golden_inputs, inputs_sha1
+
     z = np.load(GOLDEN)
-    return {k: z[k] for k in z.files}
+    out = {k: z[k] for k in z.files}
+    inputs = golden_inputs()
+    if not np.array_equal(inputs_sha1(inputs), out.pop("inputs_sha1")):
+        raise RuntimeError("the seeded golden inputs no longer regenerate bit for bit (NumPy random stream changed?)")
+    out.update(inputs)
+    return out
 
 
 def golden_cases(prefix):

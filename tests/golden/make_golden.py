@@ -1,10 +1,7 @@
 #!/usr/bin/env python3
 """Generate tests/golden/hotpath_golden.npz by running the REAL reference.
 
-Run in the build container only (the reference tree does not travel to the GPU
-box):
-
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py [/root/reference]
+    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py <reference checkout>
 
 The reference (BrantleighBunting/linalg) ships no known-answer vectors for
 qr / householder_qr / least_squares_* / svd (SURVEY.md section 8c), so the
@@ -12,35 +9,21 @@ fixtures are outputs of the unmodified reference functions on seeded float64
 inputs.  Inputs replay the reference's own seeded test cases where it has them
 (tests/test_svd.py:13-16, 38-42, 60-70; tests/test_qr.py:29) plus the
 BASELINE.json shape classes at fixture-friendly sizes.
+
+To keep the file small, the seeded inputs are not stored: ``golden_inputs()``
+regenerates them bit for bit (tests/conftest.py checks them against the SHA-1
+stored under ``inputs_sha1``).  Only inputs drawn by the reference's own
+generator (``random_nonsingular_upper``) are stored with the outputs.
 """
+import hashlib
 import os
 import sys
 
 import numpy as np
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
-sys.path.insert(0, REF)
-sys.dont_write_bytecode = True
+PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "hotpath_golden.npz")
 
-from linalg.qr import (  # noqa: E402
-    householder_qr,
-    least_squares_householder_qr,
-    least_squares_qr,
-    qr,
-)
-from linalg.svd import svd  # noqa: E402
-from linalg.utils import random_nonsingular_upper  # noqa: E402
-
-out = {}
-
-
-def put(name, **arrays):
-    for k, v in arrays.items():
-        out[f"{name}/{k}"] = np.ascontiguousarray(np.asarray(v, dtype=np.float64))
-
-
-# ---- Householder / MGS QR ------------------------------------------------
-qr_cases = {
+QR_CASES = {
     "sq32": (32, 32, 2),
     "sq5": (5, 5, 11),
     "tall8x5": (8, 5, 13),
@@ -53,92 +36,131 @@ qr_cases = {
     "one1x1": (1, 1, 24),
     "col7x1": (7, 1, 25),
 }
-for name, (m, n, seed) in qr_cases.items():
-    A = np.random.default_rng(seed).standard_normal((m, n))
-    Q, R = householder_qr(A)
-    put(f"hh/{name}", A=A, Q=Q, R=R)
-    Q, R = qr(A)
-    put(f"mgs/{name}", A=A, Q=Q, R=R)
-    Q, R = qr(A, reorth=True)
-    put(f"mgs_reorth/{name}", A=A, Q=Q, R=R)
+BATCHED32 = 12  # matrices of the cfg2 shape class (the first 12 of a seed-2 draw of 24)
 
-# Householder edge cases: a zero column (skip branch, qr.py:79-80), negative
-# pivots, an already upper-triangular matrix, integer dtype input.
-A = np.random.default_rng(31).standard_normal((12, 6))
-A[:, 2] = 0.0
-Q, R = householder_qr(A)
-put("hh/zero_col", A=A, Q=Q, R=R)
-A = np.random.default_rng(32).standard_normal((9, 9))
-A[3:, 3] = 0.0  # remaining part of column 3 is exactly zero at step 3? (not after updates) -- generic case
-Q, R = householder_qr(A)
-put("hh/partial_zero", A=A, Q=Q, R=R)
-A = np.triu(np.random.default_rng(33).uniform(-5, 5, (10, 10)))
-Q, R = householder_qr(A)
-put("hh/upper_tri", A=A, Q=Q, R=R)
-A = np.zeros((6, 4))
-Q, R = householder_qr(A)
-put("hh/all_zero", A=A, Q=Q, R=R)
-A = np.random.default_rng(34).integers(-9, 10, (16, 8)).astype(np.float64)
-Q, R = householder_qr(A)
-put("hh/integers", A=A, Q=Q, R=R)
 
-# batched 32x32 (cfg2 shape class): 24 matrices, seed 2 stream
-A = np.random.default_rng(2).standard_normal((24, 32, 32))
-put(
-    "batched32",
-    A=A,
-    Q_hh=np.stack([np.ascontiguousarray(householder_qr(a)[0]) for a in A]),
-    R_hh=np.stack([householder_qr(a)[1] for a in A]),
-    Q_mgs=np.stack([qr(a)[0] for a in A]),
-    R_mgs=np.stack([qr(a)[1] for a in A]),
-)
+def golden_inputs():
+    """Every seeded input of the fixtures, keyed like the fixture file (``<case>/A``, ``<case>/B``, ``<case>/b``)."""
+    inp = {}
 
-# ---- least squares -----------------------------------------------------------
-for i in range(3):  # tests/test_qr.py:23-47 style, seeded
-    U = random_nonsingular_upper(50, seed=100 + i)
-    x_true = np.random.default_rng(200 + i).random(50)
-    b = U @ x_true
-    put(f"ls/upper50_{i}", A=U, b=b, x_hh=least_squares_householder_qr(U, b), x_mgs=least_squares_qr(U, b))
-A = np.random.default_rng(3).standard_normal((2, 256, 64))
-B = np.random.default_rng(4).standard_normal((2, 256, 16))
-put(
-    "ls/cfg3",
-    A=A,
-    B=B,
-    X_hh=np.stack([least_squares_householder_qr(A[i], B[i]) for i in range(2)]),
-    X_mgs=np.stack([least_squares_qr(A[i], B[i]) for i in range(2)]),
-)
-A = np.random.default_rng(5).standard_normal((40, 12))
-b = np.random.default_rng(6).standard_normal(40)
-put("ls/vec40x12", A=A, b=b, x_hh=least_squares_householder_qr(A, b), x_mgs=least_squares_qr(A, b))
-B2 = np.random.default_rng(7).standard_normal((40, 3))
-put("ls/mat40x12x3", A=A, b=B2, x_hh=least_squares_householder_qr(A, B2), x_mgs=least_squares_qr(A, B2))
+    # ---- Householder / MGS QR: the three routines see the same matrices
+    for name, (m, n, seed) in QR_CASES.items():
+        A = np.random.default_rng(seed).standard_normal((m, n))
+        for fam in ("hh", "mgs", "mgs_reorth"):
+            inp[f"{fam}/{name}/A"] = A
+    # Householder edge cases: a zero column (skip branch, qr.py:79-80), negative
+    # pivots, an already upper-triangular matrix, integer dtype input.
+    A = np.random.default_rng(31).standard_normal((12, 6))
+    A[:, 2] = 0.0
+    inp["hh/zero_col/A"] = A
+    A = np.random.default_rng(32).standard_normal((9, 9))
+    A[3:, 3] = 0.0
+    inp["hh/partial_zero/A"] = A
+    inp["hh/upper_tri/A"] = np.triu(np.random.default_rng(33).uniform(-5, 5, (10, 10)))
+    inp["hh/all_zero/A"] = np.zeros((6, 4))
+    inp["hh/integers/A"] = np.random.default_rng(34).integers(-9, 10, (16, 8)).astype(np.float64)
+    # batched 32x32 (cfg2 shape class), seed 2 stream
+    inp["batched32/A"] = np.random.default_rng(2).standard_normal((24, 32, 32))[:BATCHED32]
 
-# ---- svd -----------------------------------------------------------------------
-for m, n in [(8, 5), (20, 20), (50, 10)]:  # tests/test_svd.py:13-16
-    A = np.random.default_rng(seed=m + n).normal(size=(m, n))
-    U, s, Vt = svd(A)
-    put(f"svd/recon_{m}x{n}", A=A, U=U, s=s, Vt=Vt)
-for m, n in [(12, 7), (30, 15)]:  # tests/test_svd.py:38-42
-    A = np.random.default_rng(seed=4 * m + n).standard_normal(size=(m, n))
-    U, s, Vt = svd(A)
-    put(f"svd/np_{m}x{n}", A=A, U=U, s=s, Vt=Vt)
-for k in (0, 1, 3):  # tests/test_svd.py:60-70 (U's completion columns are random upstream)
-    A = np.random.default_rng(123 + k).normal(size=(10, 7))
-    if k:
-        A[:, -k:] = 0.0
-    np.random.seed(999)
-    U, s, Vt = svd(A)
-    put(f"svd/rankdef_{k}", A=A, U=U, s=s, Vt=Vt)
-A = np.random.default_rng(50).standard_normal((5, 9))  # wide -> transpose branch svd.py:37-39
-U, s, Vt = svd(A)
-put("svd/wide_5x9", A=A, U=U, s=s, Vt=Vt)
-A = np.random.default_rng(51).standard_normal((1024, 128))  # cfg5 shape class, reduced rows
-U, s, Vt = svd(A)
-put("svd/tall_1024x128", A=A, s=s, Vt=Vt)  # U omitted; checked through invariants
-Q, R = qr(A[:1024, :64])
-put("tsqr/mgs_1024x64", A=A[:1024, :64], R=R)
+    # ---- least squares (ls/upper50_* come from the reference's generator and are stored)
+    inp["ls/cfg3/A"] = np.random.default_rng(3).standard_normal((2, 256, 64))
+    inp["ls/cfg3/B"] = np.random.default_rng(4).standard_normal((2, 256, 16))
+    A = np.random.default_rng(5).standard_normal((40, 12))
+    inp["ls/vec40x12/A"] = inp["ls/mat40x12x3/A"] = A
+    inp["ls/vec40x12/b"] = np.random.default_rng(6).standard_normal(40)
+    inp["ls/mat40x12x3/b"] = np.random.default_rng(7).standard_normal((40, 3))
 
-path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "hotpath_golden.npz")
-np.savez_compressed(path, **out)
-print(f"wrote {path}: {len(out)} arrays, {os.path.getsize(path)/1e6:.2f} MB")
+    # ---- svd
+    for m, n in [(8, 5), (20, 20), (50, 10)]:  # tests/test_svd.py:13-16
+        inp[f"svd/recon_{m}x{n}/A"] = np.random.default_rng(seed=m + n).normal(size=(m, n))
+    for m, n in [(12, 7), (30, 15)]:  # tests/test_svd.py:38-42
+        inp[f"svd/np_{m}x{n}/A"] = np.random.default_rng(seed=4 * m + n).standard_normal(size=(m, n))
+    for k in (0, 1, 3):  # tests/test_svd.py:60-70 (U's completion columns are random upstream)
+        A = np.random.default_rng(123 + k).normal(size=(10, 7))
+        if k:
+            A[:, -k:] = 0.0
+        inp[f"svd/rankdef_{k}/A"] = A
+    inp["svd/wide_5x9/A"] = np.random.default_rng(50).standard_normal((5, 9))  # wide -> transpose branch svd.py:37-39
+    A = np.random.default_rng(51).standard_normal((1024, 128))  # cfg5 shape class, reduced rows
+    inp["svd/tall_1024x128/A"] = A
+    inp["tsqr/mgs_1024x64/A"] = A[:1024, :64]
+    return {k: np.array(v, dtype=np.float64, order="C") for k, v in inp.items()}  # one private copy per key
+
+
+def inputs_sha1(inputs):
+    """SHA-1 over the names, shapes and bytes of ``inputs`` (as uint8, so it can live in the .npz)."""
+    h = hashlib.sha1()
+    for k in sorted(inputs):
+        v = np.ascontiguousarray(inputs[k], dtype=np.float64)
+        h.update(k.encode() + repr(v.shape).encode() + v.tobytes())
+    return np.frombuffer(h.digest(), dtype=np.uint8)
+
+
+def main(ref):
+    sys.path.insert(0, ref)
+    sys.dont_write_bytecode = True
+    from linalg.qr import householder_qr, least_squares_householder_qr, least_squares_qr, qr
+    from linalg.svd import svd
+    from linalg.utils import random_nonsingular_upper
+
+    inp = golden_inputs()
+    out = {}
+
+    def put(name, **arrays):
+        for k, v in arrays.items():
+            out[f"{name}/{k}"] = np.ascontiguousarray(np.asarray(v, dtype=np.float64))
+
+    for name in QR_CASES:
+        A = inp[f"hh/{name}/A"]
+        Q, R = householder_qr(A)
+        put(f"hh/{name}", Q=Q, R=R)
+        Q, R = qr(A)
+        put(f"mgs/{name}", Q=Q, R=R)
+        Q, R = qr(A, reorth=True)
+        put(f"mgs_reorth/{name}", Q=Q, R=R)
+    for name in ("zero_col", "partial_zero", "upper_tri", "all_zero", "integers"):
+        Q, R = householder_qr(inp[f"hh/{name}/A"])
+        put(f"hh/{name}", Q=Q, R=R)
+    A = inp["batched32/A"]
+    put(
+        "batched32",
+        Q_hh=np.stack([np.ascontiguousarray(householder_qr(a)[0]) for a in A]),
+        R_hh=np.stack([householder_qr(a)[1] for a in A]),
+        Q_mgs=np.stack([qr(a)[0] for a in A]),
+        R_mgs=np.stack([qr(a)[1] for a in A]),
+    )
+
+    for i in range(3):  # tests/test_qr.py:23-47 style, seeded
+        U = random_nonsingular_upper(50, seed=100 + i)
+        x_true = np.random.default_rng(200 + i).random(50)
+        b = U @ x_true
+        put(f"ls/upper50_{i}", A=U, b=b, x_hh=least_squares_householder_qr(U, b), x_mgs=least_squares_qr(U, b))
+    A, B = inp["ls/cfg3/A"], inp["ls/cfg3/B"]
+    put(
+        "ls/cfg3",
+        X_hh=np.stack([least_squares_householder_qr(A[i], B[i]) for i in range(2)]),
+        X_mgs=np.stack([least_squares_qr(A[i], B[i]) for i in range(2)]),
+    )
+    for name in ("vec40x12", "mat40x12x3"):
+        A, b = inp[f"ls/{name}/A"], inp[f"ls/{name}/b"]
+        put(f"ls/{name}", x_hh=least_squares_householder_qr(A, b), x_mgs=least_squares_qr(A, b))
+
+    for name in ("recon_8x5", "recon_20x20", "recon_50x10", "np_12x7", "np_30x15",
+                 "rankdef_0", "rankdef_1", "rankdef_3", "wide_5x9"):
+        np.random.seed(999)  # the rank-deficient completion draws from the global state
+        U, s, Vt = svd(inp[f"svd/{name}/A"])
+        put(f"svd/{name}", U=U, s=s, Vt=Vt)
+    _, s, Vt = svd(inp["svd/tall_1024x128/A"])
+    put("svd/tall_1024x128", s=s, Vt=Vt)  # U omitted; checked through invariants
+    _, R = qr(inp["tsqr/mgs_1024x64/A"])
+    put("tsqr/mgs_1024x64", R=R)
+
+    out["inputs_sha1"] = inputs_sha1(inp)
+    np.savez_compressed(PATH, **out)
+    print(f"wrote {PATH}: {len(out)} arrays, {os.path.getsize(PATH)/1e6:.2f} MB")
+
+
+if __name__ == "__main__":
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

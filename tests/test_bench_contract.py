@@ -46,3 +46,31 @@ def test_own_arm_needs_a_gpu():
     assert out.returncode != 0
     assert out.stdout.strip() == ""          # no JSON line from a machine without the device
     assert "no CPU fallback" in out.stderr
+
+
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and out.stdout.strip() == "" and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_steps_factors(tmp_path):
+    """--dump-outputs writes Q and R of the timed path for a seeded sample of the batch; they factor the seeded inputs."""
+    import numpy as np
+
+    batch = 4096
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--batch", str(batch),
+                          "--no-extras", "--no-cpu", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout)
+    assert line["steps"] == 2 and line["gpu_launches"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["Q.npy", "R.npy"]
+    Q, R = np.load(tmp_path / "Q.npy"), np.load(tmp_path / "R.npy")
+    assert Q.dtype == R.dtype == np.float64 and Q.shape == R.shape == (2048, 32, 32)
+    assert Q.nbytes + R.nbytes <= 64 << 20
+    idx = np.sort(np.random.default_rng(0).choice(batch, size=2048, replace=False))
+    A = np.random.default_rng(2).standard_normal((batch, 32, 32))[idx]
+    assert np.max(np.linalg.norm(A - Q @ R, axis=(1, 2)) / np.linalg.norm(A, axis=(1, 2))) <= 1e-12
+    assert np.all(np.tril(R, -1) == 0.0)
