@@ -64,7 +64,8 @@ int lq_set_option(lq_ctx* ctx, const char* name, int value);
 
 /* ---- a1: householder_qr  (linalg/qr.py:52-100) ------------------------------------------- */
 /* A (batch, m, n) -> Q (batch, m, n), R (batch, n, n); requires m >= n >= 1.
- * variant: 0 = library default; other values select a specific kernel (bench/tests). */
+ * variant: must be 0 (the library's kernel for each shape); any other value returns LQ_ERR_ARG.  The argument is kept
+ * for ABI compatibility. */
 int lq_householder_qr_batched_dev(lq_ctx* ctx, const double* A, int64_t batch, int m, int n, double* Q, double* R,
                                   int variant);
 int lq_householder_qr_batched(lq_ctx* ctx, const double* A, int64_t batch, int m, int n, double* Q, double* R);

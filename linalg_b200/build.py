@@ -25,10 +25,6 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC,-O2",
     "--expt-relaxed-constexpr",
 ]
-# the hh32 design-space variants measured in profiles/ (tools/sweep_hh32.py) are compiled only on request: the default
-# library ships the kernels the entry points and the tests use (1/4 of the code size and build time)
-if os.environ.get("LINALG_B200_ALL_VARIANTS"):
-    NVCC_FLAGS.append("-DLQ_ALL_VARIANTS")
 
 
 def _nvcc() -> str:

@@ -3,214 +3,26 @@
 
 #include "../../include/linalg_b200.h"
 #include "batched_qr32.cuh"
-#include "batched_qr32_pipe.cuh"
-#include "batched_qr32_dmma.cuh"
-#include "batched_qr32_ll.cuh"
 #include "batched_qr32_c8.cuh"
-#include "batched_mgs32_c8.cuh"
 #include "batched_small.cuh"
 #include "ctx.cuh"
 #include "ops.cuh"
 
 namespace lq {
 
-// ------------------------------------------------------------------ 32x32 fast kernels
-template <int P, int C, int WARPS, bool KEEPV, int MINB, int NR = 3>
-static int launch_hh32(Ctx* c, cudaStream_t st, const double* A, long long batch, double* Q, double* R) {
-    using D = Dist32<P, C>;
-    auto kern = hh_qr32_kernel<P, C, WARPS, KEEPV, MINB, NR>;
-    const size_t smem = (size_t)WARPS * D::MPW * D::SMEM_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long per_block = (long long)WARPS * D::MPW;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, batch);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// software-pipelined kernel (R phase of pair n+1 interleaved with the Q phase of pair n), persistent grid
-template <int WARPS, int MINB, int NR>
-static int launch_hh32_pipe(Ctx* c, cudaStream_t st, const double* A, long long batch, double* Q, double* R) {
-    auto kern = hh_qr32_pipe_kernel<WARPS, MINB, NR>;
-    const size_t smem = (size_t)WARPS * Pipe32::WARP_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long pairs = (batch + 1) / 2;
-    const long long blocks = std::min<long long>((long long)c->sm_count * MINB, (pairs + WARPS - 1) / WARPS);
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, batch);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// R phase on DFMA, Q formation as compact-WY block reflectors on the FP64 tensor pipe (DMMA.8x8x4)
-template <int WARPS, int MINB, int PHASES = 3>
-static int launch_hh32_dmma(Ctx* c, cudaStream_t st, const double* A, long long batch, double* Q, double* R) {
-    auto kern = hh_qr32_dmma_kernel<WARPS, MINB, PHASES>;
-    const size_t smem = (size_t)WARPS * Dmma32::warp_doubles() * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long per_block = (long long)WARPS * 2;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, batch);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// register-light left-looking R phase (NS column stages, packed reflectors) + DMMA Q phase
-template <int NS, int WARPS, int MINB, int PHASES = 3, bool KEEPV = false>
-static int launch_hh32_ll(Ctx* c, cudaStream_t st, const double* A, long long batch, double* Q, double* R) {
-    auto kern = hh_qr32_ll_kernel<NS, WARPS, MINB, PHASES, KEEPV>;
-    const size_t smem = (size_t)WARPS * Pack32::WARP_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long per_block = (long long)WARPS * 2;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, batch);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// lane = column, four matrices per warp, left-looking panels + DMMA Q phase
-template <int WARPS, int MINB, int PHASES = 3, bool KEEPV = false, bool PF = false, bool PF2 = false, typename LAY = Col8>
-static int launch_hh32_c8(Ctx* c, cudaStream_t st, const double* A, long long batch, double* Q, double* R) {
-    auto kern = hh_qr32_c8_kernel<WARPS, MINB, PHASES, KEEPV, PF, PF2, LAY>;
-    const size_t smem = (size_t)WARPS * LAY::WARP_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long per_block = (long long)WARPS * 4;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, batch);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-template <int P, int C, int WARPS, int MINB>
-static int launch_mgs32(Ctx* c, cudaStream_t st, const double* A, long long batch, int reorth, double* Q, double* R,
-                        int* info) {
-    using D = Dist32<P, C>;
-    auto kern = mgs_qr32_kernel<P, C, WARPS, MINB>;
-    const size_t smem = (size_t)WARPS * D::MPW * D::MGS_DOUBLES * sizeof(double);
-    const long long per_block = (long long)WARPS * D::MPW;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, info, batch, reorth);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// lane = column MGS (round 2): four matrices per warp, seven warps per SM
-template <int WARPS, int MINB, bool KEEPV>
-static int launch_mgs32_c8(Ctx* c, cudaStream_t st, const double* A, long long batch, int reorth, double* Q, double* R, int* info) {
-    auto kern = mgs_qr32_c8_kernel<WARPS, MINB, KEEPV>;
-    const size_t smem = (size_t)WARPS * MgsCol8::WARP_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long per_block = (long long)WARPS * 4;
-    const long long blocks = (batch + per_block - 1) / per_block;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, Q, R, info, batch, reorth);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
 int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double* Q,
-                         double* R, int variant) {
+                         double* R, bool qr32) {
     if (batch == 0) return LQ_OK;
-    if (m == 32 && n == 32 && variant >= 0) {
-        switch (variant) {
-            case 0:   // default (round 2): lane = column, left-looking panels, Q formation on DMMA, one 8-warp CTA per SM
-            case 59: return launch_hh32_c8<8, 1, 3, true>(c, st, A, batch, Q, R);
-            case 14: return launch_hh32<2, 4, 2, true, 4, -1>(c, st, A, batch, Q, R);  // round-1 default: reciprocal seeded from the raw rsqrt
-#ifdef LQ_ALL_VARIANTS  // design-space variants measured in profiles/ (build with LINALG_B200_ALL_VARIANTS=1; tools/sweep_hh32.py)
-            case 82: return launch_hh32_c8<8, 1, 3, true, false, false, Col8P>(c, st, A, batch, Q, R);  // padded reflector storage
-            case 80: return launch_hh32_c8<8, 1, 3, true, false, true>(c, st, A, batch, Q, R);   // next panel prefetched into registers
-            case 81: return launch_hh32_c8<8, 1, 3, false, false, true>(c, st, A, batch, Q, R);
-            case 6: return launch_hh32<2, 4, 2, true, 4, 2>(c, st, A, batch, Q, R);   // 2 Newton steps, reciprocal behind the norm
-            case 13: return launch_hh32_pipe<2, 4, 2>(c, st, A, batch, Q, R);
-            case 21: return launch_hh32_dmma<4, 2>(c, st, A, batch, Q, R);
-            case 52: return launch_hh32_c8<4, 2>(c, st, A, batch, Q, R);
-            case 60: return launch_hh32_c8<8, 1, 3, false>(c, st, A, batch, Q, R);
-            case 36: return launch_hh32_ll<2, 4, 3, 3, true>(c, st, A, batch, Q, R);
-            case 5: return launch_hh32<2, 4, 2, true, 4>(c, st, A, batch, Q, R);
-            case 1: return launch_hh32<1, 1, 4, false, 3>(c, st, A, batch, Q, R);
-            case 2: return launch_hh32<1, 2, 4, false, 2>(c, st, A, batch, Q, R);
-            case 3: return launch_hh32<2, 2, 4, false, 4>(c, st, A, batch, Q, R);
-            case 4: return launch_hh32<2, 4, 2, false, 5>(c, st, A, batch, Q, R);
-            case 7: return launch_hh32<2, 4, 1, true, 8>(c, st, A, batch, Q, R);
-            case 8: return launch_hh32<4, 4, 4, true, 4>(c, st, A, batch, Q, R);
-            case 9: return launch_hh32<4, 4, 4, true, 3>(c, st, A, batch, Q, R);
-            case 10: return launch_hh32<4, 4, 4, false, 5>(c, st, A, batch, Q, R);
-            case 11: return launch_hh32<2, 2, 4, true, 3>(c, st, A, batch, Q, R);
-            case 12: return launch_hh32<4, 4, 2, true, 8, 2>(c, st, A, batch, Q, R);
-            case 20: return launch_hh32_dmma<2, 4>(c, st, A, batch, Q, R);
-            case 22: return launch_hh32_dmma<1, 8>(c, st, A, batch, Q, R);
-            case 23: return launch_hh32_dmma<4, 2, 1>(c, st, A, batch, Q, R);
-            case 50: return launch_hh32_c8<2, 5>(c, st, A, batch, Q, R);
-            case 51: return launch_hh32_c8<2, 4>(c, st, A, batch, Q, R);
-            case 53: return launch_hh32_c8<2, 5, 1>(c, st, A, batch, Q, R);
-            case 54: return launch_hh32_c8<2, 5, 2>(c, st, A, batch, Q, R);
-            case 55: return launch_hh32_c8<2, 5, 3, true>(c, st, A, batch, Q, R);
-            case 56: return launch_hh32_c8<2, 4, 3, true>(c, st, A, batch, Q, R);
-            case 57: return launch_hh32_c8<2, 5, 1, true>(c, st, A, batch, Q, R);
-            case 58: return launch_hh32_c8<4, 2, 3, true>(c, st, A, batch, Q, R);
-            case 64: return launch_hh32_c8<8, 1, 3, true, true>(c, st, A, batch, Q, R);   // + L2 prefetch of the later panels
-            case 65: return launch_hh32_c8<8, 1, 3, false, true>(c, st, A, batch, Q, R);
-            case 66: return launch_hh32_c8<4, 2, 3, true, true>(c, st, A, batch, Q, R);
-            case 61: return launch_hh32_c8<4, 2, 1, true>(c, st, A, batch, Q, R);
-            case 62: return launch_hh32_c8<4, 2, 1, false>(c, st, A, batch, Q, R);
-            case 63: return launch_hh32_c8<4, 2, 2, false>(c, st, A, batch, Q, R);
-            case 30: return launch_hh32_ll<2, 4, 4>(c, st, A, batch, Q, R);
-            case 32: return launch_hh32_ll<2, 4, 4, 1>(c, st, A, batch, Q, R);
-            case 34: return launch_hh32_ll<2, 4, 3>(c, st, A, batch, Q, R);
-            case 37: return launch_hh32_ll<2, 4, 3, 1, true>(c, st, A, batch, Q, R);
-            case 38: return launch_hh32_ll<1, 4, 2, 3, true>(c, st, A, batch, Q, R);
-            case 39: return launch_hh32_ll<1, 4, 2, 1, true>(c, st, A, batch, Q, R);
-            case 40: return launch_hh32_ll<2, 4, 4, 2>(c, st, A, batch, Q, R);
-            case 41: return launch_hh32_ll<2, 2, 6, 3, true>(c, st, A, batch, Q, R);
-            case 24: return launch_hh32_dmma<4, 2, 2>(c, st, A, batch, Q, R);
-#endif
-            default: break;
-        }
-        set_error(c, "householder_qr_batched: unknown kernel variant %d (the design-space variants need a library built with "
-                     "LINALG_B200_ALL_VARIANTS=1)", variant);
-        return LQ_ERR_ARG;
+    if (m == 32 && n == 32 && qr32) {
+        // lane = column, four matrices per warp, left-looking panels, Q formation on DMMA, one 8-warp CTA per SM
+        constexpr int WARPS = 8;
+        const size_t smem = (size_t)WARPS * Col8::WARP_DOUBLES * sizeof(double);
+        return launch_batched<hh_qr32_c8_kernel<WARPS, 1>>(c, st, (batch + 4 * WARPS - 1) / (4 * WARPS), WARPS * 32, smem,
+                                                           (int)smem, A, Q, R, batch);
     }
     const size_t smem = small_hh_smem_doubles(m, n, 0) * sizeof(double);
-    if (smem <= (size_t)c->max_smem) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(small_hh_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->max_smem));
-            configured.set(c->device);
-        }
-        small_hh_kernel<0><<<(unsigned)batch, 256, smem, st>>>(A, nullptr, Q, R, nullptr, m, n, 0);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-        return LQ_OK;
-    }
+    if (smem <= (size_t)c->max_smem)
+        return launch_batched<small_hh_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, m, n, 0);
     // too large for one CTA: blocked path, matrix by matrix (stream `st` must be the context stream)
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(blocked_householder_qr(c, A + b * (long long)m * n, m, n, Q + b * (long long)m * n,
@@ -222,29 +34,17 @@ int mgs_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long ba
                           double* Q, double* R, int* info) {
     if (batch == 0) return LQ_OK;
     if (m == 32 && n == 32) {
-        static const int mgs_variant = getenv("LINALG_B200_MGS_VARIANT") ? atoi(getenv("LINALG_B200_MGS_VARIANT")) : 0;  // read once
-        switch (mgs_variant) {
-#ifdef LQ_ALL_VARIANTS
-            // lane = column form (round-2 experiment, profiles/ubench_r2.md): 109 M matrices/s against 135 for the default
-            case 1: return launch_mgs32_c8<7, 1, true>(c, st, A, batch, reorth, Q, R, info);
-            case 2: return launch_mgs32_c8<7, 1, false>(c, st, A, batch, reorth, Q, R, info);
-            case 3: return launch_mgs32_c8<3, 2, true>(c, st, A, batch, reorth, Q, R, info);
-#endif
-            default: return launch_mgs32<2, 4, 2, 4>(c, st, A, batch, reorth, Q, R, info);
-        }
+        using D = Dist32<2, 4>;
+        constexpr int WARPS = 2;
+        const long long per_block = (long long)WARPS * D::MPW;
+        return launch_batched<mgs_qr32_kernel<2, 4, WARPS, 4>>(c, st, (batch + per_block - 1) / per_block, WARPS * 32,
+                                                               (size_t)per_block * D::MGS_DOUBLES * sizeof(double), 0, A, Q,
+                                                               R, info, batch, reorth);
     }
     const size_t smem = small_mgs_smem_doubles(m, n, 0) * sizeof(double);
-    if (smem <= (size_t)c->max_smem) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(small_mgs_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->max_smem));
-            configured.set(c->device);
-        }
-        small_mgs_kernel<0><<<(unsigned)batch, 256, smem, st>>>(A, nullptr, Q, R, nullptr, info, m, n, 0, reorth);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-        return LQ_OK;
-    }
+    if (smem <= (size_t)c->max_smem)
+        return launch_batched<small_mgs_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, info, m,
+                                                   n, 0, reorth);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_mgs_qr(c, A + b * (long long)m * n, m, n, reorth, Q + b * (long long)m * n,
                             R + b * (long long)n * n, info ? info + b : nullptr));
@@ -263,17 +63,9 @@ int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const doub
     rc = lstsq_stream_kernel_launch(c, st, A, B, batch, m, n, nrhs, X);
     if (rc != LQ_ERR_UNSUPPORTED) return rc;
     const size_t smem = small_hh_smem_doubles(m, n, nrhs) * sizeof(double);
-    if (smem <= (size_t)c->max_smem) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(small_hh_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->max_smem));
-            configured.set(c->device);
-        }
-        small_hh_kernel<1><<<(unsigned)batch, 256, smem, st>>>(A, B, nullptr, nullptr, X, m, n, nrhs);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-        return LQ_OK;
-    }
+    if (smem <= (size_t)c->max_smem)
+        return launch_batched<small_hh_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, m, n,
+                                                  nrhs);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_lstsq_householder(c, A + b * (long long)m * n, B + b * (long long)m * nrhs, m, n, nrhs,
                                        X + b * (long long)n * nrhs));
@@ -290,17 +82,9 @@ int lstsq_mgs_batched_stream(Ctx* c, cudaStream_t st, const double* A, const dou
         if (rc != LQ_ERR_UNSUPPORTED) return rc;
     }
     const size_t smem = small_mgs_smem_doubles(m, n, nrhs) * sizeof(double);
-    if (smem <= (size_t)c->max_smem) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(small_mgs_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, c->max_smem));
-            configured.set(c->device);
-        }
-        small_mgs_kernel<1><<<(unsigned)batch, 256, smem, st>>>(A, B, nullptr, nullptr, X, info, m, n, nrhs, 0);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-        return LQ_OK;
-    }
+    if (smem <= (size_t)c->max_smem)
+        return launch_batched<small_mgs_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, info, m,
+                                                   n, nrhs, 0);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_lstsq_mgs(c, A + b * (long long)m * n, B + b * (long long)m * nrhs, m, n, nrhs,
                                X + b * (long long)n * nrhs, info ? info + b : nullptr));
@@ -311,9 +95,6 @@ int lstsq_mgs_batched_stream(Ctx* c, cudaStream_t st, const double* A, const dou
 // Chunks of the batch flow through two lanes (stream + device buffers each): H2D, kernel and D2H
 // of neighbouring chunks overlap on the copy engines.  With pinned host buffers the copies are
 // truly asynchronous; pageable buffers still work (the runtime stages them).
-struct ChunkPlan {
-    long long chunk = 0;
-};
 static long long pick_chunk(long long batch, size_t bytes_per_item) {
     const size_t target = (size_t)192 << 20;  // ~192 MiB of device traffic per chunk
     long long ch = (long long)std::max<size_t>(1, target / std::max<size_t>(1, bytes_per_item));
@@ -373,8 +154,10 @@ int lq_householder_qr_batched_dev(lq_ctx* h, const double* A, int64_t batch, int
     Ctx* c = as_ctx(h);
     LQ_ARGS_QR(c, A, batch, m, n);
     LQ_REQUIRE(c, m >= n, LQ_ERR_SHAPE, "householder_qr needs m >= n (got %d x %d), linalg/qr.py:52", m, n);
+    LQ_REQUIRE(c, variant == 0, LQ_ERR_ARG, "householder_qr_batched: kernel variant %d does not exist (0 is the only one)",
+               variant);
     LQ_CUDA(c, cudaSetDevice(c->device));
-    return hh_qr_batched_stream(c, c->stream, A, batch, m, n, Q, R, variant);
+    return hh_qr_batched_stream(c, c->stream, A, batch, m, n, Q, R, true);
 }
 
 int lq_householder_qr_batched(lq_ctx* h, const double* A, int64_t batch, int m, int n, double* Q, double* R) {
@@ -390,7 +173,7 @@ int lq_householder_qr_batched(lq_ctx* h, const double* A, int64_t batch, int m, 
     }
     return run_chunked(c, batch, mn, 0, mn, nn, 0, A, nullptr, Q, R, nullptr,
                        [&](cudaStream_t st, long long cnt, void* dA, void*, void* dQ, void* dR, void*) {
-                           return hh_qr_batched_stream(c, st, (const double*)dA, cnt, m, n, (double*)dQ, (double*)dR, 0);
+                           return hh_qr_batched_stream(c, st, (const double*)dA, cnt, m, n, (double*)dQ, (double*)dR, true);
                        });
 }
 

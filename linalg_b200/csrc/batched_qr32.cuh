@@ -1,19 +1,16 @@
-// K1 / K2: batched 32x32 QR, matrix distributed over the registers of a lane group.
+// K2: batched 32x32 MGS QR, matrix distributed over the registers of a lane group.
 //
-// Reference semantics: linalg/qr.py:52-100 (householder_qr) and :14-49 (qr, MGS), applied to
-// every A[b] of a (batch, 32, 32) row-major float64 array.
+// Reference semantics: linalg/qr.py:14-49 (qr, MGS), applied to every A[b] of a (batch, 32, 32)
+// row-major float64 array.
 //
 // Layout (template P, C): a matrix is spread over L = P * (32 / C) lanes; lane (p, lc) holds
 // rows  i = P*ii + p  (ii = 0..32/P-1)  of the C column slots  col(s, lc)  (folded so that
 // finished columns retire whole slots: slot s is ascending for even s, descending for odd s).
 // With P = 2, C = 4 each lane keeps 4 columns x 16 rows = 64 doubles (128 registers), two
-// matrices share a warp, and every Householder vector element delivered through shared memory
-// feeds 4 FMAs per use; the only cross-lane traffic per reflector is the vector itself, one
-// partner exchange of the C partial dot products and one scalar broadcast.  No column norm
-// reduction is needed: the owner lane's own dot product IS the sum of squares.
-//
-// Reflector convention: H = I - beta v v^T, v = x + copysign(||x||, x0) e1, beta = 2 / v^T v
-// (algebraically the reference's unit-norm w with tau = 2), skipped when ||x|| < 1e-12.
+// matrices share a warp, and every column element delivered through shared memory feeds 4 FMAs
+// per use; the only cross-lane traffic per column is the column itself, one partner exchange of
+// the C partial dot products and one scalar broadcast.  No column norm reduction is needed: the
+// owner lane's own dot product IS the sum of squares.
 #pragma once
 
 #include "common.cuh"
@@ -28,13 +25,12 @@ struct Dist32 {
     static constexpr int MPW = 32 / L;  // matrices per warp
     static constexpr int RPL = N / P;   // rows per lane
     static_assert(L <= 32 && L >= 1 && (L & (L - 1)) == 0, "bad distribution");
-    // per-matrix shared scratch: 32 reflector rows + beta[32] + v0[32].  Row lanes (p) and the
-    // matrices of a warp are staggered by 4 banks so that the broadcast 16-byte loads of the
-    // different (matrix, p) groups of one warp never collide.
+    // per-matrix shared scratch: two alternating column buffers.  Row lanes (p) and the matrices
+    // of a warp are staggered by 4 banks so that the broadcast 16-byte loads of the different
+    // (matrix, p) groups of one warp never collide.
     static constexpr int PSTRIDE = RPL + (P > 1 ? 2 : 0);   // doubles between the p sub-rows
-    static constexpr int ROWP = P * PSTRIDE;                // doubles per reflector row
-    static constexpr int SMEM_DOUBLES = N * ROWP + 2 * N + 4;
-    static constexpr int MGS_DOUBLES = 2 * ROWP + (P > 1 ? 4 : 0);  // MGS: two alternating reflector rows per matrix
+    static constexpr int ROWP = P * PSTRIDE;                // doubles per column buffer
+    static constexpr int MGS_DOUBLES = 2 * ROWP + (P > 1 ? 4 : 0);
     __device__ __host__ static constexpr int col(int s, int lc) {
         return (s & 1) ? ((s + 1) * LC - 1 - lc) : (s * LC + lc);
     }
@@ -50,244 +46,6 @@ __device__ __forceinline__ double group_sum(double v) {
 #pragma unroll
     for (int o = D::LC; o < D::L; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Householder QR.  grid: ceil(batch / (WARPS * MPW)) blocks of WARPS warps.
-// ---------------------------------------------------------------------------------------------
-template <int P, int C, int WARPS, bool KEEPV, int MINB, int NR>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-    hh_qr32_kernel(const double* __restrict__ A, double* __restrict__ Q, double* __restrict__ R, long long batch) {
-    using D = Dist32<P, C>;
-    constexpr int N = 32, RPL = D::RPL, LC = D::LC, L = D::L;
-    extern __shared__ __align__(16) double smem[];
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int g = lane / L, lm = lane % L, p = lm / LC, lc = lm % LC;
-    const long long mat = ((long long)blockIdx.x * WARPS + warp) * D::MPW + g;
-    const bool valid = mat < batch;
-    const long long matc = valid ? mat : (batch - 1);
-
-    double* vb = smem + (size_t)(warp * D::MPW + g) * D::SMEM_DOUBLES;
-    double* betas = vb + N * D::ROWP;
-    double* v0s = betas + N;
-
-    int colv[C];
-#pragma unroll
-    for (int s = 0; s < C; ++s) colv[s] = D::col(s, lc);
-
-    // ---- load: lane (p, lc) reads A[P*ii + p][col(s, lc)]
-    double r[C][RPL];
-    {
-        const double* Ag = A + matc * (N * N) + p * N;
-#pragma unroll
-        for (int ii = 0; ii < RPL; ++ii)
-#pragma unroll
-            for (int s = 0; s < C; ++s) r[s][ii] = ld_stream(Ag + ii * (P * N) + colv[s]);
-    }
-
-    // ================= R phase: H_31 ... H_0 A = R =================
-#pragma unroll
-    for (int j = 0; j < N; ++j) {
-        const int so = D::owner_slot(j), lo = D::owner_lc(j);
-        const int iib = j / P, jp = j % P;
-        const int ii0 = iib & ~1;  // 16-byte aligned start for the paired loops
-        double* vj = vb + j * D::ROWP + p * D::PSTRIDE;
-
-        // owner lanes (both row parities) publish x = R[j:, j]
-        if (lc == lo) {
-#pragma unroll
-            for (int ii = ii0; ii < RPL; ii += 2)
-                *reinterpret_cast<double2*>(vj + ii) = make_double2(r[so][ii], r[so][ii + 1]);
-        }
-        __syncwarp();
-
-        // partial dots over rows >= j (row j enters with the raw pivot x0); two accumulators per
-        // column slot shorten the dependent DFMA chains
-        double d[C], d2[C];
-        double vkeep[KEEPV ? RPL : 2];
-#pragma unroll
-        for (int s = 0; s < C; ++s) d[s] = 0.0, d2[s] = 0.0;
-#pragma unroll
-        for (int ii = ii0; ii < RPL; ii += 2) {
-            double2 vv = *reinterpret_cast<const double2*>(vj + ii);
-            if (ii < iib) vv.x = 0.0;                                  // row below the pivot row pair
-            if (ii == iib) vv.x = (p >= jp) ? vv.x : 0.0;              // boundary row: i = P*iib + p >= j ?
-            if (ii + 1 == iib) vv.y = (p >= jp) ? vv.y : 0.0;
-            if (KEEPV) {
-                vkeep[ii] = vv.x;
-                vkeep[ii + 1] = vv.y;
-            }
-#pragma unroll
-            for (int s = so; s < C; ++s) {
-                d[s] = fma(vv.x, r[s][ii], d[s]);
-                if (C - so >= 3) d[s] = fma(vv.y, r[s][ii + 1], d[s]);   // >= 3 independent chains already
-                else d2[s] = fma(vv.y, r[s][ii + 1], d2[s]);
-            }
-        }
-        if (C - so < 3) {
-#pragma unroll
-            for (int s = so; s < C; ++s) d[s] += d2[s];
-        }
-        // sum of squares of x = the owner column's own dot product
-        double ss = group_sum<P, C>(d[so]);
-        ss = __shfl_sync(0xffffffffu, ss, lo, L);
-        const double x0 = vb[j * D::ROWP + jp * D::PSTRIDE + iib];
-
-        const double ssc = fmax(ss, 1e-300);
-        // ||x|| = ss * rsqrt(ss): the Newton-refined rsqrt is good to 2.7e-16 (lq_probe 13), so the extra
-        // correction step of sqrt_nr_t would only polish the last bit of R[j][j] while sitting on the serial chain
-        double nrm, beta;
-        if (NR >= 0) {
-            nrm = ssc * rsqrt_nr_t<(NR >= 0 ? NR : 2)>(ssc);
-        } else {
-            // NR < 0: y = 1/||x||, beta = 2 / v^T v = y^2 / (1 + |x0| y); the reciprocal is seeded from the UNREFINED y,
-            // so its MUFU runs beside the Newton steps of y instead of behind them (shorter serial chain)
-            const double ax0 = fabs(x0);
-            double y = rsqrt_seed(ssc);
-            double u = rcp_seed(fma(ax0, y, 1.0));
-            const double hx = 0.5 * ssc;
-#pragma unroll
-            for (int it = 0; it < 2; ++it) {
-                const double e = fma(-hx * y, y, 0.5);
-                y = fma(y, e, y);
-            }
-            nrm = ssc * y;
-            const double D = fma(ax0, y, 1.0);
-#pragma unroll
-            for (int it = 0; it < 2; ++it) {
-                const double e = fma(-D, u, 1.0);
-                u = fma(u, e, u);
-            }
-            beta = (y * y) * u;
-        }
-        const bool skip = nrm < kEps;  // qr.py:79-80
-        const double alpha = copysign(nrm, x0);
-        const double v0 = x0 + alpha;
-        if (NR >= 0) beta = rcp_nr_t<(NR >= 0 ? NR : 2)>(nrm * fabs(v0));  // 2 / v^T v
-        beta = skip ? 0.0 : beta;
-        if (lm == 0) {
-            betas[j] = beta;
-            v0s[j] = v0;
-        }
-        const bool piv = (p == jp);
-        const double alpha_m = piv ? alpha : 0.0;
-
-#pragma unroll
-        for (int s = so; s < C; ++s) {
-            // v^T R[:, c] = x^T R[:, c] + alpha * R[j, c]
-            const double part = group_sum<P, C>(fma(alpha_m, r[s][iib], d[s]));
-            d[s] = beta * part;
-        }
-        // R[j:, c] -= s_c v
-#pragma unroll
-        for (int ii = ii0; ii < RPL; ii += 2) {
-            double2 vv;
-            if (KEEPV) {
-                vv.x = vkeep[ii];
-                vv.y = vkeep[ii + 1];
-            } else {
-                vv = *reinterpret_cast<const double2*>(vj + ii);
-                if (ii < iib) vv.x = 0.0;
-                if (ii == iib) vv.x = (p >= jp) ? vv.x : 0.0;
-                if (ii + 1 == iib) vv.y = (p >= jp) ? vv.y : 0.0;
-            }
-            if (ii == iib) vv.x = piv ? v0 : vv.x;  // pivot row carries v0 = x0 + alpha
-            if (ii + 1 == iib) vv.y = piv ? v0 : vv.y;
-#pragma unroll
-            for (int s = so; s < C; ++s) {
-                r[s][ii] = fma(-d[s], vv.x, r[s][ii]);
-                r[s][ii + 1] = fma(-d[s], vv.y, r[s][ii + 1]);
-            }
-        }
-        // exact diagonal for the owner (mathematically the update already gives -alpha)
-        if (lc == lo && piv && !skip) r[so][iib] = -alpha;
-    }
-
-    // ---- store R (strict lower triangle forced to exact zeros, qr.py:97)
-    if (valid) {
-        double* Rg = R + mat * (N * N) + p * N;
-#pragma unroll
-        for (int ii = 0; ii < RPL; ++ii)
-#pragma unroll
-            for (int s = 0; s < C; ++s) {
-                const int i = P * ii + p;
-                st_stream(Rg + ii * (P * N) + colv[s], (colv[s] >= i) ? r[s][ii] : 0.0);
-            }
-    }
-    __syncwarp();
-
-    // ================= Q phase: Q = H_0 (H_1 (... H_31 I)) =================
-    double (&q)[C][RPL] = r;
-#pragma unroll
-    for (int ii = 0; ii < RPL; ++ii)
-#pragma unroll
-        for (int s = 0; s < C; ++s) q[s][ii] = (P * ii + p == colv[s]) ? 1.0 : 0.0;
-
-#pragma unroll
-    for (int j = N - 1; j >= 0; --j) {
-        const int so = D::owner_slot(j);
-        const int iib = j / P, jp = j % P;
-        const int ii0 = iib & ~1;
-        const double* vj = vb + j * D::ROWP + p * D::PSTRIDE;
-        const double beta = betas[j];
-        const double v0 = v0s[j];
-        const bool piv = (p == jp);
-
-        double d[C], d2[C];
-        double vkeep[KEEPV ? RPL : 2];
-#pragma unroll
-        for (int s = 0; s < C; ++s) d[s] = 0.0, d2[s] = 0.0;
-#pragma unroll
-        for (int ii = ii0; ii < RPL; ii += 2) {
-            double2 vv = *reinterpret_cast<const double2*>(vj + ii);
-            if (ii < iib) vv.x = 0.0;
-            if (ii == iib) vv.x = piv ? v0 : ((p > jp) ? vv.x : 0.0);
-            if (ii + 1 == iib) vv.y = piv ? v0 : ((p > jp) ? vv.y : 0.0);
-            if (KEEPV) {
-                vkeep[ii] = vv.x;
-                vkeep[ii + 1] = vv.y;
-            }
-#pragma unroll
-            for (int s = so; s < C; ++s) {
-                d[s] = fma(vv.x, q[s][ii], d[s]);
-                if (C - so >= 3) d[s] = fma(vv.y, q[s][ii + 1], d[s]);
-                else d2[s] = fma(vv.y, q[s][ii + 1], d2[s]);
-            }
-        }
-        if (C - so < 3) {
-#pragma unroll
-            for (int s = so; s < C; ++s) d[s] += d2[s];
-        }
-#pragma unroll
-        for (int s = so; s < C; ++s) d[s] = beta * group_sum<P, C>(d[s]);
-#pragma unroll
-        for (int ii = ii0; ii < RPL; ii += 2) {
-            double2 vv;
-            if (KEEPV) {
-                vv.x = vkeep[ii];
-                vv.y = vkeep[ii + 1];
-            } else {
-                vv = *reinterpret_cast<const double2*>(vj + ii);
-                if (ii < iib) vv.x = 0.0;
-                if (ii == iib) vv.x = piv ? v0 : ((p > jp) ? vv.x : 0.0);
-                if (ii + 1 == iib) vv.y = piv ? v0 : ((p > jp) ? vv.y : 0.0);
-            }
-#pragma unroll
-            for (int s = so; s < C; ++s) {
-                q[s][ii] = fma(-d[s], vv.x, q[s][ii]);
-                q[s][ii + 1] = fma(-d[s], vv.y, q[s][ii + 1]);
-            }
-        }
-    }
-
-    if (valid) {
-        double* Qg = Q + mat * (N * N) + p * N;
-#pragma unroll
-        for (int ii = 0; ii < RPL; ++ii)
-#pragma unroll
-            for (int s = 0; s < C; ++s) st_stream(Qg + ii * (P * N) + colv[s], q[s][ii]);
-    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -311,7 +69,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     const bool valid = mat < batch;
     const long long matc = valid ? mat : (batch - 1);
     // scratch: two alternating column buffers per matrix; the (matrix, row-lane) groups of a warp are
-    // staggered by 4 banks like in the Householder kernel (un-staggered they collide 4-way on every LDS.128)
+    // staggered by 4 banks (un-staggered they collide 4-way on every LDS.128)
     double* vb = smem + (size_t)(warp * D::MPW + g) * D::MGS_DOUBLES;
 
     int colv[C];

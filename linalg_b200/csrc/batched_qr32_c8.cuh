@@ -15,10 +15,24 @@
 //            shuffle per column for ||x||^2; the scalar chain is shared by four matrices).
 //   storage  reflector j = rows (j & ~1)..31 in natural order, pivot patched to v0 (the row above an odd pivot to 0)
 //            after the scalar chain: 544 + 32 doubles per matrix.
-//   Q phase  compact-WY on DMMA.8x8x4, one matrix at a time on all 32 lanes (see batched_qr32_dmma.cuh).
+//   Q phase  compact-WY on DMMA.8x8x4, one matrix at a time on all 32 lanes: Q^T lives in 16 accumulator tiles
+//            (32 doubles / lane).  A DMMA.8x8x4 (the only f64 MMA shape sm_100a has; every mma.sync f64 shape lowers to
+//            it) does 256 FMAs for one issue slot (the round-1 kernel's rank-1 DFMA Q phase issued ~1 930 FP64 instructions
+//            per matrix).
+//            G_p = V_p^T V_p (4 panels of 8 reflectors)                         20 DMMA
+//            T_p by the dlarft row recurrence, lane (g, t) = row g of panel t    ~36 DFMA for all four panels at once
+//            for p = 3..0:  W^T = Q^T V_p ; W2^T = W^T (-T_p)^T ; Q^T += W2^T V_p^T   28 + 20 + 60 DMMA
+//            An accumulator fragment IS a valid A operand when the contraction index is permuted (k = t <-> column
+//            2t+i), so W^T and W2^T never leave registers; V is read from shared memory directly in B-fragment order.
+//
+// Tile / fragment conventions (lane l, g = l >> 2, t = l & 3), mma.m8n8k4.f64:
+//   A[g][t], B[t][g], C[g][2t], C[g][2t+1].
+//   qt[cb][rb][i] = Q[8 rb + 2t + i][8 cb + g]          (tile (cb, rb) of Q^T)
+//   F1(p, rb, i)  = V[8 rb + 2t + i][8 p + g]           (B operand of W^T = Q^T V, A and B operand of the Gram)
+//   F3(p, rb, i)  = V[8 rb + g][8 p + 2t + i]           (B operand of the update; the panel's own W^T tile)
 #pragma once
 
-#include "batched_qr32.cuh"
+#include "common.cuh"
 
 namespace lq {
 
@@ -33,7 +47,6 @@ struct Col8 {
         for (int t = 0; t < j; ++t) o += vsize(t);
         return o;
     }
-    __device__ static __forceinline__ int voff_rt(int j) { return voff(j); }
     static constexpr int VDOUBLES = 544;
     static constexpr int BETA = VDOUBLES;
     static constexpr int MAT = 580;      // 290 16-byte words = 2 (mod 8): the four matrices of a warp hit four different bank quads
@@ -46,129 +59,61 @@ static_assert(Col8::voff_slow(32) == Col8::VDOUBLES && Col8::voff(32) == Col8::V
 static_assert(Col8::voff(7) == Col8::voff_slow(7) && Col8::voff(18) == Col8::voff_slow(18) && Col8::voff(31) == Col8::voff_slow(31),
               "closed-form offsets");
 
-// The same storage with every even vector padded so that vector 2k+1 starts 8 (mod 16) doubles behind vector 2k: the F1 fragment
-// loads of the Q phase (a quarter-warp reads 8 consecutive doubles of two neighbouring vectors with one LDS.128) then hit all
-// 32 banks once instead of colliding (6 -> 4 wavefronts per load; +112 doubles per matrix, still eight warps per SM).
-struct Col8P {
-    __host__ __device__ static constexpr int r0(int j) { return j & ~1; }
-    __host__ __device__ static constexpr int pad(int j) { return (j & 1) ? 0 : ((j + 8) & 15); }
-    __host__ __device__ static constexpr int vsize(int j) { return 32 - (j & ~1) + pad(j); }
-    __host__ __device__ static constexpr int voff(int j) {
-        int o = 0;
-        for (int t = 0; t < j; ++t) o += vsize(t);
-        return o;
-    }
-    // run-time index (Q phase prologue): closed form of the sum above.  pad(2k) = (2k + 8) & 15 has period 8 in k and sums to
-    // 56 over a period; the unpadded part is Col8's closed form
-    __device__ static __forceinline__ int voff_rt(int j) {
-        const int h = j >> 1;                                   // number of complete (even, odd) pairs before j
-        const int unp = 2 * (32 * h - h * (h - 1)) + (j & 1) * (32 - 2 * h);
-        const int per = h >> 3, rem = h & 7;                    // pads of the even vectors 0, 2, ..., 2 (h - 1)
-        // partial sums of {8, 10, 12, 14, 0, 2, 4, 6}: 0, 8, 18, 30, 44, 44, 46, 50
-        const int ps = (rem == 0) ? 0 : (rem == 1) ? 8 : (rem == 2) ? 18 : (rem == 3) ? 30 : (rem <= 5) ? 44 : (rem == 6) ? 46 : 50;
-        const int padsum = 56 * per + ps + ((j & 1) ? (((2 * h) + 8) & 15) : 0);
-        return unp + padsum;
-    }
-    static constexpr int VDOUBLES = 656;
-    static constexpr int BETA = VDOUBLES;
-    static constexpr int MAT = 692;      // 346 16-byte words = 2 (mod 8)
-    static constexpr int GSTR = 66;
-    static constexpr int SCRATCH = 3 * 4 * GSTR;
-    static constexpr int WARP_DOUBLES = 4 * MAT + SCRATCH;
-};
-static_assert(Col8P::voff(32) == Col8P::VDOUBLES, "padded size");
-static_assert((Col8P::voff(1) - Col8P::voff(0)) % 16 == 8 && (Col8P::voff(11) - Col8P::voff(10)) % 16 == 8 &&
-                  (Col8P::voff(31) - Col8P::voff(30)) % 16 == 8,
-              "odd vectors start 8 (mod 16) doubles behind their even neighbours");
-
-__device__ __forceinline__ double2 lds128v(const double* p) {
-    double2 v;
-    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(smem_u32(p)));
-    return v;
-}
-
-// PHASES: 3 = product; 1 = R phase only, 2 = Q phase only (timing diagnostics).  KEEPV: keep the broadcast reflector in
-// registers between dot product and update instead of re-reading it.
-template <int WARPS, int MINB, int PHASES = 3, bool KEEPV = false, bool PF = false, bool PF2 = false, typename LAY = Col8>
+// grid: ceil(batch / (4 WARPS)) blocks of WARPS warps, WARPS * Col8::WARP_DOUBLES doubles of dynamic shared memory.
+// The broadcast reflector is kept in registers between dot product and update instead of being re-read.
+template <int WARPS, int MINB>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     hh_qr32_c8_kernel(const double* __restrict__ A, double* __restrict__ Q, double* __restrict__ R, long long batch) {
     constexpr int N = 32;
     extern __shared__ __align__(16) double smem[];
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double* wbase = smem + (size_t)warp * LAY::WARP_DOUBLES;
+    double* wbase = smem + (size_t)warp * Col8::WARP_DOUBLES;
     const long long mat0 = ((long long)blockIdx.x * WARPS + warp) * 4;
 
-    if (PHASES & 1) {
+    {
         // ================= R phase (four matrices per warp, 8 lanes each, lane = column) =================
         const int g4 = lane >> 3, c = lane & 7;
         const long long mat = mat0 + g4;
         const bool valid = mat < batch;
         const long long matc = valid ? mat : (batch - 1);
-        double* vb = wbase + g4 * LAY::MAT;
-        double* betas = vb + LAY::BETA;
+        double* vb = wbase + g4 * Col8::MAT;
+        double* betas = vb + Col8::BETA;
 
-        if (PF) {
-            // the later panels of my four matrices: pull their lines into L2 now (a row is two 128-byte lines, panel 0 only
-            // brings the first half of the first one); 256 lines per warp = 8 prefetches per lane
-            const double* base = A + mat0 * (N * N);
-            const long long last = (batch - mat0) * (N * N) * 8 - 1;  // bytes of valid input behind base, minus one
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const long long off = ((long long)q * 32 + lane) * 128;
-                if (off <= last) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(base) + off));
-            }
-        }
-        double nxt[PF2 ? N : 1];  // PF2: the next panel's column, loaded while this panel is being factored
 #pragma unroll
         for (int p = 0; p < 4; ++p) {
             const int col = 8 * p + c;
             double a[N];
-            if (!PF2 || p == 0) {
-                const double* Ag = A + matc * (N * N) + col;
+            const double* Ag = A + matc * (N * N) + col;
 #pragma unroll
-                for (int i = 0; i < N; ++i) a[i] = ld_stream(Ag + i * N);
-            } else {
-#pragma unroll
-                for (int i = 0; i < N; ++i) a[i] = nxt[i];
-            }
+            for (int i = 0; i < N; ++i) a[i] = ld_stream(Ag + i * N);
 
             // ---- apply the reflectors of the earlier panels: a -= beta_j (v_j . a) v_j, rows j..31, all lane-local
 #pragma unroll
             for (int j = 0; j < 8 * p; ++j) {
-                const int r0 = LAY::r0(j);
-                const double* vj = vb + LAY::voff(j) - r0;  // row i of v_j at vj[i]
+                const int r0 = Col8::r0(j);
+                const double* vj = vb + Col8::voff(j) - r0;  // row i of v_j at vj[i]
                 double d[4] = {0.0, 0.0, 0.0, 0.0};
-                double vk[KEEPV ? N : 2];
+                double vk[N];
 #pragma unroll
                 for (int i = r0; i < N; i += 2) {
                     const double2 vv = *reinterpret_cast<const double2*>(vj + i);
-                    if (KEEPV) vk[i] = vv.x, vk[i + 1] = vv.y;
+                    vk[i] = vv.x, vk[i + 1] = vv.y;
                     d[(i >> 1) & 1] = fma(vv.x, a[i], d[(i >> 1) & 1]);
                     d[2 + ((i >> 1) & 1)] = fma(vv.y, a[i + 1], d[2 + ((i >> 1) & 1)]);
                 }
                 const double s = betas[j] * ((d[0] + d[1]) + (d[2] + d[3]));
 #pragma unroll
-                for (int i = r0; i < N; i += 2) {
-                    const double2 vv = KEEPV ? make_double2(vk[i], vk[i + 1]) : lds128v(vj + i);
-                    a[i] = fma(-s, vv.x, a[i]);
-                    a[i + 1] = fma(-s, vv.y, a[i + 1]);
-                }
+                for (int i = r0; i < N; ++i) a[i] = fma(-s, vk[i], a[i]);
             }
 
-            if (PF2 && p < 3) {
-                // the loads of panel p + 1 fly under the 8 column steps below (their latency was ~2 k exposed cycles per panel)
-                const double* Ag = A + matc * (N * N) + col + 8;
-#pragma unroll
-                for (int i = 0; i < N; ++i) nxt[i] = ld_stream(Ag + i * N);
-            }
             // ---- factor the 8 columns of this panel
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
                 const int j = 8 * p + jj;
-                const int r0 = LAY::r0(j);
+                const int r0 = Col8::r0(j);
                 const bool odd = (j & 1) != 0;
-                double* vj = vb + LAY::voff(j) - r0;
+                double* vj = vb + Col8::voff(j) - r0;
 
                 if (c == jj) {
 #pragma unroll
@@ -182,7 +127,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                 const double x0 = odd ? vf.y : vf.x;
 
                 double d[4];
-                double vk[KEEPV ? N : 2];
+                double vk[N];
                 d[0] = vf.x * a[r0];
                 d[2] = vf.y * a[r0 + 1];
                 d[1] = 0.0;
@@ -190,7 +135,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
 #pragma unroll
                 for (int i = r0 + 2; i < N; i += 2) {
                     const double2 vv = *reinterpret_cast<const double2*>(vj + i);
-                    if (KEEPV) vk[i] = vv.x, vk[i + 1] = vv.y;
+                    vk[i] = vv.x, vk[i + 1] = vv.y;
                     d[(i >> 1) & 1] = fma(vv.x, a[i], d[(i >> 1) & 1]);
                     d[2 + ((i >> 1) & 1)] = fma(vv.y, a[i + 1], d[2 + ((i >> 1) & 1)]);
                 }
@@ -234,11 +179,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                 a[r0] = fma(-s, vf.x, a[r0]);
                 a[r0 + 1] = fma(-s, vf.y, a[r0 + 1]);
 #pragma unroll
-                for (int i = r0 + 2; i < N; i += 2) {
-                    const double2 vv = KEEPV ? make_double2(vk[i], vk[i + 1]) : lds128v(vj + i);
-                    a[i] = fma(-s, vv.x, a[i]);
-                    a[i + 1] = fma(-s, vv.y, a[i + 1]);
-                }
+                for (int i = r0 + 2; i < N; ++i) a[i] = fma(-s, vk[i], a[i]);
                 // exact diagonal for the owner (mathematically the update already gives -alpha)
                 if (c == jj && !skip) a[j] = -alpha;
             }
@@ -261,12 +202,12 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     __syncwarp();
 
     // ================= Q phase: Q = (I - V0 T0 V0^T) ... (I - V3 T3 V3^T), backward accumulation on DMMA ==========
-    // Fragment conventions (lane l, g = l >> 2, t = l & 3) as in batched_qr32_dmma.cuh.  Software-pipelined over the four
+    // Fragment conventions as in the header comment (g = gq, t = tq).  Software-pipelined over the four
     // matrices of the warp: while the block reflectors of matrix mi are applied (DMMA chains), the T recurrence of matrix
     // mi+1 (a DFMA chain) and the Gram products of matrix mi+2 run in the same instruction stream and fill the bubbles.
     const int gq = lane >> 2, tq = lane & 3;
-    double* Gs = wbase + 4 * LAY::MAT;          // 4 panels x GSTR
-    double* Ts = Gs + 4 * LAY::GSTR;            // 2 buffers x 4 panels x GSTR (-T of the current / next matrix)
+    double* Gs = wbase + 4 * Col8::MAT;          // 4 panels x GSTR
+    double* Ts = Gs + 4 * Col8::GSTR;            // 2 buffers x 4 panels x GSTR (-T of the current / next matrix)
     const bool m1 = gq >= 2 * tq, m1b = gq >= 2 * tq + 1;   // F3 diagonal-tile masks (row g >= column 2t+i)
     const bool m0 = 2 * tq >= gq, m0b = 2 * tq + 1 >= gq;   // F1 diagonal-tile masks (row 2t+i >= column g)
     // V[r][k] lives at voff(k) + r - (k & ~1)
@@ -274,11 +215,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
 #pragma unroll
     for (int p = 0; p < 4; ++p) {
         const int k1 = 8 * p + gq;  // F1: rows 8 rb + 2 tq + {0, 1} (one 16-byte load)
-        f1o[p] = LAY::voff_rt(k1) - (k1 & ~1) + 2 * tq;
+        f1o[p] = Col8::voff(k1) - (k1 & ~1) + 2 * tq;
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const int k3 = 8 * p + 2 * tq + i;  // F3: row 8 rb + gq
-            f3o[p][i] = LAY::voff_rt(k3) - (k3 & ~1) + gq;
+            f3o[p][i] = Col8::voff(k3) - (k3 & ~1) + gq;
         }
     }
     auto F1 = [&](const double* vb, int p, int rb) -> double2 {
@@ -312,7 +253,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     };
     auto store_g = [&](const double (&G)[4][2]) {
 #pragma unroll
-        for (int p = 0; p < 4; ++p) *reinterpret_cast<double2*>(Gs + p * LAY::GSTR + gq * 8 + 2 * tq) = make_double2(G[p][0], G[p][1]);
+        for (int p = 0; p < 4; ++p) *reinterpret_cast<double2*>(Gs + p * Col8::GSTR + gq * 8 + 2 * tq) = make_double2(G[p][0], G[p][1]);
     };
     // -T of panel tq, row gq (dlarft, forward / columnwise): T[g][k] = -beta_k sum_{m=g}^{k-1} T[g][m] G[m][k]
     auto trec = [&](const double* betas, double (&Tn)[8]) {
@@ -334,7 +275,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             if (k < 7) {
 #pragma unroll
                 for (int kk = (k + 1) & ~1; kk < 8; kk += 2) {
-                    const double2 g2 = *reinterpret_cast<const double2*>(Gs + tq * LAY::GSTR + k * 8 + kk);
+                    const double2 g2 = *reinterpret_cast<const double2*>(Gs + tq * Col8::GSTR + k * 8 + kk);
                     if (kk > k) acc[kk] = fma(tk, g2.x, acc[kk]);
                     acc[kk + 1] = fma(tk, g2.y, acc[kk + 1]);
                 }
@@ -343,17 +284,17 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
     };
     auto store_t = [&](double* Tb, const double (&Tn)[8]) {
 #pragma unroll
-        for (int k = 0; k < 8; k += 2) *reinterpret_cast<double2*>(Tb + tq * LAY::GSTR + gq * 8 + k) = make_double2(Tn[k], Tn[k + 1]);
+        for (int k = 0; k < 8; k += 2) *reinterpret_cast<double2*>(Tb + tq * Col8::GSTR + gq * 8 + k) = make_double2(Tn[k], Tn[k + 1]);
     };
 
-    if (PHASES & 2) {
+    {
         double Gn[4][2], Tn[8];
         // prologue: T(0) and G(1)
         gram4(wbase, Gn);
         store_g(Gn);
         __syncwarp();
-        trec(wbase + LAY::BETA, Tn);
-        gram4(wbase + LAY::MAT, Gn);
+        trec(wbase + Col8::BETA, Tn);
+        gram4(wbase + Col8::MAT, Gn);
         __syncwarp();
         store_t(Ts, Tn);
         store_g(Gn);
@@ -361,11 +302,11 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
 
 #pragma unroll 1
         for (int mi = 0; mi < 4; ++mi) {
-            const double* vb = wbase + mi * LAY::MAT;
-            const double* Tb = Ts + (mi & 1) * 4 * LAY::GSTR;
+            const double* vb = wbase + mi * Col8::MAT;
+            const double* Tb = Ts + (mi & 1) * 4 * Col8::GSTR;
             // next matrices (indices wrap on the last iterations: harmless extra work, keeps the loop body branch-free)
-            trec(wbase + ((mi + 1) & 3) * LAY::MAT + LAY::BETA, Tn);
-            gram4(wbase + ((mi + 2) & 3) * LAY::MAT, Gn);
+            trec(wbase + ((mi + 1) & 3) * Col8::MAT + Col8::BETA, Tn);
+            gram4(wbase + ((mi + 2) & 3) * Col8::MAT, Gn);
 
             // ---- backward accumulation of matrix mi
             double qt[4][4][2];
@@ -389,7 +330,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                         f1[rb][1] = f.y;
                     }
                 }
-                const double2 tt = *reinterpret_cast<const double2*>(Tb + p * LAY::GSTR + gq * 8 + 2 * tq);
+                const double2 tt = *reinterpret_cast<const double2*>(Tb + p * Col8::GSTR + gq * 8 + 2 * tq);
                 w[p][0] = f3[p][0];
                 w[p][1] = f3[p][1];
 #pragma unroll
@@ -425,7 +366,7 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                         for (int cb = 0; cb < 4; ++cb) st_stream(Qg + (8 * rb + i) * N + 8 * cb, qt[cb][rb][i]);
             }
             __syncwarp();  // every lane has read G (for T(mi+1)) and -T(mi)
-            store_t(Ts + ((mi + 1) & 1) * 4 * LAY::GSTR, Tn);
+            store_t(Ts + ((mi + 1) & 1) * 4 * Col8::GSTR, Tn);
             store_g(Gn);
             __syncwarp();
         }

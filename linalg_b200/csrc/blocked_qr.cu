@@ -828,7 +828,7 @@ int lq_householder_qr_dev(lq_ctx* h, const double* A, int m, int n, double* Q, d
     LQ_REQUIRE(c, m >= 1 && n >= 1 && m >= n, LQ_ERR_SHAPE, "householder_qr needs m >= n >= 1 (got %d x %d)", m, n);
     LQ_CUDA(c, cudaSetDevice(c->device));
     // small problems: the one-CTA shared-memory kernel (a single launch)
-    if ((size_t)m * n <= 4096) return hh_qr_batched_stream(c, c->stream, A, 1, m, n, Q, R, -1);
+    if ((size_t)m * n <= 4096) return hh_qr_batched_stream(c, c->stream, A, 1, m, n, Q, R, false);
     // launch-latency-bound sizes: replay the whole multi-stream schedule as one CUDA graph (second call with the same
     // shape and buffers captures it, later calls replay it).  Measured (tools/check_graph.py): 256^2 0.78 -> 0.67 ms,
     // 1000^2 3.51 -> 2.99, 2048^2 6.32 -> 5.65, 4096^2 15.9 -> 14.7, 8192^2 62.1 -> 60.5.  The graph is instantiated with

@@ -7,77 +7,32 @@
 namespace lq {
 
 bool lstsq_stream_kernel_supported(int m, int n, int nrhs) {
-    if (LQ_ENV_ONCE("LINALG_B200_NO_STREAM_LSTSQ")) return false;
     return n >= 1 && n <= 64 && nrhs >= 1 && nrhs <= 32 && m >= n;
 }
 
-template <int RPT, int WARPS>
-static int launch_variant(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n, int nrhs,
-                          double* X) {
-    using Cfg = StreamCfg<3, RPT, WARPS>;
-    auto kern = lstsq_stream_kernel<RPT, WARPS>;
-    const size_t smem = Cfg::smem_doubles(n) * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, c->max_smem));
-        configured.set(c->device);
-    }
-    kern<<<(unsigned)batch, WARPS * 32, smem, st>>>(A, B, X, m, n, nrhs);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// rows per streamed block = RPT * WARPS.  Taller blocks mean fewer column steps per system (every step pays the
+// rows per streamed block = RPT * WARPS = 16 * 4.  Taller blocks mean fewer column steps per system (every step pays the
 // publish -> dots -> barrier -> norm / reciprocal chain once, whatever the block height).
 int lstsq_stream_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
                                int nrhs, double* X) {
     if (!lstsq_stream_kernel_supported(m, n, nrhs)) return LQ_ERR_UNSUPPORTED;
-    static const int variant = getenv("LINALG_B200_LSTSQ_VARIANT") ? atoi(getenv("LINALG_B200_LSTSQ_VARIANT")) : -1;
-    int v = variant;
-    if (v < 0) v = 0;
-    switch (v) {
-        case 1: return launch_variant<16, 8>(c, st, A, B, batch, m, n, nrhs, X);
-        case 2: return launch_variant<8, 8>(c, st, A, B, batch, m, n, nrhs, X);
-        case 3: return launch_variant<16, 16>(c, st, A, B, batch, m, n, nrhs, X);
-        case 4: return launch_variant<8, 16>(c, st, A, B, batch, m, n, nrhs, X);
-        default: return launch_variant<16, 4>(c, st, A, B, batch, m, n, nrhs, X);
-    }
+    constexpr int RPT = 16, WARPS = 4;
+    const size_t smem = StreamCfg<3, RPT, WARPS>::smem_doubles(n) * sizeof(double);
+    return launch_batched<lstsq_stream_kernel<RPT, WARPS>>(c, st, batch, WARPS * 32, smem, c->max_smem, A, B, X, m, n, nrhs);
 }
 
 // ---- round 2: one warp per system, block reflectors on DMMA (lstsq_tile.cuh); n <= 64, nrhs <= 16
 bool lstsq_tile_kernel_supported(int m, int n, int nrhs) {
-    static const bool off = LQ_ENV_ONCE("LINALG_B200_NO_TILE_LSTSQ");
-    return !off && n >= 1 && n <= 8 * LsTile::NCB && nrhs >= 1 && nrhs <= 8 * LsTile::NRT && m >= n;
-}
-
-template <int WARPS, int MINB, bool SSV = false>
-static int launch_tile(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n, int nrhs,
-                       double* X, int* info, int info_mode) {
-    auto kern = lstsq_tile_kernel<WARPS, MINB, SSV>;
-    const size_t smem = (size_t)WARPS * LsTile::WARP_DOUBLES * sizeof(double);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured.set(c->device);
-    }
-    const long long blocks = (batch + WARPS - 1) / WARPS;
-    kern<<<(unsigned)blocks, WARPS * 32, smem, st>>>(A, B, X, info, batch, m, n, nrhs, info_mode);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return n >= 1 && n <= 8 * LsTile::NCB && nrhs >= 1 && nrhs <= 8 * LsTile::NRT && m >= n;
 }
 
 int lstsq_tile_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
                              int nrhs, double* X, int* info, int info_mode) {
     if (!lstsq_tile_kernel_supported(m, n, nrhs)) return LQ_ERR_UNSUPPORTED;
-    static const int variant = getenv("LINALG_B200_LSTSQ_TILE_VARIANT") ? atoi(getenv("LINALG_B200_LSTSQ_TILE_VARIANT")) : 0;
-    switch (variant) {
-        case 1: return launch_tile<7, 1>(c, st, A, B, batch, m, n, nrhs, X, info, info_mode);
-        case 2: return launch_tile<8, 1>(c, st, A, B, batch, m, n, nrhs, X, info, info_mode);
-        case 3: return launch_tile<4, 2, true>(c, st, A, B, batch, m, n, nrhs, X, info, info_mode);
-        default: return launch_tile<4, 2>(c, st, A, B, batch, m, n, nrhs, X, info, info_mode);  // two 4-warp CTAs per SM: 17.4 ms (8 x 1: 17.8, 7 x 1: 19.9)
-    }
+    // two 4-warp CTAs per SM: 17.4 ms (8 x 1: 17.8, 7 x 1: 19.9)
+    constexpr int WARPS = 4;
+    const size_t smem = (size_t)WARPS * LsTile::WARP_DOUBLES * sizeof(double);
+    return launch_batched<lstsq_tile_kernel<WARPS, 2>>(c, st, (batch + WARPS - 1) / WARPS, WARPS * 32, smem, (int)smem, A, B,
+                                                       X, info, batch, m, n, nrhs, info_mode);
 }
 
 }  // namespace lq

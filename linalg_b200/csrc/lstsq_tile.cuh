@@ -54,8 +54,7 @@ static_assert(LsTile::tile(7, 7) == 35, "packed triangle");
 
 // info_mode: 0 = none, 1 = MGS semantics (first column with |R[j, j]| < 1e-12, linalg/qr.py:40-41, 1-based),
 //            2 = exactly singular R (np.linalg.solve raises LinAlgError there, linalg/qr.py:134)
-// SSV: ||x||^2 by one more shuffle from the owner column's lanes instead of its own accumulation (measured variant)
-template <int WARPS, int MINB, bool SSV = false>
+template <int WARPS, int MINB>
 __global__ void __launch_bounds__(WARPS * 32, MINB)
     lstsq_tile_kernel(const double* __restrict__ A, const double* __restrict__ B, double* __restrict__ X, int* __restrict__ info,
                       long long batch, int m, int n, int nrhs, int info_mode) {
@@ -162,24 +161,14 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                     xk[rb][1] = xrow[64 * rb + 8 + (j ^ (2 * t))];
                     d0 = fma(xk[rb][0], P[rb][0], d0);
                     d1 = fma(xk[rb][1], P[rb][1], d1);
-                    if (!SSV) {
-                        q0 = fma(xk[rb][0], xk[rb][0], q0);
-                        q1 = fma(xk[rb][1], xk[rb][1], q1);
-                    }
+                    q0 = fma(xk[rb][0], xk[rb][0], q0);
+                    q1 = fma(xk[rb][1], xk[rb][1], q1);
                 }
-                double d, q;
-                if (SSV) {
-                d = d0 + d1;
-                d += __shfl_xor_sync(0xffffffffu, d, 1);
-                d += __shfl_xor_sync(0xffffffffu, d, 2);                 // x^T a_c for c = g
-                q = __shfl_sync(0xffffffffu, d, 4 * j);                 // x^T x = the owner column's own dot product
-                } else {
-                d = d0 + d1, q = q0 + q1;
+                double d = d0 + d1, q = q0 + q1;
                 d += __shfl_xor_sync(0xffffffffu, d, 1);
                 q += __shfl_xor_sync(0xffffffffu, q, 1);
                 d += __shfl_xor_sync(0xffffffffu, d, 2);  // x^T a_c for c = g
                 q += __shfl_xor_sync(0xffffffffu, q, 2);  // x^T x
-                }
 
                 // column j - 1 of T (needs G[.][j - 1], published in the previous step, and beta_{j-1})
                 if (j > 0) {

@@ -59,9 +59,28 @@ int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, doub
                    int* rank_host, bool sharded);
 int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R, bool sharded);
 
-// ---- batched (api_batched.cu)
+// ---- batched (api_batched.cu).  qr32: 32 x 32 matrices go to the batched 32 x 32 kernel; false keeps them on the
+// one-CTA kernel (the single-matrix entry point)
 int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double* Q,
-                         double* R, int variant);
+                         double* R, bool qr32);
+
+// Launch of a batched-family kernel on stream st.  attr_smem > 0 opts the kernel in to that many bytes of dynamic shared
+// memory before its first launch on each device.  The latch is keyed on the kernel itself, not on its type: kernels with
+// the same signature (small_hh_kernel<0> and <1>) each need their own attribute.
+template <auto Kern, typename... Args>
+int launch_batched(Ctx* c, cudaStream_t st, long long blocks, int threads, size_t smem, int attr_smem, Args... args) {
+    if (attr_smem > 0) {
+        static DeviceLatch configured;
+        if (!configured.test(c->device)) {
+            LQ_CUDA(c, cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, attr_smem));
+            configured.set(c->device);
+        }
+    }
+    Kern<<<(unsigned)blocks, threads, smem, st>>>(args...);
+    LQ_CHECK_LAUNCH(c);
+    LQ_COUNT_LAUNCH(c);
+    return LQ_OK;
+}
 
 // ---- comm.cu
 int comm_allreduce_sum(Ctx* c, double* buf, long long count);

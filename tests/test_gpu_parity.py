@@ -493,47 +493,13 @@ def test_pca_matches_numpy(ctx):
     assert np.abs(pcs.T @ pcs - np.eye(k)).max() <= 1e-10
 
 
-# ------------------------------------------------------------------ alternative kernels of the same rows
-def _call_variant(ctx, dA, batch, dQ, dR, v, required=False):
-    """Run one hh32 kernel variant.  The default library ships the default kernel (0) and the round-1 kernel (14); the other
-    design-space variants exist only in a library built with LINALG_B200_ALL_VARIANTS=1 -- without it they are skipped."""
-    try:
-        ctx.call("lq_householder_qr_batched_dev", dA.ptr, batch, 32, 32, dQ.ptr, dR.ptr, v)
-        return True
-    except ValueError as exc:
-        if required or "LINALG_B200_ALL_VARIANTS" not in str(exc):
-            raise
-        if v in (6, 13):
-            pytest.skip("pipelined variant needs a library built with LINALG_B200_ALL_VARIANTS=1")
-        return False
-
-
-@pytest.mark.parametrize("batch", [1, 2, 3, 1001, 4737])
-def test_batched32_pipelined_variant_is_bitwise_identical(ctx, batch):
-    """Variant 13 (R phase of pair n+1 interleaved with the Q phase of pair n, persistent warps) performs the same
-    operations in the same order as the one-shot kernel with the same scalar chain (variant 6): identical bits, ragged
-    tails included."""
-    A = np.random.default_rng(500 + batch).standard_normal((batch, 32, 32))
-    if batch > 16:
-        A[3, :, 5] = 0.0           # skipped reflector (qr.py:79)
-        A[7, :, 9] = A[7, :, 2]    # dependent column
-    dA = ctx.upload(A)
-    out = {}
-    for v in (6, 13):
-        dQ, dR = ctx.upload(np.full_like(A, np.nan)), ctx.upload(np.full_like(A, np.nan))
-        _call_variant(ctx, dA, batch, dQ, dR, v)
-        out[v] = (ctx.download(dQ, A.shape), ctx.download(dR, A.shape))
-    assert np.array_equal(out[6][0], out[13][0]) and np.array_equal(out[6][1], out[13][1])
-    Qo, Ro = orc.householder_qr_batched(A[: min(batch, 32)])
-    assert orc.rel_max_err(out[13][0][: len(Qo)], Qo) <= REL and orc.rel_max_err(out[13][1][: len(Ro)], Ro) <= REL
-
-
+# ------------------------------------------------------------------ batched 32 x 32 Householder kernel
 @pytest.mark.parametrize("batch", [1, 5, 31, 33, 1000, 4099])
-def test_batched32_round2_kernels_agree(ctx, batch):
-    """The round-2 kernels of a1 at 32 x 32 -- the default (variant 0: lane = column, left-looking panels, Q formed by
-    compact-WY block reflectors on DMMA.8x8x4), the two-stage left-looking kernel (36) and the round-1 R phase with the
-    DMMA Q phase (21) -- against the reference semantics (oracle, 1e-10) and against the round-1 kernel (14), with ragged
-    tails, a skipped reflector (qr.py:79: zero column), a dependent column and a badly scaled matrix."""
+def test_batched32_householder_kernel_matches_oracle(ctx, batch):
+    """The 32 x 32 kernel of a1 (lane = column, left-looking panels, Q formed by compact-WY block reflectors on
+    DMMA.8x8x4) against the reference semantics (oracle, 1e-10) and the QR invariants over the whole batch, with ragged
+    tails, a skipped reflector (qr.py:79: zero column), a dependent column and a badly scaled matrix.  It is the only
+    kernel variant: any other variant number is an argument error."""
     rng = np.random.default_rng(900 + batch)
     A = rng.standard_normal((batch, 32, 32))
     if batch > 16:
@@ -544,30 +510,26 @@ def test_batched32_round2_kernels_agree(ctx, batch):
         A[13, :, 0] = 0.0           # first column skipped
         A[14, :, 31] = 0.0          # last column skipped
     dA = ctx.upload(A)
-    out = {}
-    for v in (14, 0, 36, 21, 52):
-        dQ, dR = ctx.upload(np.full_like(A, np.nan)), ctx.upload(np.full_like(A, np.nan))
-        if not _call_variant(ctx, dA, batch, dQ, dR, v, required=v in (0, 14)):
-            continue
-        out[v] = (ctx.download(dQ, A.shape), ctx.download(dR, A.shape))
-        Qv, Rv = out[v]
-        assert np.isfinite(Qv).all() and np.isfinite(Rv).all(), v
-        assert np.all(np.tril(Rv, -1) == 0.0), v
+    dQ, dR = ctx.upload(np.full_like(A, np.nan)), ctx.upload(np.full_like(A, np.nan))
+    with pytest.raises(ValueError, match="variant 14 does not exist"):
+        ctx.call("lq_householder_qr_batched_dev", dA.ptr, batch, 32, 32, dQ.ptr, dR.ptr, 14)
+    ctx.call("lq_householder_qr_batched_dev", dA.ptr, batch, 32, 32, dQ.ptr, dR.ptr, 0)
+    Qv, Rv = ctx.download(dQ, A.shape), ctx.download(dR, A.shape)
+    assert np.isfinite(Qv).all() and np.isfinite(Rv).all()
+    assert np.all(np.tril(Rv, -1) == 0.0)
     nref = min(batch, 48)
     Qo, Ro = orc.householder_qr_batched(A[:nref])
-    for v, (Qv, Rv) in out.items():
-        for i in range(nref):
-            if batch > 16 and i == 7:
-                # dependent column: the reflector of column 9 is built from rounding noise, Q is not unique there;
-                # the invariants still hold
-                assert orc.qr_residual(A[i], Qv[i], Rv[i]) <= 1e-12 and orc.orth_error(Qv[i]) <= 1e-12, (v, i)
-                continue
-            assert orc.rel_max_err(Qv[i], Qo[i]) <= REL and orc.rel_max_err(Rv[i], Ro[i]) <= REL, (v, i)
-    # every matrix of the batch: invariants, and agreement with the round-1 kernel
-    for v, (Qv, Rv) in out.items():
-        resid = np.linalg.norm(A - Qv @ Rv, axis=(1, 2)) / np.linalg.norm(A, axis=(1, 2))
-        orth = np.abs(np.swapaxes(Qv, 1, 2) @ Qv - np.eye(32)).max(axis=(1, 2))
-        assert resid.max() <= 1e-12 and orth.max() <= 1e-12, (v, resid.max(), orth.max())
+    for i in range(nref):
+        if batch > 16 and i == 7:
+            # dependent column: the reflector of column 9 is built from rounding noise, Q is not unique there;
+            # the invariants still hold
+            assert orc.qr_residual(A[i], Qv[i], Rv[i]) <= 1e-12 and orc.orth_error(Qv[i]) <= 1e-12, i
+            continue
+        assert orc.rel_max_err(Qv[i], Qo[i]) <= REL and orc.rel_max_err(Rv[i], Ro[i]) <= REL, i
+    # every matrix of the batch: invariants
+    resid = np.linalg.norm(A - Qv @ Rv, axis=(1, 2)) / np.linalg.norm(A, axis=(1, 2))
+    orth = np.abs(np.swapaxes(Qv, 1, 2) @ Qv - np.eye(32)).max(axis=(1, 2))
+    assert resid.max() <= 1e-12 and orth.max() <= 1e-12, (resid.max(), orth.max())
 
 
 @pytest.mark.parametrize("m", [33, 64, 300, 1000, 4096, 8192])

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""First GPU bring-up: probes + batched 32x32 variants + small kernels vs the oracle.
+"""First GPU bring-up: probes + batched 32x32 kernels + small kernels vs the oracle.
 
 Run on the GPU box:  python tools/gpu_check1.py > gpurun_out/check1.log 2>&1
 """
@@ -47,7 +47,7 @@ guarded(probes)
 
 # ------------------------------------------------------------------ batched 32x32 correctness
 def hh32_correct():
-    section("hh32 correctness per variant")
+    section("hh32 correctness")
     nb = 1000  # not a multiple of the per-block matrix count -> exercises the tail
     A = np.random.default_rng(2).standard_normal((nb, 32, 32))
     A[5, :, 7] = 0.0  # zero column -> skip branch
@@ -56,26 +56,19 @@ def hh32_correct():
     dA = ctx.upload(A)
     dQ = ctx.alloc(A.nbytes)
     dR = ctx.alloc(A.nbytes)
-    res = {}
-    for variant in range(0, 10):
-        try:
-            ctx.call("lq_memset", dQ.ptr, 0xFF, A.nbytes)
-            ctx.call("lq_memset", dR.ptr, 0xFF, A.nbytes)
-            ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, variant)
-            ctx.sync()
-            Q = ctx.download(dQ, A.shape)
-            R = ctx.download(dR, A.shape)
-            eq = orc.rel_max_err(Q[:64], Qo)
-            er = orc.rel_max_err(R[:64], Ro)
-            resid = max(orc.qr_residual(A[i], Q[i], R[i]) for i in range(nb))
-            orth = orc.orth_error(Q)
-            low = float(np.max(np.abs(np.tril(R, -1))))
-            res[variant] = dict(q=eq, r=er, resid=resid, orth=orth, lower=low)
-            print(variant, res[variant], flush=True)
-        except Exception as e:  # noqa: BLE001
-            print(variant, "FAILED", repr(e), flush=True)
-            res[variant] = repr(e)
-    out["hh32_correct"] = res
+    ctx.call("lq_memset", dQ.ptr, 0xFF, A.nbytes)
+    ctx.call("lq_memset", dR.ptr, 0xFF, A.nbytes)
+    ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, 0)
+    ctx.sync()
+    Q = ctx.download(dQ, A.shape)
+    R = ctx.download(dR, A.shape)
+    eq = orc.rel_max_err(Q[:64], Qo)
+    er = orc.rel_max_err(R[:64], Ro)
+    resid = max(orc.qr_residual(A[i], Q[i], R[i]) for i in range(nb))
+    orth = orc.orth_error(Q)
+    low = float(np.max(np.abs(np.tril(R, -1))))
+    out["hh32_correct"] = dict(q=eq, r=er, resid=resid, orth=orth, lower=low)
+    print(out["hh32_correct"], flush=True)
 
 
 guarded(hh32_correct)
@@ -182,24 +175,6 @@ def hh32_time():
     dQ = ctx.alloc(A.nbytes)
     dR = ctx.alloc(A.nbytes)
     dI = ctx.alloc(nb * 4)
-    res = {}
-    for variant in list(range(1, 10)):
-        try:
-            for _ in range(2):
-                ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, variant)
-            ctx.sync()
-            ts = []
-            for _ in range(5):
-                ctx.record(0)
-                ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, variant)
-                ctx.record(1)
-                ts.append(ctx.elapsed_ms(0, 1))
-            t = min(ts)
-            res[variant] = dict(ms=t, mat_per_s=nb / t * 1e3, gbs=nb * 24576 / t / 1e6)
-            print("variant", variant, res[variant], flush=True)
-        except Exception as e:  # noqa: BLE001
-            print("variant", variant, "FAILED", repr(e), flush=True)
-    out["hh32_time"] = res
     for reorth in (0, 1):
         for _ in range(2):
             ctx.call("lq_mgs_qr_batched_dev", dA.ptr, nb, 32, 32, reorth, dQ.ptr, dR.ptr, dI.ptr)

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""GPU bring-up 2: probes, GEMM, blocked Householder QR, batched variants re-timed."""
+"""GPU bring-up 2: probes, GEMM, blocked Householder QR."""
 import json
 import os
 import sys
@@ -14,7 +14,7 @@ from oracle import linalg_oracle as orc  # noqa: E402
 
 out = {}
 ctx = nat.Context(0)
-what = set(sys.argv[1:]) or {"probes", "gemm", "blocked", "hh32"}
+what = set(sys.argv[1:]) or {"probes", "gemm", "blocked"}
 
 
 def section(name):
@@ -143,38 +143,7 @@ def blocked():
             print("8192 resid", orc.qr_residual(A, Q, R), "orth", orc.orth_error(Q[:, :512]), flush=True)
 
 
-def hh32():
-    section("hh32 timing (2^18 matrices)")
-    nb = 1 << 18
-    A = np.random.default_rng(2).standard_normal((nb, 32, 32))
-    dA = ctx.upload(A)
-    dQ = ctx.alloc(A.nbytes)
-    dR = ctx.alloc(A.nbytes)
-    Qo, Ro = orc.householder_qr_batched(A[:32])
-    res = {}
-    for variant in range(1, 13):
-        try:
-            for _ in range(2):
-                ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, variant)
-            ctx.sync()
-            ts = []
-            for _ in range(5):
-                ctx.record(0)
-                ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, variant)
-                ctx.record(1)
-                ts.append(ctx.elapsed_ms(0, 1))
-            t = min(ts)
-            Q = ctx.download(dQ, (32, 32, 32))
-            R = ctx.download(dR, (32, 32, 32))
-            res[variant] = dict(ms=t, mat_per_s=nb / t * 1e3, gbs=nb * 24576 / t / 1e6, q=orc.rel_max_err(Q, Qo),
-                                r=orc.rel_max_err(R, Ro), orth=orc.orth_error(Q))
-            print("variant", variant, res[variant], flush=True)
-        except Exception as e:  # noqa: BLE001
-            print("variant", variant, "FAILED", repr(e), flush=True)
-    out["hh32_time"] = res
-
-
-for name in ("probes", "gemm", "blocked", "hh32"):
+for name in ("probes", "gemm", "blocked"):
     if name in what:
         guarded(globals()[name])
 

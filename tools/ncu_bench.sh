@@ -1,7 +1,7 @@
 #!/bin/bash
 # usage: tools/ncu_bench.sh <tag> [kernel-regex]
 # Launch list (per-launch gpu time) of a short bench.py run + one --set full capture of the top kernel.
-TAG=${1:-r1}; KREGEX=${2:-hh_qr32_kernel}
+TAG=${1:-r1}; KREGEX=${2:-hh_qr32_c8_kernel}
 CMD="python bench.py --steps 3 --warmup 3 --no-cpu --no-extras --e2e-steps 1"
 mkdir -p gpurun_out
 $CMD > gpurun_out/${TAG}_plain.log 2>&1 || { echo "plain run failed"; tail gpurun_out/${TAG}_plain.log; exit 1; }

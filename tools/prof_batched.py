@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Tiny driver for ncu: run the batched 32x32 kernels a few times on device-resident data.
 
-usage: python tools/prof_batched.py [log2_batch=16] [variants=0] [mgs=0]
+usage: python tools/prof_batched.py [log2_batch=16] [mgs=0]
 """
 import os
 import sys
@@ -12,8 +12,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from linalg_b200 import _native as nat  # noqa: E402
 
 lg = int(sys.argv[1]) if len(sys.argv) > 1 else 16
-variants = [int(v) for v in (sys.argv[2] if len(sys.argv) > 2 else "0").split(",")]
-mgs = int(sys.argv[3]) if len(sys.argv) > 3 else 0
+mgs = int(sys.argv[2]) if len(sys.argv) > 2 else 0
 reps = int(os.environ.get('PROF_REPS', '3'))
 nb = 1 << lg
 ctx = nat.Context(0)
@@ -22,13 +21,12 @@ dA = ctx.upload(A)
 dQ = ctx.alloc(A.nbytes)
 dR = ctx.alloc(A.nbytes)
 dI = ctx.alloc(nb * 4)
-for v in variants:
-    for _ in range(reps):
-        ctx.record(0)
-        ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, v)
-        ctx.record(1)
-        ms = ctx.elapsed_ms(0, 1)
-    print(f"variant {v}: {ms:.3f} ms  {nb/ms/1e3:.1f} M mat/s")
+for _ in range(reps):
+    ctx.record(0)
+    ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, 0)
+    ctx.record(1)
+    ms = ctx.elapsed_ms(0, 1)
+print(f"householder: {ms:.3f} ms  {nb/ms/1e3:.1f} M mat/s")
 if mgs:
     for _ in range(reps):
         ctx.record(0)

@@ -30,8 +30,6 @@ nb = 40003
 A = rng.standard_normal((nb, 32, 32)); dA = ctx.upload(A); dQ, dR, dI = ctx.alloc(A.nbytes), ctx.alloc(A.nbytes), ctx.alloc(4 * nb)
 soak("householder_qr_batched 32x32 (c8 kernel)", lambda: ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, 0),
      [(dQ, (nb, 32, 32), np.float64), (dR, (nb, 32, 32), np.float64)])
-soak("householder_qr_batched 32x32 (round-1 kernel)", lambda: ctx.call("lq_householder_qr_batched_dev", dA.ptr, nb, 32, 32, dQ.ptr, dR.ptr, 14),
-     [(dQ, (nb, 32, 32), np.float64), (dR, (nb, 32, 32), np.float64)])
 for re in (0, 1):
     soak(f"qr_batched 32x32 (MGS, reorth={re})", lambda: ctx.call("lq_mgs_qr_batched_dev", dA.ptr, nb, 32, 32, re, dQ.ptr, dR.ptr, dI.ptr),
          [(dQ, (nb, 32, 32), np.float64), (dR, (nb, 32, 32), np.float64), (dI, (nb,), np.int32)])
