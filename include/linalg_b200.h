@@ -58,8 +58,8 @@ int lq_flush_l2(lq_ctx* ctx);        /* overwrite a 256 MiB scratch buffer (> 12
 int64_t lq_kernel_launches(lq_ctx* ctx); /* number of this library's kernels launched so far */
 
 /* diagnostics: kernel-selection switches of one context.  name is the LINALG_B200_<NAME> environment variable without
- * its prefix ("TSQR_HOUSEHOLDER", "JACOBI_TWO_SIDED", "OLD_CHOL"); the environment only gives the initial value at
- * lq_create, hot entry points never call getenv. */
+ * its prefix ("TSQR_HOUSEHOLDER", "JACOBI_TWO_SIDED"); any other name returns LQ_ERR_ARG.  The environment only gives
+ * the initial value at lq_create, hot entry points never call getenv. */
 int lq_set_option(lq_ctx* ctx, const char* name, int value);
 
 /* ---- a1: householder_qr  (linalg/qr.py:52-100) ------------------------------------------- */
@@ -152,7 +152,7 @@ int lq_svd_gram_sharded_dev(lq_ctx* ctx, const double* A_local, int64_t m_local,
  * Newton-refined rcp / rsqrt / sqrt used by the kernels [max relative error]. */
 int lq_probe(lq_ctx* ctx, int kind, double* result);
 /* diagnostics: one 32-column panel factorisation of the blocked path with an explicit kernel version
- * (0 default, 1 barrier.cluster kernel, 2 / 3 st.async kernels with 512 / 256 rows per CTA) */
+ * (0 default, 1 barrier.cluster kernel, 3 st.async kernel with 256 rows per CTA); any other version returns LQ_ERR_ARG */
 int lq_debug_panel(lq_ctx* ctx, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, int nb, int version);
 /* the same with clock64() stamps of the column-step phases: trace[2 warps][32 columns][8 phases] (device pointer) */
 int lq_debug_panel_trace(lq_ctx* ctx, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, long long* trace);

@@ -180,7 +180,7 @@ class Context:
         check(self.lib, self.handle, rc, name)
 
     def set_option(self, name: str, value: bool):
-        """Diagnostic kernel-selection switch (``TSQR_HOUSEHOLDER``, ``JACOBI_TWO_SIDED``, ``OLD_CHOL``)."""
+        """Diagnostic kernel-selection switch (``TSQR_HOUSEHOLDER`` or ``JACOBI_TWO_SIDED``); any other name raises ValueError."""
         self.call("lq_set_option", name.encode(), int(bool(value)))
 
     def props(self):

@@ -228,7 +228,6 @@ int lq_create(int device, lq_ctx** out) {
     LQ_CUDA(c, cudaDeviceGetDefaultMemPool(&pool, device));
     unsigned long long thr = ~0ull;
     LQ_CUDA(c, cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
-    c->env_old_chol = getenv("LINALG_B200_OLD_CHOL") != nullptr;
     c->env_tsqr_householder = getenv("LINALG_B200_TSQR_HOUSEHOLDER") != nullptr;
     c->env_jacobi_two_sided = getenv("LINALG_B200_JACOBI_TWO_SIDED") != nullptr;
     c->env_no_graph = getenv("LINALG_B200_NO_GRAPH") != nullptr;
@@ -260,8 +259,7 @@ int lq_set_option(lq_ctx* h, const char* name, int value) {
     Ctx* c = as_ctx(h);
     if (!c || !name) return LQ_ERR_ARG;
     const std::string n(name);
-    if (n == "OLD_CHOL") c->env_old_chol = value != 0;
-    else if (n == "TSQR_HOUSEHOLDER") c->env_tsqr_householder = value != 0;
+    if (n == "TSQR_HOUSEHOLDER") c->env_tsqr_householder = value != 0;
     else if (n == "JACOBI_TWO_SIDED") c->env_jacobi_two_sided = value != 0;
     else {
         set_error(c, "lq_set_option: unknown option '%s'", name);

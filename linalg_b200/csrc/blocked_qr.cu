@@ -264,7 +264,6 @@ int detect_max_cluster(Ctx* c) {
         }
         cudaGetLastError();
     }
-    if (const char* env = getenv("LINALG_B200_MAX_CLUSTER")) best = std::max(1, std::min(best, atoi(env)));
     cached[c->device] = best;
     c->max_cluster = best;
     return best;
@@ -289,42 +288,31 @@ int launch_cluster(Ctx* c, Kern kern, int cs, int threads, Args... args) {
     return LQ_OK;
 }
 
-// version: 0 = default choice (panels of up to 256 rows: the one-CTA SOLO kernel), 1 = barrier.cluster kernel (panel.cuh), 2 = st.async kernel (panel2.cuh), 16 rows per lane,
-// 3 = st.async kernel with 8 rows per lane (256 rows per CTA), 4 = st.async kernels for every height (256 rows per CTA up to
-// 4096 rows, 512 above)
+// version: 0 = default choice (panels of up to 256 rows: the one-CTA SOLO kernel), 1 = barrier.cluster kernel (panel.cuh),
+// 3 = st.async kernel (panel2.cuh) with 8 rows per lane (256 rows per CTA) wherever a cluster of it holds the panel
 int panel_factor_v(Ctx* c, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, int nb, int version) {
     using Cfg = PanelCfg<4, 16>;
     const int maxcs = detect_max_cluster(c);
-    if (version == 0) {
-        static const int env_version = getenv("LINALG_B200_PANEL") ? atoi(getenv("LINALG_B200_PANEL")) : 0;
-        version = env_version;
-    }
     if (nb == P2_NB && version != 1) {
         static bool attr_done[64] = {};
         if (!attr_done[c->device]) {
-            cudaFuncSetAttribute(panel2_cluster_kernel<16, false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
             cudaFuncSetAttribute(panel2_cluster_kernel<8, false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
             attr_done[c->device] = true;
         }
         // default: the 256-rows-per-CTA kernel whenever the panel fits a cluster of it (half the FP64 work per SM and
         // column); taller panels run next to the side stream's big GEMMs, where the barrier.cluster kernel measured
-        // better in situ (tools/blocked_trace.py), although the 512-row st.async kernel wins stand-alone
-        if (version == 0 && mp <= Panel2Cfg<8>::ROWS_PER_CTA && !LQ_ENV_ONCE("LINALG_B200_NO_SOLO_PANEL")) {
+        // better in situ (tools/blocked_trace.py) than a 512-row st.async kernel, although that one won stand-alone
+        if (version == 0 && mp <= Panel2Cfg<8>::ROWS_PER_CTA) {
             // one CTA, no cluster exchange: ~17 us instead of 48 us per panel of up to 256 rows
             panel2_cluster_kernel<8, false, true><<<1, P2_THREADS, 0, c->stream>>>(A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
             LQ_CHECK_LAUNCH(c);
             LQ_COUNT_LAUNCH(c);
             return LQ_OK;
         }
-        if (version != 2 && mp <= maxcs * Panel2Cfg<8>::ROWS_PER_CTA) {
+        if (mp <= maxcs * Panel2Cfg<8>::ROWS_PER_CTA) {
             int cs = 1;
             while (cs * Panel2Cfg<8>::ROWS_PER_CTA < mp) cs *= 2;
             return launch_cluster(c, panel2_cluster_kernel<8, false>, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
-        }
-        if ((version == 2 || version == 4) && mp <= maxcs * Panel2Cfg<16>::ROWS_PER_CTA) {
-            int cs = 1;
-            while (cs * Panel2Cfg<16>::ROWS_PER_CTA < mp) cs *= 2;
-            return launch_cluster(c, panel2_cluster_kernel<16, false>, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
         }
     }
     int cs = 1;
@@ -344,9 +332,8 @@ inline int grid_for(Ctx* c, long long total) {
 // apply the block reflector  C <- (I - V op(T) V^T) C   to C (mk x nc, ldc); V (mk x kb, ldv); T (kb x kb, ldt)
 // trans_t = true -> T^T (factorisation order H_kb ... H_1), false -> T (Q formation order H_1 ... H_kb)
 int apply_block_reflector(Ctx* c, const double* V, int ldv, const double* T, int ldt, bool trans_t, int mk, int kb,
-                          double* Cm, int ldc, int nc, double* W, double* W2) {
+                          double* Cm, int ldc, int nc, double* W2) {
     if (nc <= 0 || kb <= 0 || mk <= 0) return LQ_OK;
-    (void)W;
     LQ_TRY(gemm_vtc_apply_t(c, kb, nc, mk, V, ldv, Cm, ldc, T, ldt, trans_t, W2));         // W2 = op(T) (V^T C)
     LQ_TRY(gemm(c, false, false, mk, nc, kb, -1.0, V, ldv, W2, nc, 1.0, Cm, ldc));         // C -= V W2
     return LQ_OK;
@@ -390,22 +377,18 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
                   int nrhs_pad, Factored* keep) {
     const int nblocks = (nfac + NB_OUT - 1) / NB_OUT;
     cudaStream_t s_main = c->stream, s_side = c->lane[0], s_aux = c->lane[1], s_merge = c->lane[2], s_side2 = c->lane[3];
-    const bool lookahead = (!LQ_ENV_ONCE("LINALG_B200_NO_LOOKAHEAD")) && nblocks > 1;
+    const bool lookahead = nblocks > 1;
     // Gram scratch of the T merge: one buffer per stream that may run a merge (main: blocks without panel-wise look-ahead,
     // e.g. the last one; merge stream: all the others) -- the two streams are not ordered against each other
-    DevBuf Tloc, G, Gmerge, W, W2, Ws, W2s, W2s2;
+    DevBuf Tloc, G, Gmerge, W2, W2s, W2s2;
     LQ_TRY(G.alloc(c, sizeof(double) * NB_OUT * NB_OUT));
     LQ_TRY(Gmerge.alloc(c, sizeof(double) * NB_OUT * NB_OUT));
     const int wcols = std::max(npad, nrhs_pad);
-    LQ_TRY(W.alloc(c, sizeof(double) * NB_OUT * (size_t)wcols));
     LQ_TRY(W2.alloc(c, sizeof(double) * NB_OUT * (size_t)wcols));
-    DevBuf Wa, W2a;  // scratch of the aux stream (panel-wise application to the next outer block)
-    const bool pw_lookahead = !LQ_ENV_ONCE("LINALG_B200_NO_PANELWISE");
+    DevBuf W2a;  // scratch of the aux stream (panel-wise application to the next outer block)
     if (lookahead) {
-        LQ_TRY(Ws.alloc(c, sizeof(double) * NB_OUT * (size_t)wcols));
         LQ_TRY(W2s.alloc(c, sizeof(double) * NB_OUT * (size_t)wcols));
         LQ_TRY(W2s2.alloc(c, sizeof(double) * NB_OUT * (size_t)wcols));
-        LQ_TRY(Wa.alloc(c, sizeof(double) * NB_IN * (size_t)NB_OUT));
         LQ_TRY(W2a.alloc(c, sizeof(double) * NB_IN * (size_t)NB_OUT));
     }
     double* Tall;
@@ -460,7 +443,7 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
         // block on the aux stream as soon as the panel exists, in the shadow of the following panels, so the chain
         // never waits for the Gram matrix / T merge of the whole block (they move to the side stream, where only the
         // big trailing update and the Q formation need the merged T)
-        const bool pw = lookahead && pw_lookahead && nnext > 0 && nin > 1;
+        const bool pw = lookahead && nnext > 0 && nin > 1;
         cudaEvent_t ev_aux_done = nullptr;
         for (int ip = 0; ip < nin; ++ip) {
             const int c0 = k0 + ip * NB_IN;
@@ -479,7 +462,7 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
                 LQ_CUDA(c, cudaStreamWaitEvent(s_aux, ev_p, 0));
                 if (ip == 0 && ev_rest_prev) LQ_CUDA(c, cudaStreamWaitEvent(s_aux, ev_rest_prev, 0));  // block b+1's columns were in rest(b-1)
                 LQ_TRY(apply_block_reflector(c, Vp, ldv, Tp, ldtp, true, mp, NB_IN, A + (size_t)c0 * lda + k0 + kb, lda, nnext,
-                                             Wa.as<double>(), W2a.as<double>()));
+                                             W2a.as<double>()));
                 if (ip == nin - 1) {
                     LQ_TRY(pool.make(c, &ev_aux_done));
                     LQ_CUDA(c, cudaEventRecord(ev_aux_done, s_aux));
@@ -488,7 +471,7 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
             const int nrem = k0 + kb - (c0 + NB_IN);
             if (nrem > 0)
                 LQ_TRY(apply_block_reflector(c, Vp, ldv, Tp, ldtp, true, mp, NB_IN, Ap + NB_IN, lda, nrem,
-                                             W.as<double>(), W2.as<double>()));
+                                             W2.as<double>()));
         }
         if (trace_blocks) {
             LQ_TRY(pool.make(c, &btrace[blk].panels));
@@ -508,11 +491,10 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
         if (!lookahead) {
             LQ_TRY(merge_block_t(G.as<double>()));
             if (ntr > 0)
-                LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, Ctr, lda, ntr, W.as<double>(),
-                                             W2.as<double>()));
+                LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, Ctr, lda, ntr, W2.as<double>()));
             if (B && nrhs_pad > 0)
                 LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, B + (size_t)k0 * ldb, ldb, nrhs_pad,
-                                             W.as<double>(), W2.as<double>()));
+                                             W2.as<double>()));
             continue;
         }
         cudaEvent_t ev_panel;
@@ -526,8 +508,7 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
             LQ_TRY(merge_block_t(G.as<double>()));
             if (nnext > 0) {
                 if (ev_rest_prev) LQ_CUDA(c, cudaStreamWaitEvent(s_main, ev_rest_prev, 0));
-                LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, Ctr, lda, nnext, W.as<double>(),
-                                             W2.as<double>()));
+                LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, Ctr, lda, nnext, W2.as<double>()));
             }
         }
         if (trace_blocks) {
@@ -554,7 +535,7 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
                 StreamScope side(c, s_side);  // columns [c_lo, c_mid)
                 LQ_CUDA(c, cudaStreamWaitEvent(s_side, ev_after, 0));
                 LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, A + (size_t)k0 * lda + c_lo, lda, c_mid - c_lo,
-                                             Ws.as<double>(), W2s.as<double>()));
+                                             W2s.as<double>()));
                 LQ_TRY(pool.make(c, &ev_left));
                 LQ_CUDA(c, cudaEventRecord(ev_left, s_side));
                 ev_rest_last[0] = ev_left;
@@ -564,10 +545,10 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
                 LQ_CUDA(c, cudaStreamWaitEvent(s_side2, ev_after, 0));
                 if (npad > c_mid)
                     LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, A + (size_t)k0 * lda + c_mid, lda, npad - c_mid,
-                                                 Ws.as<double>(), W2s2.as<double>()));
+                                                 W2s2.as<double>()));
                 if (B && nrhs_pad > 0)
                     LQ_TRY(apply_block_reflector(c, Vb, ldv, Tblk, NB_OUT, true, mk, kb, B + (size_t)k0 * ldb, ldb, nrhs_pad,
-                                                 Ws.as<double>(), W2s2.as<double>()));
+                                                 W2s2.as<double>()));
                 LQ_TRY(pool.make(c, &ev_right));
                 LQ_CUDA(c, cudaEventRecord(ev_right, s_side2));
                 ev_rest_last[1] = ev_right;
@@ -711,7 +692,7 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
         Qp = Qw.as<double>();
         ldq = npad;
     }
-    // the A workspace is free now: reuse it for W / W2
+    // the A workspace is free now: reuse it for the scratch of the main stream (W2) and of the side stream (W)
     double* W = Aw.as<double>();
     double* W2 = W + (size_t)NB_OUT * npad;
     const bool ws_fits = (size_t)m * npad >= 2 * (size_t)NB_OUT * npad;
@@ -724,12 +705,11 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
     set_identity_kernel<<<grid_for(c, (long long)m * ldq), 256, 0, c->stream>>>(Qp, ldq, m, ldq);
     LQ_CHECK_LAUNCH(c);
     LQ_COUNT_LAUNCH(c);
-    const bool skip_q = LQ_ENV_ONCE("LINALG_B200_DEBUG_SKIP_Q");  // timing experiments only (Q = I)
     // A block reflector transforms every COLUMN of Q independently, so the columns are split into two contiguous
     // ranges that run the whole chain of applications on two streams with no synchronisation in between: the launch
     // gaps, split-K reductions and partial last waves of one range are filled by the other.  The split balances the
     // flops (block b touches the columns >= 128 b only): 3 s^2 - s^3 = 1  ->  s = 0.65.
-    const bool two_ranges = ldq >= 2048 && ws_fits && !LQ_ENV_ONCE("LINALG_B200_NO_LOOKAHEAD");
+    const bool two_ranges = ldq >= 2048 && ws_fits;
     const int split = two_ranges ? (int)(0.65 * ldq) / NB_OUT * NB_OUT : 0;
     cudaStream_t s_main = c->stream, s_side = c->lane[0];
     EventPool qpool;
@@ -739,7 +719,7 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
         LQ_CUDA(c, cudaEventRecord(e0, s_main));
         LQ_CUDA(c, cudaStreamWaitEvent(s_side, e0, 0));
     }
-    for (int blk = keep.nblocks - 1; blk >= 0 && !skip_q; --blk) {
+    for (int blk = keep.nblocks - 1; blk >= 0; --blk) {
         const int k0 = blk * NB_OUT;
         const int kb = std::min(NB_OUT, npad - k0);
         const int mk = m - k0;
@@ -748,10 +728,10 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
         const double* Tblk = keep.Tall.as<double>() + (size_t)blk * NB_OUT * NB_OUT;
         // only columns >= k0 of Q are touched by this block (Q[k0:, :k0] is still zero)
         const int c_hi = std::max(k0, split);  // main stream: columns [c_hi, ldq); side stream: [k0, split)
-        LQ_TRY(apply_block_reflector(c, Vb, npad, Tblk, NB_OUT, false, mk, kb, Qp + (size_t)k0 * ldq + c_hi, ldq, ldq - c_hi, W, W2));
+        LQ_TRY(apply_block_reflector(c, Vb, npad, Tblk, NB_OUT, false, mk, kb, Qp + (size_t)k0 * ldq + c_hi, ldq, ldq - c_hi, W2));
         if (k0 < split) {
             StreamScope side(c, s_side);
-            LQ_TRY(apply_block_reflector(c, Vb, npad, Tblk, NB_OUT, false, mk, kb, Qp + (size_t)k0 * ldq + k0, ldq, split - k0, W, W));
+            LQ_TRY(apply_block_reflector(c, Vb, npad, Tblk, NB_OUT, false, mk, kb, Qp + (size_t)k0 * ldq + k0, ldq, split - k0, W));
         }
     }
     if (two_ranges) {
@@ -800,6 +780,8 @@ extern "C" {
 int lq_debug_panel(lq_ctx* h, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, int nb, int version) {
     Ctx* c = as_ctx(h);
     if (!c) return LQ_ERR_ARG;
+    LQ_REQUIRE(c, version == 0 || version == 1 || version == 3, LQ_ERR_ARG,
+               "debug_panel: panel kernel version %d does not exist (0, 1 and 3 do)", version);
     LQ_CUDA(c, cudaSetDevice(c->device));
     return panel_factor_v(c, A, lda, V, ldv, T, ldt, mp, nb, version);
 }
@@ -811,7 +793,7 @@ int lq_debug_panel_trace(lq_ctx* h, double* A, int lda, double* V, int ldv, doub
     LQ_CUDA(c, cudaSetDevice(c->device));
     const int maxcs = detect_max_cluster(c);
     LQ_REQUIRE(c, mp <= maxcs * Panel2Cfg<8>::ROWS_PER_CTA, LQ_ERR_SHAPE, "panel too tall for the traced kernel");
-    if (mp <= Panel2Cfg<8>::ROWS_PER_CTA && !LQ_ENV_ONCE("LINALG_B200_NO_SOLO_PANEL")) {  // the one-CTA kernel's stamps
+    if (mp <= Panel2Cfg<8>::ROWS_PER_CTA) {  // the one-CTA kernel's stamps
         panel2_cluster_kernel<8, true, true><<<1, P2_THREADS, 0, c->stream>>>(A, lda, V, ldv, T, ldt, mp, trace);
         LQ_CHECK_LAUNCH(c);
         return LQ_OK;

@@ -33,7 +33,7 @@ struct Ctx : lq_ctx {
     int nranks = 1, rank = 0;
     // diagnostic kernel-selection switches: initialised from LINALG_B200_<NAME> when the context is created, changed with
     // lq_set_option (never read from the environment on a hot entry point)
-    bool env_old_chol = false, env_tsqr_householder = false, env_jacobi_two_sided = false;
+    bool env_tsqr_householder = false, env_jacobi_two_sided = false;
     // CUDA-graph replay of the blocked QR schedule for small single matrices (launch-latency bound: 52 launches over five
     // streams at 256^2).  Keyed by shape and the caller's device pointers; state 0 = seen once (warm-up call, runs the
     // plain path so that every per-kernel attribute latch is set outside a capture), 1 = graph ready, -1 = not capturable.

@@ -572,12 +572,10 @@ __global__ void __launch_bounds__(1024) reduce_apply_t_kernel(const double* __re
 // C = alpha * A * B + beta * C  (NN) where the contraction is short (the 128 reflectors of a block update
 // C -= V W, or U = A (V S^-1), Q = A R^-1 on tall-skinny matrices).  With K = 128 a 128 x 128 output tile has only
 // 8 k-tiles, so the generic kernel spends a third of each CTA's life filling its pipeline and reading C.  Here a
-// persistent CTA keeps ONE operand tile resident in shared memory for its whole life and walks along the other
-// dimension: ASTAT = the A row tile (128 x K, eight swizzled TMA boxes) stays and the B / C column tiles stream
-// (block updates); !ASTAT = the B column tile (K x 128) stays and the A / C row tiles stream (tall-skinny).  The
-// producer warp runs ahead across tile boundaries, so the next tile's operands land during the current epilogue.
+// persistent CTA keeps the B column tile (K x 128) resident in shared memory for its whole life and walks down the
+// A / C row tiles (tall-skinny products).  The producer warp runs ahead across tile boundaries, so the next tile's
+// operands land during the current epilogue.
 constexpr int RK_KT_MAX = 8;  // K <= 128
-constexpr size_t RK_SMEM_ASTAT = (size_t)RK_KT_MAX * BM * BK * 8 + (size_t)STAGES * TILE_BYTES + 16 * sizeof(uint64_t) + 1024;
 constexpr size_t RK_SMEM_BSTAT = (size_t)RK_KT_MAX * TILE_BYTES + (size_t)STAGES * BM * BK * 8 + 16 * sizeof(uint64_t) + 1024;
 
 struct RankArgs {
@@ -589,15 +587,14 @@ struct RankArgs {
     double alpha, beta;
 };
 
-template <bool ASTAT>
 __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankArgs g, const __grid_constant__ CUtensorMap mapA) {
     extern __shared__ unsigned char smem_dyn[];
     unsigned char* smem_raw = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
     constexpr int ABOX = BM * BK;  // doubles per swizzled A box
-    // layout: [resident operand][streamed ring][barriers]
+    // layout: [resident B tile][streamed A ring][barriers]
     double* res = reinterpret_cast<double*>(smem_raw);
-    double* ring = res + (ASTAT ? RK_KT_MAX * ABOX : RK_KT_MAX * TILE_DOUBLES);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(ring + (ASTAT ? STAGES * TILE_DOUBLES : STAGES * ABOX));
+    double* ring = res + RK_KT_MAX * TILE_DOUBLES;
+    uint64_t* bars = reinterpret_cast<uint64_t*>(ring + STAGES * ABOX);
     uint64_t* full = bars;
     uint64_t* empty = bars + STAGES;
     uint64_t* res_full = bars + 2 * STAGES;
@@ -605,12 +602,10 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankAr
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int KT = g.K / BK;
     const long long tm = (g.M + BM - 1) / BM;
-    const int tn = (g.N + BN - 1) / BN;
-    // fixed tile index (resident operand) and walk (streamed operand)
-    const long long fix = ASTAT ? blockIdx.y : blockIdx.x;
-    const long long walk0 = ASTAT ? blockIdx.x : blockIdx.y;
-    const long long walk_step = ASTAT ? gridDim.x : gridDim.y;
-    const long long walk_n = ASTAT ? tn : tm;
+    // fixed column tile (resident B) and walk over the row tiles (streamed A)
+    const long long fix = blockIdx.x;
+    const long long walk0 = blockIdx.y;
+    const long long walk_step = gridDim.y;
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < STAGES; ++s) {
@@ -624,40 +619,22 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankAr
 
     if (warp == 8) {
         // ===================== producer =====================
-        if (ASTAT) {
-            const long long m0 = fix * BM;
-            if (lane == 0) {
-                mbar_expect_tx(res_full, (uint32_t)(KT * ABOX * 8));
-                for (int kt = 0; kt < KT; ++kt) tma_load_2d(res + kt * ABOX, &mapA, kt * BK, (int)m0, res_full);
-            }
-        } else {
-            const int n0 = (int)fix * BN;
-            const int nvalid = min(BN, g.N - n0);
-            if (lane == 0) mbar_expect_tx(res_full, (uint32_t)(KT * BK * nvalid * 8));
-            __syncwarp();
-            if (lane < BK)
-                for (int kt = 0; kt < KT; ++kt)
-                    bulk_g2s(res + kt * TILE_DOUBLES + lane * PM, g.B + (long long)(kt * BK + lane) * g.ldb + n0, nvalid * 8, res_full);
-        }
+        const int n0 = (int)fix * BN;
+        const int nvalid = min(BN, g.N - n0);
+        if (lane == 0) mbar_expect_tx(res_full, (uint32_t)(KT * BK * nvalid * 8));
+        __syncwarp();
+        if (lane < BK)
+            for (int kt = 0; kt < KT; ++kt)
+                bulk_g2s(res + kt * TILE_DOUBLES + lane * PM, g.B + (long long)(kt * BK + lane) * g.ldb + n0, nvalid * 8, res_full);
         int it = 0;
-        for (long long w = walk0; w < walk_n; w += walk_step) {
+        for (long long w = walk0; w < tm; w += walk_step) {
             for (int kt = 0; kt < KT; ++kt, ++it) {
                 const int s = it % STAGES;
                 const uint32_t ph = (it / STAGES) & 1;
                 mbar_wait(&empty[s], ph ^ 1);
-                if (ASTAT) {
-                    const int n0 = (int)w * BN;
-                    const int nvalid = min(BN, g.N - n0);
-                    if (lane == 0) mbar_expect_tx(&full[s], (uint32_t)(BK * nvalid * 8));
-                    __syncwarp();
-                    if (lane < BK)
-                        bulk_g2s(ring + s * TILE_DOUBLES + lane * PM, g.B + (long long)(kt * BK + lane) * g.ldb + n0, nvalid * 8,
-                                 &full[s]);
-                } else {
-                    if (lane == 0) {
-                        mbar_expect_tx(&full[s], (uint32_t)(ABOX * 8));
-                        tma_load_2d(ring + s * ABOX, &mapA, kt * BK, (int)(w * BM), &full[s]);
-                    }
+                if (lane == 0) {
+                    mbar_expect_tx(&full[s], (uint32_t)(ABOX * 8));
+                    tma_load_2d(ring + s * ABOX, &mapA, kt * BK, (int)(w * BM), &full[s]);
                 }
             }
         }
@@ -669,9 +646,9 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankAr
     const int gq = lane >> 2, tq = lane & 3;
     mbar_wait(res_full, 0);
     int it = 0;
-    for (long long w = walk0; w < walk_n; w += walk_step) {
-        const long long m0 = (ASTAT ? fix : w) * BM;
-        const int n0 = (int)(ASTAT ? w : fix) * BN;
+    for (long long w = walk0; w < tm; w += walk_step) {
+        const long long m0 = w * BM;
+        const int n0 = (int)fix * BN;
         const int mvalid = (int)min((long long)BM, g.M - m0);
         const int nvalid = min(BN, g.N - n0);
         if (g.beta != 0.0 && g.beta != 1.0 && tq == 0) {
@@ -697,8 +674,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankAr
             const int s = it % STAGES;
             const uint32_t ph = (it / STAGES) & 1;
             mbar_wait(&full[s], ph);
-            const double* sA = ASTAT ? res + kt * ABOX : ring + s * ABOX;
-            const double* sB = ASTAT ? ring + s * TILE_DOUBLES : res + kt * TILE_DOUBLES;
+            const double* sA = ring + s * ABOX;
+            const double* sB = res + kt * TILE_DOUBLES;
 #pragma unroll
             for (int ks = 0; ks < BK / 8; ++ks) {
                 double bf[4][2];
@@ -783,40 +760,29 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_rank_kernel(const RankAr
 // returns LQ_ERR_UNSUPPORTED when the shape is not a rank-K product this kernel takes
 int gemm_rank(Ctx* c, long long M, int N, int K, double alpha, const double* A, int lda, const double* B, int ldb, double beta,
               double* C, int ldc) {
-    if (LQ_ENV_ONCE("LINALG_B200_NO_RANK_GEMM")) return LQ_ERR_UNSUPPORTED;
     if (K > RK_KT_MAX * BK || K % BK != 0 || K < BK || (N % 2) != 0 || M < 2 * BM) return LQ_ERR_UNSUPPORTED;
     const long long tm = (M + BM - 1) / BM;
     const int tn = (N + BN - 1) / BN;
-    // which operand stays: the one whose tile is reused more often
-    const bool astat = tn >= 4;
-    if (!astat && tm < 4) return LQ_ERR_UNSUPPORTED;
-    // measured on B200: the B-stationary walk wins on tall-skinny products (30.2 vs 27.8 TFLOP/s at 2^20 x 128 x 128),
-    // the A-stationary walk does not beat the generic kernel on square block updates (23.6 vs 25.0) -> opt-in only
-    if (astat && !LQ_ENV_ONCE("LINALG_B200_RANK_ASTAT")) return LQ_ERR_UNSUPPORTED;
+    // measured on B200: the B-stationary walk wins on tall-skinny products (30.2 vs 27.8 TFLOP/s at 2^20 x 128 x 128).
+    // Wide outputs (4+ column tiles) and short ones stay on the generic kernel: an A-stationary walk for square block
+    // updates did not beat it (23.6 vs 25.0).
+    if (tn >= 4 || tm < 4) return LQ_ERR_UNSUPPORTED;
     static DeviceLatch configured;
     if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_rank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_SMEM_ASTAT));
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_rank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_SMEM_BSTAT));
+        LQ_CUDA(c, cudaFuncSetAttribute(gemm_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_SMEM_BSTAT));
         configured.set(c->device);
     }
     CUtensorMap mapA;
     LQ_TRY(make_kmajor_map(c, &mapA, A, M, K, lda));
     RankArgs g;
     g.B = B; g.C = C; g.M = M; g.N = N; g.K = K; g.ldb = ldb; g.ldc = ldc; g.alpha = alpha; g.beta = beta;
-    const long long fixed_tiles = astat ? tm : tn;
-    const long long walk_tiles = astat ? tn : tm;
-    // CTAs per fixed tile: fill the SMs once (persistent), at most one CTA per walked tile
-    long long per_fixed = std::max<long long>(1, std::min<long long>(walk_tiles, (c->sm_count + fixed_tiles - 1) / fixed_tiles));
+    // CTAs per column tile: fill the SMs once (persistent), at most one CTA per row tile
+    long long per_fixed = std::max<long long>(1, std::min<long long>(tm, (c->sm_count + tn - 1) / tn));
     // prefer a whole number of equal walks
-    while (per_fixed > 1 && fixed_tiles * per_fixed > (long long)c->sm_count && fixed_tiles * (per_fixed - 1) >= c->sm_count * 3 / 4)
+    while (per_fixed > 1 && tn * per_fixed > (long long)c->sm_count && tn * (per_fixed - 1) >= c->sm_count * 3 / 4)
         --per_fixed;
-    if (astat) {
-        dim3 grid((unsigned)per_fixed, (unsigned)tm);
-        gemm_rank_kernel<true><<<grid, GEMM_THREADS, RK_SMEM_ASTAT, c->stream>>>(g, mapA);
-    } else {
-        dim3 grid((unsigned)tn, (unsigned)per_fixed);
-        gemm_rank_kernel<false><<<grid, GEMM_THREADS, RK_SMEM_BSTAT, c->stream>>>(g, mapA);
-    }
+    dim3 grid((unsigned)tn, (unsigned)per_fixed);
+    gemm_rank_kernel<<<grid, GEMM_THREADS, RK_SMEM_BSTAT, c->stream>>>(g, mapA);
     LQ_CHECK_LAUNCH(c);
     LQ_COUNT_LAUNCH(c);
     return LQ_OK;
@@ -967,7 +933,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2) gemm_upd_kernel(const UpdArgs
 // C (+)= alpha * A * B for row-major A (M x K, lda), B (K x N, ldb), K a small multiple of 16; LQ_ERR_UNSUPPORTED otherwise
 int gemm_update(Ctx* c, long long M, int N, int K, double alpha, const double* A, int lda, const double* B, int ldb, double* C,
                 int ldc, bool overwrite) {
-    if (LQ_ENV_ONCE("LINALG_B200_NO_UPD_GEMM")) return LQ_ERR_UNSUPPORTED;
     if (K % BK != 0 || K < BK || K > 512 || (N % 2) != 0 || (ldc % 2) != 0 || !aligned16(C) || M < BM || N < UBN)
         return LQ_ERR_UNSUPPORTED;
     const long long tm = (M + BM - 1) / BM;
@@ -1012,7 +977,6 @@ int gemm(Ctx* c, bool ta, bool tb, long long M, int N, int K, double alpha, cons
     bool fast = Kmain >= BK && aligned16(A) && aligned16(B) && (lda % 2 == 0) && (ldb % 2 == 0) && (M * (long long)N >= 32 * 32);
     if (ta) fast = fast && (M % 2 == 0);   // M-major rows copied in whole 16-byte units
     if (!tb) fast = fast && (N % 2 == 0);
-    if (LQ_ENV_ONCE("LINALG_B200_NO_FAST_GEMM")) fast = false;
     if (!fast) {
         if (ta && tb) return launch_generic<true, true>(c, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc);
         if (ta) return launch_generic<true, false>(c, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc);
@@ -1055,13 +1019,9 @@ int vtc_finish(Ctx* c, const double* partials, int splits, long long stride, int
 int gemm_vtc_apply_t(Ctx* c, int kb, int nc, int mk, const double* V, int ldv, const double* Cm, int ldc, const double* T,
                      int ldt, bool trans_t, double* W2) {
     if (kb <= 0 || nc <= 0) return LQ_OK;
-    if (LQ_ENV_ONCE("LINALG_B200_VTC_CLUSTER") && vtc_cluster_supported(kb, nc, mk, V, ldv, Cm, ldc)) {
-        const int rc = vtc_cluster(c, trans_t ? 1 : 2, kb, nc, mk, V, ldv, Cm, ldc, T, ldt, W2);
-        if (rc != LQ_ERR_UNSUPPORTED) return rc;
-    }
     const int Kmain = mk - mk % BK;
     const bool fast = kb <= 128 && Kmain >= BK && Kmain == mk && aligned16(V) && aligned16(Cm) && (ldv % 2 == 0) &&
-                      (ldc % 2 == 0) && (kb % 4 == 0) && (nc % 2 == 0) && !LQ_ENV_ONCE("LINALG_B200_NO_FAST_GEMM");
+                      (ldc % 2 == 0) && (kb % 4 == 0) && (nc % 2 == 0);
     if (!fast) {
         DevBuf W;
         LQ_TRY(W.alloc(c, sizeof(double) * (size_t)kb * nc));

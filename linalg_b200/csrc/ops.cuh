@@ -19,11 +19,6 @@ int gemm_vtc_apply_t(Ctx* c, int kb, int nc, int mk, const double* V, int ldv, c
 int vtc_finish(Ctx* c, const double* partials, int splits, long long stride, int kb, int nc, const double* T, int ldt,
                bool trans_t, double* W2);
 
-// ---- vtc_cluster.cu: the same product in one cluster launch (split-K over DSMEM); mode 0: no T, 1: T^T, 2: T
-bool vtc_cluster_supported(int kb, int nc, int mk, const double* V, int ldv, const double* Cm, int ldc);
-int vtc_cluster(Ctx* c, int mode, int kb, int nc, int mk, const double* V, int ldv, const double* Cm, int ldc, const double* T,
-                int ldt, double* W2);
-
 // ---- blocked_qr.cu: single-matrix blocked compact-WY Householder (linalg/qr.py:52-100)
 int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, double* R);
 // factor only: A (m x n, lda) overwritten by R (upper) ; V (m x n, ldv) receives unit-norm reflectors

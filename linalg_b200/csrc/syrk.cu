@@ -156,8 +156,7 @@ __global__ void __launch_bounds__(256)
 }  // namespace
 
 bool syrk_tn_supported(const double* A, int lda, long long m, int n) {
-    static const bool off = getenv("LINALG_B200_NO_SYRK") != nullptr;
-    return !off && n >= 2 && n <= 128 && (n % 2 == 0) && (lda % 2 == 0) && ((reinterpret_cast<uintptr_t>(A) & 15) == 0) &&
+    return n >= 2 && n <= 128 && (n % 2 == 0) && (lda % 2 == 0) && ((reinterpret_cast<uintptr_t>(A) & 15) == 0) &&
            m >= 16LL * 64 && m / SBK < (1LL << 31);
 }
 

@@ -528,20 +528,6 @@ __global__ void __launch_bounds__(256) svd_post_kernel(const double* __restrict_
 }
 
 // ------------------------------------------------------------------ small triangular helpers (single CTA)
-// Rinv = R^{-1} for an upper-triangular R (n x n, row-major); column-parallel back substitution.
-__global__ void __launch_bounds__(256) triu_inverse_kernel(const double* __restrict__ R, int n, double* __restrict__ Rinv) {
-    for (int col = blockIdx.x * blockDim.x + threadIdx.x; col < n; col += gridDim.x * blockDim.x) {
-        for (int i = n - 1; i >= 0; --i) {
-            double acc = (i == col) ? 1.0 : 0.0;
-            if (i > col) {
-                Rinv[(size_t)i * n + col] = 0.0;
-                continue;
-            }
-            for (int k = i + 1; k <= col; ++k) acc = fma(-R[(size_t)i * n + k], Rinv[(size_t)k * n + col], acc);
-            Rinv[(size_t)i * n + col] = acc / R[(size_t)i * n + i];
-        }
-    }
-}
 // make diag(R) > 0: R <- S R, and return S (n) so that Q <- Q S
 __global__ void __launch_bounds__(256) sign_fix_R_kernel(double* __restrict__ R, int n, double* __restrict__ sgn) {
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -559,61 +545,9 @@ __global__ void __launch_bounds__(256) scale_cols_kernel(double* __restrict__ M,
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n * n; e += gridDim.x * blockDim.x) M[e] *= sgn[e % n];
 }
 
-// Upper Cholesky factor R (R^T R = G) of an n x n (n <= 128) SPD matrix, one CTA, right-looking in shared memory.
-// stat[0] = 1 if a pivot is not safely positive (breakdown), stat[1] = max_j G_jj / min_j R_jj^2  (~ cond(A)^2).
-__global__ void __launch_bounds__(1024) chol_upper_kernel(const double* __restrict__ G, int n, double* __restrict__ R,
-                                                          double* __restrict__ stat) {
-    extern __shared__ double chol_sm[];
-    double (*S)[129] = reinterpret_cast<double (*)[129]>(chol_sm);
-    __shared__ double s_dmax, s_pmin;
-    __shared__ int s_bad;
-    const int tid = threadIdx.x, nt = blockDim.x;
-    for (int e = tid; e < n * n; e += nt) S[e / n][e % n] = G[e];
-    if (tid == 0) {
-        s_dmax = 0.0;
-        s_pmin = 1e300;
-        s_bad = 0;
-    }
-    __syncthreads();
-    if (tid == 0) {
-        double dm = 0.0;
-        for (int j = 0; j < n; ++j) dm = fmax(dm, S[j][j]);
-        s_dmax = dm;
-    }
-    __syncthreads();
-    for (int j = 0; j < n; ++j) {
-        const double piv = S[j][j];
-        if (!(piv > 0.0)) {  // also catches NaN
-            if (tid == 0) s_bad = 1;
-            break;           // uniform: every thread reads the same S[j][j]
-        }
-        const double d = sqrt(piv);
-        __syncthreads();
-        if (tid == 0) s_pmin = fmin(s_pmin, piv);
-        for (int cidx = j + tid; cidx < n; cidx += nt) S[j][cidx] = (cidx == j) ? d : S[j][cidx] / d;
-        __syncthreads();
-        const int rem = n - j - 1;
-        for (int e = tid; e < rem * rem; e += nt) {
-            const int i = j + 1 + e / rem, cidx = j + 1 + e % rem;
-            if (cidx >= i) S[i][cidx] = fma(-S[j][i], S[j][cidx], S[i][cidx]);
-        }
-        __syncthreads();
-    }
-    __syncthreads();
-    for (int e = tid; e < n * n; e += nt) {
-        const int i = e / n, cidx = e % n;
-        R[e] = (cidx >= i) ? S[i][cidx] : 0.0;
-    }
-    if (tid == 0) {
-        stat[0] = s_bad ? 1.0 : 0.0;
-        stat[1] = s_bad ? 1e300 : s_dmax / s_pmin;
-    }
-}
-
-constexpr size_t CHOL_SMEM = 128 * 129 * sizeof(double);
-
-// ---- register-resident versions for n <= 128 (the CholeskyQR2 path of TSQR runs two of each per call; the generic
-// kernels above cost 0.20 + 0.36 ms, a fifth of the whole 2^20 x 128 TSQR)
+// ---- register-resident kernels for n <= 128.  Every caller has n <= 128: tsqr_local sends wider matrices to tsqr_wide,
+// whose panels are at most 128 columns.  The CholeskyQR2 path of TSQR runs two of each per call; shared-memory
+// versions cost 0.20 + 0.36 ms, a fifth of the whole 2^20 x 128 TSQR.
 //
 // Inverse of an upper-triangular R: warp w solves the columns w, w + 32, w + 64, w + 96 of R X = I together (four
 // independent recurrences interleaved); lane l holds rows l + 32 u of each right-hand side in registers, R sits in
@@ -671,8 +605,8 @@ __global__ void __launch_bounds__(128) triu_inverse128_kernel(const double* __re
 
 // Upper Cholesky factor for n <= 128 with the matrix in registers: thread (ty, tx) of a 32 x 32 block owns the
 // elements (ty + 32 a, tx + 32 b).  Per column: the diagonal owner publishes the pivot, the owners of row j publish
-// the scaled row, everybody updates its 16 elements (8 shared loads, 16 FMAs, no index arithmetic).  Same outputs
-// as chol_upper_kernel.
+// the scaled row, everybody updates its 16 elements (8 shared loads, 16 FMAs, no index arithmetic).
+// stat[0] = 1 if a pivot is not safely positive (breakdown), stat[1] = max_j G_jj / min_j R_jj^2  (~ cond(A)^2).
 __global__ void __launch_bounds__(1024) chol_upper128_kernel(const double* __restrict__ G, int n, double* __restrict__ R,
                                                              double* __restrict__ stat) {
     __shared__ double rowbuf[2][128];
@@ -750,16 +684,13 @@ __global__ void __launch_bounds__(1024) chol_upper128_kernel(const double* __res
 }
 
 int launch_triu_inverse(Ctx* c, const double* R, int n, double* Rinv) {
-    if (n <= 128) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(triu_inverse128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 129 * 8));
-            configured.set(c->device);
-        }
-        triu_inverse128_kernel<<<8, 128, 128 * 129 * 8, c->stream>>>(R, n, Rinv);
-    } else {
-        triu_inverse_kernel<<<1, 256, 0, c->stream>>>(R, n, Rinv);
+    LQ_REQUIRE(c, n <= 128, LQ_ERR_UNSUPPORTED, "triangular inverse supports n <= 128 (got %d)", n);
+    static DeviceLatch configured;
+    if (!configured.test(c->device)) {
+        LQ_CUDA(c, cudaFuncSetAttribute(triu_inverse128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 129 * 8));
+        configured.set(c->device);
     }
+    triu_inverse128_kernel<<<8, 128, 128 * 129 * 8, c->stream>>>(R, n, Rinv);
     LQ_CHECK_LAUNCH(c);
     return LQ_OK;
 }
@@ -775,7 +706,6 @@ __global__ void __launch_bounds__(256) scale_cols_tall_kernel(double* __restrict
 int eigh_configure(Ctx* c) {
     static DeviceLatch done;
     if (done.test(c->device)) return LQ_OK;
-    LQ_CUDA(c, cudaFuncSetAttribute(chol_upper_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CHOL_SMEM));
     cudaFuncAttributes fa{};
     LQ_CUDA(c, cudaFuncGetAttributes(&fa, jacobi_kernel));
     LQ_CUDA(c, cudaFuncSetAttribute(jacobi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -850,9 +780,7 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
     const int max_sweeps = 40;
     // a pair is rotated while |a_pq| > rel_tol * sqrt(a_pp a_qq); 4 eps stops the tail of sweeps that only chase
     // rounding noise (eigenvalues move by O(a_pq^2 / gap), the eigenvector basis stays a product of exact rotations)
-    double rel_tol = 4.0 * 1.1102230246251565e-16;
-    static const double env_tol = getenv("LINALG_B200_JACOBI_TOL") ? atof(getenv("LINALG_B200_JACOBI_TOL")) : 0.0;  // read once
-    if (env_tol > 0.0) rel_tol = env_tol * 1.1102230246251565e-16;
+    const double rel_tol = 4.0 * 1.1102230246251565e-16;
     DevBuf Aw, rot, nr, lam, Vraw, ptab;
     LQ_TRY(nr.alloc(c, 16));
     LQ_TRY(lam.alloc(c, sizeof(double) * n));
@@ -863,7 +791,7 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
         LQ_TRY(Aw.alloc(c, sizeof(double) * (size_t)ne * ne));
         LQ_TRY(rot.alloc(c, sizeof(double2) * (size_t)(max_sweeps + 1) * jacobi1s_steps_per_sweep(ne) * 64));
         LQ_TRY(ptab.alloc(c, sizeof(unsigned short) * (size_t)jacobi1s_steps_per_sweep(ne) * 64));
-        const int direct = (psd && !LQ_ENV_ONCE("LINALG_B200_JACOBI_ALWAYS_REPLAY")) ? 1 : 0;
+        const int direct = psd ? 1 : 0;
         if (ne == 128)
             jacobi1s_kernel<8><<<1, 512, sizeof(double) * (size_t)ne * ne, c->stream>>>(G, n, ne, rot.as<double2>(), max_sweeps, rel_tol,
                                                                                        nr.as<int>(), Aw.as<double>(), ptab.as<unsigned short>(), lam.as<double>(), direct);
@@ -1010,7 +938,6 @@ struct CholQrScratch {
 // into the two spare words behind G so that it is summed over the ranks by the first all-reduce (G[n*n]).
 static int cholqr2_enqueue(Ctx* c, const double* A, int lda, long long m, int n, double* Q, int ldq, double* R, int ldr,
                            bool sharded, CholQrScratch& w, double* stat, double short_flag) {
-    const bool new_chol = n <= 128 && !c->env_old_chol;
     double* G = w.G.as<double>();
     const bool carry = short_flag >= 0.0;
     if (carry) {
@@ -1020,16 +947,14 @@ static int cholqr2_enqueue(Ctx* c, const double* A, int lda, long long m, int n,
     // pass 1
     LQ_TRY(gram_ld(c, A, lda, m, n, G));
     if (sharded) LQ_TRY(comm_allreduce_sum(c, G, (long long)n * n + (carry ? 2 : 0)));
-    if (new_chol) chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R1.as<double>(), stat);
-    else chol_upper_kernel<<<1, 1024, CHOL_SMEM, c->stream>>>(G, n, w.R1.as<double>(), stat);
+    chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R1.as<double>(), stat);
     LQ_CHECK_LAUNCH(c);
     LQ_TRY(launch_triu_inverse(c, w.R1.as<double>(), n, w.Rinv.as<double>()));
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, lda, w.Rinv.as<double>(), n, 0.0, w.Q1.as<double>(), n));
     // pass 2
     LQ_TRY(gram_ld(c, w.Q1.as<double>(), n, m, n, G));
     if (sharded) LQ_TRY(comm_allreduce_sum(c, G, (long long)n * n));
-    if (new_chol) chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R2.as<double>(), stat + 2);
-    else chol_upper_kernel<<<1, 1024, CHOL_SMEM, c->stream>>>(G, n, w.R2.as<double>(), stat + 2);
+    chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R2.as<double>(), stat + 2);
     LQ_CHECK_LAUNCH(c);
     LQ_TRY(launch_triu_inverse(c, w.R2.as<double>(), n, w.Rinv.as<double>()));
     c->launches += 4 + (carry ? 1 : 0);

@@ -533,9 +533,10 @@ def test_batched32_householder_kernel_matches_oracle(ctx, batch):
 
 
 @pytest.mark.parametrize("m", [33, 64, 300, 1000, 4096, 8192])
-def test_panel_kernels_agree(ctx, m):
-    """The three panel factorisations of the blocked path (barrier.cluster kernel, st.async kernels with 512 / 256
-    rows per CTA) produce the same R rows, unit-norm reflectors and compact-WY factor, and (I - V T V^T)^T A = [R; 0]."""
+def test_panel_kernel_versions_agree(ctx, m):
+    """The panel factorisations of the blocked path (barrier.cluster kernel, st.async kernel with 256 rows per CTA, and
+    the default choice, which is the one-CTA SOLO kernel up to 256 rows) produce the same R rows, unit-norm reflectors
+    and compact-WY factor, and (I - V T V^T)^T A = [R; 0].  Versions 2 and 4 do not exist."""
     lda = 64
     A = np.random.default_rng(m).standard_normal((m, 32))
     if m == 300:
@@ -552,13 +553,16 @@ def test_panel_kernels_agree(ctx, m):
 
     ref = run(1)
     scale = np.abs(A).max()
-    for version in (2, 3):
-        if m > 16 * (512 if version == 2 else 256):
+    for version in (3, 0):
+        if version == 3 and m > 16 * 256:
             continue
         R, V, T = run(version)
         assert orc.rel_max_err(R, ref[0]) <= 1e-13 and orc.rel_max_err(V, ref[1]) <= 1e-13 and orc.rel_max_err(T, ref[2]) <= 1e-12
         QtA = A - V @ (T.T @ (V.T @ A))
         assert np.abs(QtA[:32] - R).max() <= 1e-13 * scale * np.sqrt(m) and (m == 32 or np.abs(QtA[32:]).max() <= 1e-13 * scale * np.sqrt(m))
+    for version in (2, 4):
+        with pytest.raises(ValueError):
+            run(version)
 
 
 def test_eigh_one_sided_matches_two_sided(ctx):

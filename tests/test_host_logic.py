@@ -171,3 +171,16 @@ def test_fan_out_splits_contiguously_and_reraises():
         nat.fan_out([1, 1], 8, fn, _contexts="ab")
     with pytest.raises(ValueError):
         nat.fan_out([], 8, fn)
+
+
+def test_native_environment_switches_are_the_documented_ones():
+    """Kernel selection depends on the input shape: the native sources read only the switches of DESIGN.md §5 that select
+    nothing or that the GPU tests use to reach a path well-conditioned input does not take."""
+    import glob
+    import re
+
+    found = set()
+    for path in glob.glob(os.path.join(ROOT, "linalg_b200", "csrc", "*.cu*")):
+        with open(path) as fh:
+            found |= set(re.findall(r"LINALG_B200_([A-Z_]+)", fh.read()))
+    assert found == {"TRACE_BLOCKS", "NO_GRAPH", "TSQR_HOUSEHOLDER", "JACOBI_TWO_SIDED", "NCCL_LIB"}

@@ -29,9 +29,8 @@ for m in (8192, 5000, 4096, 2048, 1000, 512, 300, 256, 200, 64, 33, 32):
     Qn, Rn = np.linalg.qr(A)
     ref = run(A, 1, 20)
     line = f"m={m:5d} v1 {ref[3]:7.1f} us"
-    for ver in (2, 3, 0):
+    for ver in (3, 0):
         if ver == 0 and m > 256: continue   # version 0 = default: the one-CTA SOLO kernel up to 256 rows
-        if ver == 2 and m > 16 * 512: continue
         if ver == 3 and m > 16 * 256: continue
         got = run(A, ver, 20)
         # invariants: (I - V T V^T)^T A = [R; 0]
