@@ -22,7 +22,8 @@ int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long bat
     }
     const size_t smem = small_hh_smem_doubles(m, n, 0) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_hh_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, m, n, 0);
+        return launch_batched<small_hh_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, nullptr,
+                                                  m, n, 0);
     // too large for one CTA: blocked path, matrix by matrix (stream `st` must be the context stream)
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(blocked_householder_qr(c, A + b * (long long)m * n, m, n, Q + b * (long long)m * n,
@@ -52,23 +53,21 @@ int mgs_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long ba
 }
 
 // info (device, may be null): per system 0, or 1 + the first column whose R[j][j] is exactly 0 (np.linalg.solve raises
-// LinAlgError("Singular matrix") there, linalg/qr.py:134); reported by the warp-per-system kernel (n <= 64, nrhs <= 16),
-// 0 for the other shapes
+// LinAlgError("Singular matrix") there, linalg/qr.py:134); every route writes it
 int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
                             int nrhs, double* X, int* info = nullptr) {
     if (batch == 0) return LQ_OK;
     int rc = lstsq_tile_kernel_launch(c, st, A, B, batch, m, n, nrhs, X, info, 2);
     if (rc != LQ_ERR_UNSUPPORTED) return rc;
-    if (info) LQ_CUDA(c, cudaMemsetAsync(info, 0, sizeof(int) * (size_t)batch, st));
-    rc = lstsq_stream_kernel_launch(c, st, A, B, batch, m, n, nrhs, X);
+    rc = lstsq_stream_kernel_launch(c, st, A, B, batch, m, n, nrhs, X, info);
     if (rc != LQ_ERR_UNSUPPORTED) return rc;
     const size_t smem = small_hh_smem_doubles(m, n, nrhs) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_hh_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, m, n,
-                                                  nrhs);
+        return launch_batched<small_hh_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, info, m,
+                                                  n, nrhs);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_lstsq_householder(c, A + b * (long long)m * n, B + b * (long long)m * nrhs, m, n, nrhs,
-                                       X + b * (long long)n * nrhs));
+                                       X + b * (long long)n * nrhs, info ? info + b : nullptr));
     return LQ_OK;
 }
 
@@ -246,16 +245,18 @@ static int lstsq_hh_host(lq_ctx* h, const double* A, const double* B, int64_t ba
         !lstsq_tile_kernel_supported(m, n, nrhs)) {
         LQ_CUDA(c, cudaSetDevice(c->device));
         for (int64_t b = 0; b < batch; ++b) {
-            DevBuf dA, dB, dX;
+            DevBuf dA, dB, dX, dI;
             LQ_TRY(dA.alloc(c, mn));
             LQ_TRY(dB.alloc(c, mk));
             LQ_TRY(dX.alloc(c, nk));
+            if (info) LQ_TRY(dI.alloc(c, 16));
             LQ_CUDA(c, cudaMemcpyAsync(dA.p, A + b * (size_t)m * n, mn, cudaMemcpyHostToDevice, c->stream));
             LQ_CUDA(c, cudaMemcpyAsync(dB.p, B + b * (size_t)m * nrhs, mk, cudaMemcpyHostToDevice, c->stream));
-            LQ_TRY(large_lstsq_householder(c, dA.as<double>(), dB.as<double>(), m, n, nrhs, dX.as<double>()));
+            LQ_TRY(large_lstsq_householder(c, dA.as<double>(), dB.as<double>(), m, n, nrhs, dX.as<double>(),
+                                           info ? dI.as<int>() : nullptr));
             LQ_CUDA(c, cudaMemcpyAsync(X + b * (size_t)n * nrhs, dX.p, nk, cudaMemcpyDeviceToHost, c->stream));
+            if (info) LQ_CUDA(c, cudaMemcpyAsync(info + b, dI.p, 4, cudaMemcpyDeviceToHost, c->stream));
             LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-            if (info) info[b] = 0;
         }
         return LQ_OK;
     }

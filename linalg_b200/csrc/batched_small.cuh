@@ -32,11 +32,12 @@ __device__ __forceinline__ double block_sum(double v, double* red /*>=33 doubles
     return t;  // every thread has the total
 }
 
-// mode: 0 = QR (write Q m x n and R n x n), 1 = least squares (write X n x nrhs)
+// mode: 0 = QR (write Q m x n and R n x n), 1 = least squares (write X n x nrhs and, when info is not null, per system
+// 0 or 1 + the first column whose R[j][j] is exactly 0: np.linalg.solve raises there, linalg/qr.py:134)
 template <int MODE>
 __global__ void __launch_bounds__(256)
     small_hh_kernel(const double* __restrict__ A, const double* __restrict__ B, double* __restrict__ Q,
-                    double* __restrict__ R, double* __restrict__ X, int m, int n, int nrhs) {
+                    double* __restrict__ R, double* __restrict__ X, int* __restrict__ info, int m, int n, int nrhs) {
     extern __shared__ __align__(16) double sm[];
     const int ld = small_pitch(m);
     const int nc = n + nrhs;
@@ -133,6 +134,12 @@ __global__ void __launch_bounds__(256)
             Qg[e] = W[(size_t)c * ld + i];
         }
     } else {
+        if (info != nullptr && tid == 0) {
+            int bad = 0;
+            for (int j = n - 1; j >= 0; --j)
+                if (rdiag[j] == 0.0) bad = j + 1;
+            info[b] = bad;
+        }
         // back-substitution R x = (Q^T B)[:n]; one thread per right-hand side
         for (int k = tid; k < nrhs; k += nt) {
             double* y = W + (size_t)(n + k) * ld;

@@ -632,6 +632,17 @@ __global__ void __launch_bounds__(256) backsub_diag_kernel(const double* __restr
 }
 constexpr size_t BACKSUB_SMEM = (128 * 129 + 128 * 33) * sizeof(double);
 
+// *info = 0, or 1 + the first j with R[j][j] exactly 0 (R: n x n, ldr); one CTA
+__global__ void __launch_bounds__(256) singular_diag_kernel(const double* __restrict__ R, int ldr, int n, int* __restrict__ info) {
+    __shared__ int first;
+    if (threadIdx.x == 0) first = n;
+    __syncthreads();
+    for (int j = threadIdx.x; j < n; j += blockDim.x)
+        if (R[(long long)j * ldr + j] == 0.0) atomicMin(&first, j);
+    __syncthreads();
+    if (threadIdx.x == 0) *info = (first < n) ? first + 1 : 0;
+}
+
 // R X = Y in place (Y: n x k, ldy; k even when the tensor-core GEMM is to be used for the off-diagonal part)
 int back_substitute(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n, int k) {
     if (n <= 256) {
@@ -748,7 +759,7 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
     return LQ_OK;
 }
 
-int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X) {
+int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info) {
     LQ_REQUIRE(c, m >= n && n >= 1 && nrhs >= 1, LQ_ERR_SHAPE, "least squares needs m >= n >= 1, nrhs >= 1");
     LQ_TRY(configure_once(c));
     const int npad = (n + 31) / 32 * 32;
@@ -763,6 +774,11 @@ int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int
     c->launches += 2;
     LQ_CUDA(c, cudaMemsetAsync(Vw.p, 0, sizeof(double) * (size_t)m * npad, c->stream));
     LQ_TRY(factor_padded(c, Aw.as<double>(), npad, m, npad, n, Vw.as<double>(), npad, Bw.as<double>(), kpad, kpad, nullptr));
+    if (info) {
+        singular_diag_kernel<<<1, 256, 0, c->stream>>>(Aw.as<double>(), npad, n, info);
+        LQ_CHECK_LAUNCH(c);
+        LQ_COUNT_LAUNCH(c);
+    }
     LQ_TRY(back_substitute(c, Aw.as<double>(), npad, Bw.as<double>(), kpad, n, kpad));
     unpad_copy_kernel<<<grid_for(c, (long long)n * nrhs), 256, 0, c->stream>>>(Bw.as<double>(), kpad, X, nrhs, n, nrhs);
     LQ_CHECK_LAUNCH(c);

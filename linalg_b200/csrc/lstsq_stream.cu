@@ -13,11 +13,12 @@ bool lstsq_stream_kernel_supported(int m, int n, int nrhs) {
 // rows per streamed block = RPT * WARPS = 16 * 4.  Taller blocks mean fewer column steps per system (every step pays the
 // publish -> dots -> barrier -> norm / reciprocal chain once, whatever the block height).
 int lstsq_stream_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
-                               int nrhs, double* X) {
+                               int nrhs, double* X, int* info) {
     if (!lstsq_stream_kernel_supported(m, n, nrhs)) return LQ_ERR_UNSUPPORTED;
     constexpr int RPT = 16, WARPS = 4;
     const size_t smem = StreamCfg<3, RPT, WARPS>::smem_doubles(n) * sizeof(double);
-    return launch_batched<lstsq_stream_kernel<RPT, WARPS>>(c, st, batch, WARPS * 32, smem, c->max_smem, A, B, X, m, n, nrhs);
+    return launch_batched<lstsq_stream_kernel<RPT, WARPS>>(c, st, batch, WARPS * 32, smem, c->max_smem, A, B, X, info, m, n,
+                                                           nrhs);
 }
 
 // ---- round 2: one warp per system, block reflectors on DMMA (lstsq_tile.cuh); n <= 64, nrhs <= 16

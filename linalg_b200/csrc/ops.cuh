@@ -25,16 +25,18 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
 // (zeros above the diagonal), skipped reflectors are zero columns.  Optional B (m x nrhs) gets Q^T B.
 int blocked_householder_factor(Ctx* c, double* A, int lda, int m, int n, double* V, int ldv, double* B, int ldb,
                                int nrhs);
-int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X);
+// info (device, may be null): 0, or 1 + the first column whose R[j][j] is exactly 0 (the solve is singular)
+int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info);
 
 // ---- large_mgs.cu: single-matrix MGS for shapes beyond one CTA's shared memory
 int large_mgs_qr(Ctx* c, const double* A, int m, int n, int reorth, double* Q, double* R, int* info);
 int large_lstsq_mgs(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info);
 
-// ---- lstsq_stream.cu: K3 streaming Householder least squares (n = 64 specialisation)
+// ---- lstsq_stream.cu: K3 streaming Householder least squares (n <= 64, nrhs <= 32).  info (may be null): per system 0,
+// or 1 + the first column whose R[j][j] is exactly 0.  LQ_ERR_UNSUPPORTED if the shape is not covered.
 bool lstsq_stream_kernel_supported(int m, int n, int nrhs);
 int lstsq_stream_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m,
-                               int n, int nrhs, double* X);  // LQ_ERR_UNSUPPORTED if the shape is not covered
+                               int n, int nrhs, double* X, int* info);
 
 // round 2: one warp per system, block reflectors on DMMA (n <= 64, nrhs <= 16).  info (may be null): per system, 0 or
 // 1 + the first column with |R[j][j]| < 1e-12 (info_mode 1, the MGS test of linalg/qr.py:40-41) / == 0 (info_mode 2)

@@ -127,12 +127,13 @@ __device__ __forceinline__ void stream_factor_block(double (&r)[C][RPT], double*
 
 // ---------------------------------------------------------------------------------------------
 // K3: batched Householder least squares, one CTA per system.  A (batch, m, n), B (batch, m, nrhs),
-// X (batch, n, nrhs); n <= 64 (two column slots for A), nrhs <= 32 (third slot).
+// X (batch, n, nrhs); n <= 64 (two column slots for A), nrhs <= 32 (third slot).  info (may be null): per system 0, or
+// 1 + the first column whose R[j][j] is exactly 0 (np.linalg.solve raises there, linalg/qr.py:134).
 // ---------------------------------------------------------------------------------------------
 template <int RPT, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32)
-    lstsq_stream_kernel(const double* __restrict__ A, const double* __restrict__ B, double* __restrict__ X, int m, int n,
-                        int nrhs) {
+    lstsq_stream_kernel(const double* __restrict__ A, const double* __restrict__ B, double* __restrict__ X,
+                        int* __restrict__ info, int m, int n, int nrhs) {
     constexpr int C = 3;
     using Cfg = StreamCfg<C, RPT, WARPS>;
     constexpr int NCAP = Cfg::NCAP;
@@ -166,6 +167,12 @@ __global__ void __launch_bounds__(WARPS * 32)
         stream_factor_block<C, RPT, WARPS>(r, Rs, part, vbuf, n, lane, warp);
     }
 
+    if (info != nullptr && threadIdx.x == 0) {
+        int bad = 0;
+        for (int j = n - 1; j >= 0; --j)
+            if (Rs[j * NCAP + j] == 0.0) bad = j + 1;
+        info[sys] = bad;
+    }
     // back-substitution R x = y, y = Rs[:, 64 + k]; one thread per right-hand side
     if (threadIdx.x < nrhs) {
         const int k = 64 + threadIdx.x;
