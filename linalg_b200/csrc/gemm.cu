@@ -402,10 +402,17 @@ __global__ void __launch_bounds__(256) gemm_generic_kernel(const double* __restr
 template <bool AT, bool BT>
 int launch_generic(Ctx* c, long long M, int N, int K, double alpha, const double* A, int lda, const double* B, int ldb,
                    double beta, double* C, int ldc) {
-    dim3 grid((N + 31) / 32, (unsigned)((M + 31) / 32));
-    gemm_generic_kernel<AT, BT><<<grid, 256, 0, c->stream>>>(A, B, C, M, N, K, lda, ldb, ldc, alpha, beta);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    // one 32-row tile per blockIdx.y (<= 65535): a taller product -- gemm's 2^21-row chunks are 65536 tiles -- is launched
+    // in row slices; every output row is computed the same way in either case
+    constexpr long long MAX_ROWS = 65535LL * 32;
+    for (long long r = 0; r < M; r += MAX_ROWS) {
+        const long long mr = std::min(MAX_ROWS, M - r);
+        const double* Ar = AT ? A + r : A + r * (long long)lda;
+        dim3 grid((N + 31) / 32, (unsigned)((mr + 31) / 32));
+        gemm_generic_kernel<AT, BT><<<grid, 256, 0, c->stream>>>(Ar, B, C + r * (long long)ldc, mr, N, K, lda, ldb, ldc, alpha, beta);
+        LQ_CHECK_LAUNCH(c);
+        LQ_COUNT_LAUNCH(c);
+    }
     return LQ_OK;
 }
 
@@ -958,7 +965,7 @@ int gemm(Ctx* c, bool ta, bool tb, long long M, int N, int K, double alpha, cons
          int ldb, double beta, double* C, int ldc) {
     if (M <= 0 || N <= 0) return LQ_OK;
     // the kernels index the row tiles with blockIdx.y (<= 65535): very tall products (2^23 x 128 on one GPU) go in row chunks
-    constexpr long long ROW_CHUNK = 1LL << 21;  // 65536 generic 32-row tiles
+    constexpr long long ROW_CHUNK = 1LL << 21;  // 16384 tiles of 128 rows (launch_generic slices its 32-row tiles further)
     if (M > ROW_CHUNK) {
         for (long long r = 0; r < M; r += ROW_CHUNK) {
             const long long mc = std::min(ROW_CHUNK, M - r);

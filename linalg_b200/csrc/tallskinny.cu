@@ -809,7 +809,7 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
         LQ_CHECK_LAUNCH(c);
         eig_sort_kernel<<<small_grid(c, n), 256, sizeof(int) * n, c->stream>>>(lam.as<double>(), Vraw.as<double>(), n, lambda_desc, V);
         LQ_CHECK_LAUNCH(c);
-        c->launches += 5;
+        c->launches += direct ? 5 : 4;
         return LQ_OK;
     }
     const int ne = (n + 1) & ~1, ld = ne | 1, half = ne / 2;

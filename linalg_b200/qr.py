@@ -209,7 +209,7 @@ def least_squares_qr_batched(A, B, *, out=None, ctx=None, devices=None) -> np.nd
 
 # ----------------------------------------------------------------------------- a7
 def tsqr(A, *, ctx=None) -> Tuple[np.ndarray, np.ndarray]:
-    """Thin QR of a tall-skinny (m, n <= 128) matrix with ``diag(R) > 0`` (the ``qr`` convention)."""
+    """Thin QR of a tall-skinny (m, n) matrix, m >= n, with ``diag(R) > 0`` (the ``qr`` convention)."""
     A = as_f64_matrix(A)
     m, n = A.shape
     if m < n:
