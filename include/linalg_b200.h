@@ -55,7 +55,9 @@ int lq_sync(lq_ctx* ctx);
 int lq_event_record(lq_ctx* ctx, int slot);                       /* slot 0..15, on ctx stream */
 int lq_event_elapsed_ms(lq_ctx* ctx, int slot_a, int slot_b, float* ms); /* syncs on slot_b */
 int lq_flush_l2(lq_ctx* ctx);        /* overwrite a 256 MiB scratch buffer (> 126 MB L2) */
-int64_t lq_kernel_launches(lq_ctx* ctx); /* number of this library's kernels launched so far */
+/* kernels the linear-algebra entry points launched on ctx so far, each counted once by the launch helper that launched it
+ * (a CUDA-graph replay adds the kernels it holds); the measurement utilities lq_probe and lq_flush_l2 are not counted */
+int64_t lq_kernel_launches(lq_ctx* ctx);
 
 /* diagnostics: kernel-selection switches of one context.  name is the LINALG_B200_<NAME> environment variable without
  * its prefix ("TSQR_HOUSEHOLDER", "JACOBI_TWO_SIDED"); any other name returns LQ_ERR_ARG.  The environment only gives

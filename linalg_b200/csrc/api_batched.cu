@@ -17,13 +17,12 @@ int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long bat
         // lane = column, four matrices per warp, left-looking panels, Q formation on DMMA, one 8-warp CTA per SM
         constexpr int WARPS = 8;
         const size_t smem = (size_t)WARPS * Col8::WARP_DOUBLES * sizeof(double);
-        return launch_batched<hh_qr32_c8_kernel<WARPS, 1>>(c, st, (batch + 4 * WARPS - 1) / (4 * WARPS), WARPS * 32, smem,
-                                                           (int)smem, A, Q, R, batch);
+        return launch<hh_qr32_c8_kernel<WARPS, 1>>(c, (batch + 4 * WARPS - 1) / (4 * WARPS), WARPS * 32, smem, st, (int)smem, A,
+                                                   Q, R, batch);
     }
     const size_t smem = small_hh_smem_doubles(m, n, 0) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_hh_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, nullptr,
-                                                  m, n, 0);
+        return launch<small_hh_kernel<0>>(c, batch, 256, smem, st, c->max_smem, A, nullptr, Q, R, nullptr, nullptr, m, n, 0);
     // too large for one CTA: blocked path, matrix by matrix (stream `st` must be the context stream)
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(blocked_householder_qr(c, A + b * (long long)m * n, m, n, Q + b * (long long)m * n,
@@ -38,14 +37,14 @@ int mgs_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long ba
         using D = Dist32<2, 4>;
         constexpr int WARPS = 2;
         const long long per_block = (long long)WARPS * D::MPW;
-        return launch_batched<mgs_qr32_kernel<2, 4, WARPS, 4>>(c, st, (batch + per_block - 1) / per_block, WARPS * 32,
-                                                               (size_t)per_block * D::MGS_DOUBLES * sizeof(double), 0, A, Q,
-                                                               R, info, batch, reorth);
+        return launch<mgs_qr32_kernel<2, 4, WARPS, 4>>(c, (batch + per_block - 1) / per_block, WARPS * 32,
+                                                       (size_t)per_block * D::MGS_DOUBLES * sizeof(double), st, 0, A, Q, R, info,
+                                                       batch, reorth);
     }
     const size_t smem = small_mgs_smem_doubles(m, n, 0) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_mgs_kernel<0>>(c, st, batch, 256, smem, c->max_smem, A, nullptr, Q, R, nullptr, info, m,
-                                                   n, 0, reorth);
+        return launch<small_mgs_kernel<0>>(c, batch, 256, smem, st, c->max_smem, A, nullptr, Q, R, nullptr, info, m, n, 0,
+                                           reorth);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_mgs_qr(c, A + b * (long long)m * n, m, n, reorth, Q + b * (long long)m * n,
                             R + b * (long long)n * n, info ? info + b : nullptr));
@@ -63,8 +62,7 @@ int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const doub
     if (rc != LQ_ERR_UNSUPPORTED) return rc;
     const size_t smem = small_hh_smem_doubles(m, n, nrhs) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_hh_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, info, m,
-                                                  n, nrhs);
+        return launch<small_hh_kernel<1>>(c, batch, 256, smem, st, c->max_smem, A, B, nullptr, nullptr, X, info, m, n, nrhs);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_lstsq_householder(c, A + b * (long long)m * n, B + b * (long long)m * nrhs, m, n, nrhs,
                                        X + b * (long long)n * nrhs, info ? info + b : nullptr));
@@ -82,8 +80,8 @@ int lstsq_mgs_batched_stream(Ctx* c, cudaStream_t st, const double* A, const dou
     }
     const size_t smem = small_mgs_smem_doubles(m, n, nrhs) * sizeof(double);
     if (smem <= (size_t)c->max_smem)
-        return launch_batched<small_mgs_kernel<1>>(c, st, batch, 256, smem, c->max_smem, A, B, nullptr, nullptr, X, info, m,
-                                                   n, nrhs, 0);
+        return launch<small_mgs_kernel<1>>(c, batch, 256, smem, st, c->max_smem, A, B, nullptr, nullptr, X, info, m, n, nrhs,
+                                           0);
     for (long long b = 0; b < batch; ++b)
         LQ_TRY(large_lstsq_mgs(c, A + b * (long long)m * n, B + b * (long long)m * nrhs, m, n, nrhs,
                                X + b * (long long)n * nrhs, info ? info + b : nullptr));

@@ -5,7 +5,7 @@
 #include <mutex>
 
 #include "../../include/linalg_b200.h"
-#include "ctx.cuh"
+#include "ops.cuh"
 
 namespace lq {
 
@@ -214,6 +214,7 @@ int lq_create(int device, lq_ctx** out) {
     }
     c->sm_count = c->prop.multiProcessorCount;
     c->max_smem = (int)c->prop.sharedMemPerBlockOptin;
+    LQ_TRY(measure_max_cluster(c));
     // the context stream carries the latency-bound chains (panel factorisations); the side lanes carry bulk
     // work that overlaps with them, so the main stream gets the higher scheduling priority
     int prio_lo = 0, prio_hi = 0;
@@ -389,7 +390,6 @@ int lq_probe(lq_ctx* h, int kind, double* result) {
             else if (kind == 1) probe_dmma_kernel<<<blocks, threads, 0, c->stream>>>(out.as<double>(), iters, 1.0);
             else probe_mixed_kernel<<<blocks, threads, 0, c->stream>>>(out.as<double>(), iters, 1.0);
             LQ_CHECK_LAUNCH(c);
-            LQ_COUNT_LAUNCH(c);
             LQ_CUDA(c, cudaEventRecord(e1, c->stream));
             LQ_CUDA(c, cudaEventSynchronize(e1));
             LQ_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));
@@ -415,7 +415,6 @@ int lq_probe(lq_ctx* h, int kind, double* result) {
             LQ_CUDA(c, cudaEventRecord(e0, c->stream));
             probe_copy_kernel<<<c->sm_count * 16, 256, 0, c->stream>>>(a.as<double4>(), b.as<double4>(), bytes / 32);
             LQ_CHECK_LAUNCH(c);
-            LQ_COUNT_LAUNCH(c);
             LQ_CUDA(c, cudaEventRecord(e1, c->stream));
             LQ_CUDA(c, cudaEventSynchronize(e1));
             LQ_CUDA(c, cudaEventElapsedTime(&ms, e0, e1));

@@ -223,102 +223,39 @@ int panel_generic(Ctx* c, double* A, int lda, double* V, int ldv, double* T, int
     GPanelState* st = stb.as<GPanelState>();
     const int ctas = std::max(1, std::min(c->sm_count * 2, (mp + 255) / 256));
     const int rpc = (mp + ctas - 1) / ctas;
-    gpanel_clear_kernel<<<1, 64, 0, c->stream>>>(st, 1);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<gpanel_clear_kernel>(c, 1, 64, 0, c->stream, 0, st, 1));
     for (int j = 0; j < nb; ++j) {
-        gpanel_dots_kernel<<<ctas, 256, 0, c->stream>>>(A, lda, mp, nb, j, st, rpc);
-        gpanel_update_kernel<<<ctas, 256, 0, c->stream>>>(A, lda, mp, nb, j, st, rpc);
-        gpanel_clear_kernel<<<1, 64, 0, c->stream>>>(st, 0);
-        c->launches += 3;
+        LQ_TRY(launch<gpanel_dots_kernel>(c, ctas, 256, 0, c->stream, 0, A, lda, mp, nb, j, st, rpc));
+        LQ_TRY(launch<gpanel_update_kernel>(c, ctas, 256, 0, c->stream, 0, A, lda, mp, nb, j, st, rpc));
+        LQ_TRY(launch<gpanel_clear_kernel>(c, 1, 64, 0, c->stream, 0, st, 0));
     }
-    gpanel_store_kernel<<<std::min(ctas, 64), 256, 0, c->stream>>>(A, lda, V, ldv, T, ldt, mp, nb, st);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
-}
-
-// ------------------------------------------------------------------ cluster panel launch
-int detect_max_cluster(Ctx* c) {
-    static int cached[64] = {};
-    if (cached[c->device]) return cached[c->device];
-    auto kern = panel_cluster_kernel<4, 16>;
-    int best = 1;
-    cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    for (int cs : {16, 8, 4, 2}) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3(cs);
-        cfg.blockDim = dim3(PANEL_THREADS);
-        cfg.dynamicSmemBytes = 0;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = cs;
-        at[0].val.clusterDim.y = 1;
-        at[0].val.clusterDim.z = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
-        int n = 0;
-        cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
-        if (e == cudaSuccess && n >= 1) {
-            best = cs;
-            break;
-        }
-        cudaGetLastError();
-    }
-    cached[c->device] = best;
-    c->max_cluster = best;
-    return best;
-}
-
-template <typename Kern, typename... Args>
-int launch_cluster(Ctx* c, Kern kern, int cs, int threads, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(cs);
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = 0;
-    cfg.stream = c->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = cs;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    LQ_CUDA(c, cudaLaunchKernelEx(&cfg, kern, args...));
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<gpanel_store_kernel>(c, std::min(ctas, 64), 256, 0, c->stream, 0, A, lda, V, ldv, T, ldt, mp, nb, st);
 }
 
 // version: 0 = default choice (panels of up to 256 rows: the one-CTA SOLO kernel), 1 = barrier.cluster kernel (panel.cuh),
 // 3 = st.async kernel (panel2.cuh) with 8 rows per lane (256 rows per CTA) wherever a cluster of it holds the panel
 int panel_factor_v(Ctx* c, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, int nb, int version) {
     using Cfg = PanelCfg<4, 16>;
-    const int maxcs = detect_max_cluster(c);
+    const int maxcs = c->max_cluster;
     if (nb == P2_NB && version != 1) {
-        static bool attr_done[64] = {};
-        if (!attr_done[c->device]) {
-            cudaFuncSetAttribute(panel2_cluster_kernel<8, false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            attr_done[c->device] = true;
-        }
         // default: the 256-rows-per-CTA kernel whenever the panel fits a cluster of it (half the FP64 work per SM and
         // column); taller panels run next to the side stream's big GEMMs, where the barrier.cluster kernel measured
         // better in situ (tools/blocked_trace.py) than a 512-row st.async kernel, although that one won stand-alone
         if (version == 0 && mp <= Panel2Cfg<8>::ROWS_PER_CTA) {
             // one CTA, no cluster exchange: ~17 us instead of 48 us per panel of up to 256 rows
-            panel2_cluster_kernel<8, false, true><<<1, P2_THREADS, 0, c->stream>>>(A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
-            LQ_CHECK_LAUNCH(c);
-            LQ_COUNT_LAUNCH(c);
-            return LQ_OK;
+            return launch<panel2_cluster_kernel<8, false, true>>(c, 1, P2_THREADS, 0, c->stream, 0, A, lda, V, ldv, T, ldt, mp,
+                                                                 (long long*)nullptr);
         }
         if (mp <= maxcs * Panel2Cfg<8>::ROWS_PER_CTA) {
             int cs = 1;
             while (cs * Panel2Cfg<8>::ROWS_PER_CTA < mp) cs *= 2;
-            return launch_cluster(c, panel2_cluster_kernel<8, false>, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
+            return launch_cluster<panel2_cluster_kernel<8, false>>(c, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, (long long*)nullptr);
         }
     }
     int cs = 1;
     while (cs * Cfg::ROWS_PER_CTA < mp && cs < maxcs) cs *= 2;
     if (cs * Cfg::ROWS_PER_CTA < mp || nb > Cfg::NBMAX) return panel_generic(c, A, lda, V, ldv, T, ldt, mp, nb);
-    return launch_cluster(c, panel_cluster_kernel<4, 16>, cs, PANEL_THREADS, A, lda, V, ldv, T, ldt, mp, nb);
+    return launch_cluster<panel_cluster_kernel<4, 16>>(c, cs, PANEL_THREADS, A, lda, V, ldv, T, ldt, mp, nb);
 }
 
 int panel_factor(Ctx* c, double* A, int lda, double* V, int ldv, double* T, int ldt, int mp, int nb) {
@@ -482,11 +419,9 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
         auto merge_block_t = [&](double* Gs) -> int {
             if (nin <= 1) return LQ_OK;
             LQ_TRY(gemm(c, true, false, kb, kb, mk, 1.0, Vb, ldv, Vb, ldv, 0.0, Gs, NB_OUT));  // G = V^T V
-            if (kb == 128) merge_t_kernel<128><<<1, 1024, MERGE_T_SMEM, c->stream>>>(Gs, NB_OUT, Tblk, NB_OUT, kb);
-            else merge_t_kernel<0><<<1, 1024, MERGE_T_SMEM, c->stream>>>(Gs, NB_OUT, Tblk, NB_OUT, kb);
-            LQ_CHECK_LAUNCH(c);
-            LQ_COUNT_LAUNCH(c);
-            return LQ_OK;
+            if (kb == 128)
+                return launch<merge_t_kernel<128>>(c, 1, 1024, MERGE_T_SMEM, c->stream, (int)MERGE_T_SMEM, Gs, NB_OUT, Tblk, NB_OUT, kb);
+            return launch<merge_t_kernel<0>>(c, 1, 1024, MERGE_T_SMEM, c->stream, (int)MERGE_T_SMEM, Gs, NB_OUT, Tblk, NB_OUT, kb);
         };
         if (!lookahead) {
             LQ_TRY(merge_block_t(G.as<double>()));
@@ -576,15 +511,6 @@ int factor_padded(Ctx* c, double* A, int lda, int m, int npad, int nfac, double*
     return LQ_OK;
 }
 
-int configure_once(Ctx* c) {
-    static bool done[64] = {};
-    if (done[c->device]) return LQ_OK;
-    LQ_CUDA(c, cudaFuncSetAttribute(merge_t_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MERGE_T_SMEM));
-    LQ_CUDA(c, cudaFuncSetAttribute(merge_t_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MERGE_T_SMEM));
-    done[c->device] = true;
-    return LQ_OK;
-}
-
 // back-substitution  R X = Y  for an upper-triangular R (n x n, ldr) and Y (n x k, ldy) in place.
 // Small systems: one thread per right-hand side.
 __global__ void __launch_bounds__(256) backsub_kernel(const double* __restrict__ R, int ldr, double* __restrict__ Y, int ldy,
@@ -645,55 +571,65 @@ __global__ void __launch_bounds__(256) singular_diag_kernel(const double* __rest
 
 // R X = Y in place (Y: n x k, ldy; k even when the tensor-core GEMM is to be used for the off-diagonal part)
 int back_substitute(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n, int k) {
-    if (n <= 256) {
-        backsub_kernel<<<std::max(1, (k + 255) / 256), 256, 0, c->stream>>>(R, ldr, Y, ldy, n, k);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-        return LQ_OK;
-    }
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(backsub_diag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BACKSUB_SMEM));
-        configured.set(c->device);
-    }
+    if (n <= 256) return launch<backsub_kernel>(c, std::max(1, (k + 255) / 256), 256, 0, c->stream, 0, R, ldr, Y, ldy, n, k);
     const int nblk = (n + 127) / 128;
     for (int b = nblk - 1; b >= 0; --b) {
         const int r0 = b * 128, nb = std::min(128, n - r0), after = n - (r0 + nb);
         if (after > 0)  // Y_b -= R[b, after] X[after]
             LQ_TRY(gemm(c, false, false, nb, k, after, -1.0, R + (size_t)r0 * ldr + r0 + nb, ldr, Y + (size_t)(r0 + nb) * ldy, ldy,
                         1.0, Y + (size_t)r0 * ldy, ldy));
-        backsub_diag_kernel<<<(k + 31) / 32, 256, BACKSUB_SMEM, c->stream>>>(R + (size_t)r0 * ldr + r0, ldr, Y + (size_t)r0 * ldy,
-                                                                            ldy, nb, k);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
+        LQ_TRY(launch<backsub_diag_kernel>(c, (k + 31) / 32, 256, BACKSUB_SMEM, c->stream, (int)BACKSUB_SMEM,
+                                           R + (size_t)r0 * ldr + r0, ldr, Y + (size_t)r0 * ldy, ldy, nb, k));
     }
     return LQ_OK;
 }
 
 }  // namespace
 
+int measure_max_cluster(Ctx* c) {
+    constexpr auto kern = panel_cluster_kernel<4, 16>;
+    LQ_TRY(set_attributes_once<kern>(c, 0, true));
+    c->max_cluster = 1;
+    for (int cs : {16, 8, 4, 2}) {
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3(cs);
+        cfg.blockDim = dim3(PANEL_THREADS);
+        cfg.dynamicSmemBytes = 0;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeClusterDimension;
+        at[0].val.clusterDim.x = cs;
+        at[0].val.clusterDim.y = 1;
+        at[0].val.clusterDim.z = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
+        int n = 0;
+        cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
+        if (e == cudaSuccess && n >= 1) {
+            c->max_cluster = cs;
+            break;
+        }
+        cudaGetLastError();
+    }
+    return LQ_OK;
+}
+
 int blocked_householder_factor(Ctx* c, double* A, int lda, int m, int n, double* V, int ldv, double* B, int ldb,
                                int nrhs) {
-    LQ_TRY(configure_once(c));
     return factor_padded(c, A, lda, m, n, n, V, ldv, B, ldb, nrhs, nullptr);
 }
 
 int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, double* R) {
     LQ_REQUIRE(c, m >= n && n >= 1, LQ_ERR_SHAPE, "householder_qr needs m >= n >= 1 (got %d x %d)", m, n);
-    LQ_TRY(configure_once(c));
     const int npad = (n + 31) / 32 * 32;
     DevBuf Aw, Vw, Qw;
     LQ_TRY(Aw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Vw.alloc(c, sizeof(double) * (size_t)m * npad));
-    pad_copy_kernel<<<grid_for(c, (long long)m * npad), 256, 0, c->stream>>>(A, n, Aw.as<double>(), npad, m, n, npad);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * npad), 256, 0, c->stream, 0, A, n, Aw.as<double>(), npad, m, n,
+                                   npad));
     LQ_CUDA(c, cudaMemsetAsync(Vw.p, 0, sizeof(double) * (size_t)m * npad, c->stream));
     Factored keep;
     LQ_TRY(factor_padded(c, Aw.as<double>(), npad, m, npad, n, Vw.as<double>(), npad, nullptr, 0, 0, &keep));
-    extract_upper_kernel<<<grid_for(c, (long long)n * n), 256, 0, c->stream>>>(Aw.as<double>(), npad, R, n);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<extract_upper_kernel>(c, grid_for(c, (long long)n * n), 256, 0, c->stream, 0, Aw.as<double>(), npad, R, n));
 
     // ---- Q = H_0 H_1 ... H_{n-1} I  (thin, m x n), block reflectors applied in reverse order
     double* Qp = Q;
@@ -713,9 +649,7 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
         W = Wx.as<double>();
         W2 = W + (size_t)NB_OUT * npad;
     }
-    set_identity_kernel<<<grid_for(c, (long long)m * ldq), 256, 0, c->stream>>>(Qp, ldq, m, ldq);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<set_identity_kernel>(c, grid_for(c, (long long)m * ldq), 256, 0, c->stream, 0, Qp, ldq, m, ldq));
     // A block reflector transforms every COLUMN of Q independently, so the columns are split into two contiguous
     // ranges that run the whole chain of applications on two streams with no synchronisation in between: the launch
     // gaps, split-K reductions and partial last waves of one range are filled by the other.  The split balances the
@@ -751,39 +685,28 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
         LQ_CUDA(c, cudaEventRecord(e1, s_side));
         LQ_CUDA(c, cudaStreamWaitEvent(s_main, e1, 0));
     }
-    if (Qp != Q) {
-        unpad_copy_kernel<<<grid_for(c, (long long)m * n), 256, 0, c->stream>>>(Qp, ldq, Q, n, m, n);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-    }
+    if (Qp != Q) return launch<unpad_copy_kernel>(c, grid_for(c, (long long)m * n), 256, 0, c->stream, 0, Qp, ldq, Q, n, m, n);
     return LQ_OK;
 }
 
 int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info) {
     LQ_REQUIRE(c, m >= n && n >= 1 && nrhs >= 1, LQ_ERR_SHAPE, "least squares needs m >= n >= 1, nrhs >= 1");
-    LQ_TRY(configure_once(c));
     const int npad = (n + 31) / 32 * 32;
     const int kpad = (nrhs + 1) / 2 * 2;
     DevBuf Aw, Vw, Bw;
     LQ_TRY(Aw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Vw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Bw.alloc(c, sizeof(double) * (size_t)m * kpad));
-    pad_copy_kernel<<<grid_for(c, (long long)m * npad), 256, 0, c->stream>>>(A, n, Aw.as<double>(), npad, m, n, npad);
-    pad_copy_kernel<<<grid_for(c, (long long)m * kpad), 256, 0, c->stream>>>(B, nrhs, Bw.as<double>(), kpad, m, nrhs, kpad);
-    LQ_CHECK_LAUNCH(c);
-    c->launches += 2;
+    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * npad), 256, 0, c->stream, 0, A, n, Aw.as<double>(), npad, m, n,
+                                   npad));
+    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * kpad), 256, 0, c->stream, 0, B, nrhs, Bw.as<double>(), kpad, m,
+                                   nrhs, kpad));
     LQ_CUDA(c, cudaMemsetAsync(Vw.p, 0, sizeof(double) * (size_t)m * npad, c->stream));
     LQ_TRY(factor_padded(c, Aw.as<double>(), npad, m, npad, n, Vw.as<double>(), npad, Bw.as<double>(), kpad, kpad, nullptr));
-    if (info) {
-        singular_diag_kernel<<<1, 256, 0, c->stream>>>(Aw.as<double>(), npad, n, info);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
-    }
+    if (info) LQ_TRY(launch<singular_diag_kernel>(c, 1, 256, 0, c->stream, 0, Aw.as<double>(), npad, n, info));
     LQ_TRY(back_substitute(c, Aw.as<double>(), npad, Bw.as<double>(), kpad, n, kpad));
-    unpad_copy_kernel<<<grid_for(c, (long long)n * nrhs), 256, 0, c->stream>>>(Bw.as<double>(), kpad, X, nrhs, n, nrhs);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<unpad_copy_kernel>(c, grid_for(c, (long long)n * nrhs), 256, 0, c->stream, 0, Bw.as<double>(), kpad, X, nrhs, n,
+                                     nrhs);
 }
 
 }  // namespace lq
@@ -807,17 +730,12 @@ int lq_debug_panel_trace(lq_ctx* h, double* A, int lda, double* V, int ldv, doub
     Ctx* c = as_ctx(h);
     if (!c) return LQ_ERR_ARG;
     LQ_CUDA(c, cudaSetDevice(c->device));
-    const int maxcs = detect_max_cluster(c);
-    LQ_REQUIRE(c, mp <= maxcs * Panel2Cfg<8>::ROWS_PER_CTA, LQ_ERR_SHAPE, "panel too tall for the traced kernel");
-    if (mp <= Panel2Cfg<8>::ROWS_PER_CTA) {  // the one-CTA kernel's stamps
-        panel2_cluster_kernel<8, true, true><<<1, P2_THREADS, 0, c->stream>>>(A, lda, V, ldv, T, ldt, mp, trace);
-        LQ_CHECK_LAUNCH(c);
-        return LQ_OK;
-    }
-    cudaFuncSetAttribute(panel2_cluster_kernel<8, true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    LQ_REQUIRE(c, mp <= c->max_cluster * Panel2Cfg<8>::ROWS_PER_CTA, LQ_ERR_SHAPE, "panel too tall for the traced kernel");
+    if (mp <= Panel2Cfg<8>::ROWS_PER_CTA)  // the one-CTA kernel's stamps
+        return launch<panel2_cluster_kernel<8, true, true>>(c, 1, P2_THREADS, 0, c->stream, 0, A, lda, V, ldv, T, ldt, mp, trace);
     int cs = 1;
     while (cs * Panel2Cfg<8>::ROWS_PER_CTA < mp) cs *= 2;
-    return launch_cluster(c, panel2_cluster_kernel<8, true>, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, trace);
+    return launch_cluster<panel2_cluster_kernel<8, true>>(c, cs, P2_THREADS, A, lda, V, ldv, T, ldt, mp, trace);
 }
 
 int lq_householder_qr_dev(lq_ctx* h, const double* A, int m, int n, double* Q, double* R) {

@@ -4,7 +4,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -58,17 +57,6 @@ void set_error(Ctx* c, const char* fmt, ...);
 
 // Diagnostic environment switches are read ONCE per call site (never on a hot path: a blocked QR issues thousands of GEMMs)
 #define LQ_ENV_ONCE(name) ([]() -> bool { static const bool v = ::getenv(name) != nullptr; return v; }())
-
-// Per-device "this kernel's attributes are set" latch.  Two host threads (two contexts) may race to the first launch:
-// both then set the (idempotent) attribute and both publish the flag -- no torn state, no lock on the hot path.
-// Devices beyond the table are simply configured on every call.
-struct DeviceLatch {
-    std::atomic<unsigned char> f[64];
-    bool test(int d) const { return d >= 0 && d < 64 && f[d].load(std::memory_order_acquire) != 0; }
-    void set(int d) {
-        if (d >= 0 && d < 64) f[d].store(1, std::memory_order_release);
-    }
-};
 
 // ------------------------------------------------------------------ device math helpers
 __device__ __forceinline__ double rcp_seed(double x) {

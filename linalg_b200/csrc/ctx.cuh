@@ -24,7 +24,7 @@ struct Ctx : lq_ctx {
     cudaDeviceProp prop{};
     int sm_count = 0;
     int max_smem = 0;        // opt-in dynamic shared memory per block
-    int max_cluster = 1;     // largest cluster size the panel kernel may use
+    int max_cluster = 1;     // largest cluster size the panel kernel may use (measure_max_cluster)
     std::string err;
     void* flush_buf = nullptr;
     long long launches = 0;
@@ -82,7 +82,5 @@ struct DevBuf {
         return static_cast<T*>(p);
     }
 };
-
-#define LQ_COUNT_LAUNCH(ctx) ((ctx)->launches++)
 
 }  // namespace lq

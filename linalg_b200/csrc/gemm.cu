@@ -409,9 +409,8 @@ int launch_generic(Ctx* c, long long M, int N, int K, double alpha, const double
         const long long mr = std::min(MAX_ROWS, M - r);
         const double* Ar = AT ? A + r : A + r * (long long)lda;
         dim3 grid((N + 31) / 32, (unsigned)((mr + 31) / 32));
-        gemm_generic_kernel<AT, BT><<<grid, 256, 0, c->stream>>>(Ar, B, C + r * (long long)ldc, mr, N, K, lda, ldb, ldc, alpha, beta);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
+        LQ_TRY((launch<gemm_generic_kernel<AT, BT>>(c, grid, 256, 0, c->stream, 0, Ar, B, C + r * (long long)ldc, mr, N, K, lda,
+                                                    ldb, ldc, alpha, beta)));
     }
     return LQ_OK;
 }
@@ -429,13 +428,6 @@ template <bool AT, bool BT>
 int launch_fast(Ctx* c, long long M, int N, int Kmain, double alpha, const double* A, int lda, const double* B, int ldb,
                 double beta, double* C, int ldc, Partials* parts = nullptr) {
     const bool skinny = AT && !BT && (M <= 64 || N <= 96);
-    auto kern = skinny ? gemm_dmma_kernel<AT, BT, AT && !BT> : gemm_dmma_kernel<AT, BT, false>;
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_dmma_kernel<AT, BT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM));
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_dmma_kernel<AT, BT, AT && !BT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_SMEM));
-        configured.set(c->device);
-    }
     const long long tm = (M + BM - 1) / BM;
     const int tn = (N + BN - 1) / BN;
     const int KT = Kmain / BK;
@@ -483,9 +475,11 @@ int launch_fast(Ctx* c, long long M, int N, int Kmain, double alpha, const doubl
     if (!AT) LQ_TRY(make_kmajor_map(c, &mapA, A, M, Kmain, lda));   // A stored M x K
     if (BT) LQ_TRY(make_kmajor_map(c, &mapB, B, N, Kmain, ldb));    // B stored N x K
     dim3 grid(tn, (unsigned)tm, splits);
-    kern<<<grid, GEMM_THREADS, GEMM_SMEM, c->stream>>>(g, mapA, mapB);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    if (skinny)
+        LQ_TRY((launch<gemm_dmma_kernel<AT, BT, AT && !BT>>(c, grid, GEMM_THREADS, GEMM_SMEM, c->stream, (int)GEMM_SMEM, g, mapA,
+                                                            mapB)));
+    else
+        LQ_TRY((launch<gemm_dmma_kernel<AT, BT, false>>(c, grid, GEMM_THREADS, GEMM_SMEM, c->stream, (int)GEMM_SMEM, g, mapA, mapB)));
     if (parts) {
         parts->splits = splits;
         parts->stride = g.split_stride;
@@ -494,9 +488,8 @@ int launch_fast(Ctx* c, long long M, int N, int Kmain, double alpha, const doubl
     if (splits > 1) {
         const long long total = M * N;
         const int blocks = (int)std::min<long long>((total + 255) / 256, (long long)c->sm_count * 8);
-        splitk_reduce_kernel<<<blocks, 256, 0, c->stream>>>(g.C, splits, g.split_stride, M, N, alpha, beta, C, ldc);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
+        return launch<splitk_reduce_kernel>(c, blocks, 256, 0, c->stream, 0, g.C, splits, g.split_stride, M, N, alpha, beta, C,
+                                            ldc);
     }
     return LQ_OK;
 }
@@ -774,11 +767,6 @@ int gemm_rank(Ctx* c, long long M, int N, int K, double alpha, const double* A, 
     // Wide outputs (4+ column tiles) and short ones stay on the generic kernel: an A-stationary walk for square block
     // updates did not beat it (23.6 vs 25.0).
     if (tn >= 4 || tm < 4) return LQ_ERR_UNSUPPORTED;
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RK_SMEM_BSTAT));
-        configured.set(c->device);
-    }
     CUtensorMap mapA;
     LQ_TRY(make_kmajor_map(c, &mapA, A, M, K, lda));
     RankArgs g;
@@ -789,10 +777,7 @@ int gemm_rank(Ctx* c, long long M, int N, int K, double alpha, const double* A, 
     while (per_fixed > 1 && tn * per_fixed > (long long)c->sm_count && tn * (per_fixed - 1) >= c->sm_count * 3 / 4)
         --per_fixed;
     dim3 grid((unsigned)tn, (unsigned)per_fixed);
-    gemm_rank_kernel<<<grid, GEMM_THREADS, RK_SMEM_BSTAT, c->stream>>>(g, mapA);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<gemm_rank_kernel>(c, grid, GEMM_THREADS, RK_SMEM_BSTAT, c->stream, (int)RK_SMEM_BSTAT, g, mapA);
 }
 
 
@@ -945,20 +930,12 @@ int gemm_update(Ctx* c, long long M, int N, int K, double alpha, const double* A
     const long long tm = (M + BM - 1) / BM;
     const int tn = (N + UBN - 1) / UBN;
     if (tm * tn < 2LL * c->sm_count) return LQ_ERR_UNSUPPORTED;  // small outputs: the split-K / one-tile paths
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(gemm_upd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)UPD_SMEM));
-        configured.set(c->device);
-    }
     CUtensorMap mapA;
     LQ_TRY(make_kmajor_map(c, &mapA, A, M, K, lda));
     UpdArgs g;
     g.B = B; g.C = C; g.M = M; g.N = N; g.K = K; g.ldb = ldb; g.ldc = ldc; g.alpha = alpha; g.overwrite = overwrite ? 1 : 0;
     dim3 grid((unsigned)tn, (unsigned)tm);
-    gemm_upd_kernel<<<grid, GEMM_THREADS, UPD_SMEM, c->stream>>>(g, mapA);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<gemm_upd_kernel>(c, grid, GEMM_THREADS, UPD_SMEM, c->stream, (int)UPD_SMEM, g, mapA);
 }
 
 int gemm(Ctx* c, bool ta, bool tb, long long M, int N, int K, double alpha, const double* A, int lda, const double* B,
@@ -1042,18 +1019,11 @@ int gemm_vtc_apply_t(Ctx* c, int kb, int nc, int mk, const double* V, int ldv, c
 
 int vtc_finish(Ctx* c, const double* partials, int splits, long long stride, int kb, int nc, const double* T, int ldt,
                bool trans_t, double* W2) {
+    // opted in once to the 128-column maximum, whatever kb the first call has
     const size_t rat_smem = ((size_t)kb * (kb + 1) + (size_t)kb * 33 + 8) * sizeof(double);
-    static DeviceLatch rat_configured;
-    if (!rat_configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(reduce_apply_t_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        (int)((128 * 129 + 128 * 33 + 8) * sizeof(double))));
-        rat_configured.set(c->device);
-    }
-    reduce_apply_t_kernel<<<(nc + 31) / 32, 1024, rat_smem, c->stream>>>(partials, splits, stride, kb, nc, T, ldt,
-                                                                       trans_t ? 1 : 0, W2);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<reduce_apply_t_kernel>(c, (nc + 31) / 32, 1024, rat_smem, c->stream,
+                                         (int)((128 * 129 + 128 * 33 + 8) * sizeof(double)), partials, splits, stride, kb, nc, T,
+                                         ldt, trans_t ? 1 : 0, W2);
 }
 
 }  // namespace lq

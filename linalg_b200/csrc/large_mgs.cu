@@ -92,25 +92,16 @@ int large_mgs_qr(Ctx* c, const double* A, int m, int n, int reorth, double* Q, d
     DevBuf At;
     LQ_TRY(At.alloc(c, sizeof(double) * (size_t)m * n));
     dim3 g1((n + 31) / 32, (m + 31) / 32);
-    transpose_kernel<<<g1, 256, 0, c->stream>>>(A, m, n, At.as<double>());
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<transpose_kernel>(c, g1, 256, 0, c->stream, 0, A, m, n, At.as<double>()));
     LQ_CUDA(c, cudaMemsetAsync(R, 0, sizeof(double) * (size_t)n * n, c->stream));
     if (info) LQ_CUDA(c, cudaMemsetAsync(info, 0, sizeof(int), c->stream));
     for (int sweep = 0; sweep <= (reorth ? 1 : 0); ++sweep) {
-        mgs_norm_kernel<<<1, 256, 0, c->stream>>>(At.as<double>(), m, n, 0, R, info);
-        LQ_COUNT_LAUNCH(c);
-        for (int j = 0; j + 1 < n; ++j) {
-            mgs_update_kernel<<<n - 1 - j, 256, 0, c->stream>>>(At.as<double>(), m, n, j, R, info);
-            LQ_COUNT_LAUNCH(c);
-        }
-        LQ_CHECK_LAUNCH(c);
+        LQ_TRY(launch<mgs_norm_kernel>(c, 1, 256, 0, c->stream, 0, At.as<double>(), m, n, 0, R, info));
+        for (int j = 0; j + 1 < n; ++j)
+            LQ_TRY(launch<mgs_update_kernel>(c, n - 1 - j, 256, 0, c->stream, 0, At.as<double>(), m, n, j, R, info));
     }
     dim3 g2((m + 31) / 32, (n + 31) / 32);
-    transpose_kernel<<<g2, 256, 0, c->stream>>>(At.as<double>(), n, m, Q);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<transpose_kernel>(c, g2, 256, 0, c->stream, 0, At.as<double>(), n, m, Q);
 }
 
 int large_lstsq_mgs(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info) {
@@ -119,10 +110,7 @@ int large_lstsq_mgs(Ctx* c, const double* A, const double* B, int m, int n, int 
     LQ_TRY(Rb.alloc(c, sizeof(double) * (size_t)n * n));
     LQ_TRY(large_mgs_qr(c, A, m, n, 0, Qb.as<double>(), Rb.as<double>(), info));
     LQ_TRY(gemm(c, true, false, n, nrhs, m, 1.0, Qb.as<double>(), n, B, nrhs, 0.0, X, nrhs));  // y = Q^T b  (qr.py:113)
-    backsub_cols_kernel<<<(nrhs + 255) / 256, 256, 0, c->stream>>>(Rb.as<double>(), n, X, nrhs);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<backsub_cols_kernel>(c, (nrhs + 255) / 256, 256, 0, c->stream, 0, Rb.as<double>(), n, X, nrhs);
 }
 
 }  // namespace lq

@@ -17,8 +17,7 @@ int lstsq_stream_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const d
     if (!lstsq_stream_kernel_supported(m, n, nrhs)) return LQ_ERR_UNSUPPORTED;
     constexpr int RPT = 16, WARPS = 4;
     const size_t smem = StreamCfg<3, RPT, WARPS>::smem_doubles(n) * sizeof(double);
-    return launch_batched<lstsq_stream_kernel<RPT, WARPS>>(c, st, batch, WARPS * 32, smem, c->max_smem, A, B, X, info, m, n,
-                                                           nrhs);
+    return launch<lstsq_stream_kernel<RPT, WARPS>>(c, batch, WARPS * 32, smem, st, c->max_smem, A, B, X, info, m, n, nrhs);
 }
 
 // ---- round 2: one warp per system, block reflectors on DMMA (lstsq_tile.cuh); n <= 64, nrhs <= 16
@@ -32,8 +31,8 @@ int lstsq_tile_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const dou
     // two 4-warp CTAs per SM: 17.4 ms (8 x 1: 17.8, 7 x 1: 19.9)
     constexpr int WARPS = 4;
     const size_t smem = (size_t)WARPS * LsTile::WARP_DOUBLES * sizeof(double);
-    return launch_batched<lstsq_tile_kernel<WARPS, 2>>(c, st, (batch + WARPS - 1) / WARPS, WARPS * 32, smem, (int)smem, A, B,
-                                                       X, info, batch, m, n, nrhs, info_mode);
+    return launch<lstsq_tile_kernel<WARPS, 2>>(c, (batch + WARPS - 1) / WARPS, WARPS * 32, smem, st, (int)smem, A, B, X, info,
+                                               batch, m, n, nrhs, info_mode);
 }
 
 }  // namespace lq

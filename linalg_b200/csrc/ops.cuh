@@ -1,6 +1,8 @@
 // Internal (device-pointer) operations shared between the translation units.
 #pragma once
 
+#include <atomic>
+
 #include "ctx.cuh"
 
 namespace lq {
@@ -27,6 +29,9 @@ int blocked_householder_factor(Ctx* c, double* A, int lda, int m, int n, double*
                                int nrhs);
 // info (device, may be null): 0, or 1 + the first column whose R[j][j] is exactly 0 (the solve is singular)
 int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info);
+// Largest cluster of the barrier.cluster panel kernel the device holds (16, 8, 4, 2 or 1) -> c->max_cluster.  One
+// occupancy query when the context is created; launches nothing.
+int measure_max_cluster(Ctx* c);
 
 // ---- large_mgs.cu: single-matrix MGS for shapes beyond one CTA's shared memory
 int large_mgs_qr(Ctx* c, const double* A, int m, int n, int reorth, double* Q, double* R, int* info);
@@ -61,21 +66,72 @@ int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R
 int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double* Q,
                          double* R, bool qr32);
 
-// Launch of a batched-family kernel on stream st.  attr_smem > 0 opts the kernel in to that many bytes of dynamic shared
-// memory before its first launch on each device.  The latch is keyed on the kernel itself, not on its type: kernels with
-// the same signature (small_hh_kernel<0> and <1>) each need their own attribute.
-template <auto Kern, typename... Args>
-int launch_batched(Ctx* c, cudaStream_t st, long long blocks, int threads, size_t smem, int attr_smem, Args... args) {
-    if (attr_smem > 0) {
-        static DeviceLatch configured;
-        if (!configured.test(c->device)) {
-            LQ_CUDA(c, cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, attr_smem));
-            configured.set(c->device);
-        }
+// ---- kernel launches.  Every kernel of the linear-algebra entry points goes through launch<Kern> (launch_cluster<Kern>
+// for one cluster of CTAs), which in this order
+//   1. sets the kernel's attributes before its first launch on each device, if any are requested;
+//   2. launches on stream st;
+//   3. checks the launch with cudaGetLastError;
+//   4. adds 1 to c->launches, the count lq_kernel_launches reports.
+// opt_in_smem: 0 requests nothing, > 0 opts the kernel in to that many bytes of dynamic shared memory, SMEM_OPT_IN_REST
+// to the device's opt-in maximum minus the kernel's static shared memory.  Cluster launches also allow cluster sizes
+// beyond the portable 8.  The latch is keyed on the kernel itself, not on its type: kernels with the same signature
+// (small_hh_kernel<0> and <1>) each need their own attribute.  Two host threads (two contexts) may race to the first
+// launch: both then set the (idempotent) attribute and both publish the flag -- no torn state, no lock on the hot path.
+// Devices beyond the table are configured on every launch.
+struct DeviceLatch {
+    std::atomic<unsigned char> f[64];
+    bool test(int d) const { return d >= 0 && d < 64 && f[d].load(std::memory_order_acquire) != 0; }
+    void set(int d) {
+        if (d >= 0 && d < 64) f[d].store(1, std::memory_order_release);
     }
-    Kern<<<(unsigned)blocks, threads, smem, st>>>(args...);
+};
+
+constexpr int SMEM_OPT_IN_REST = -1;
+
+template <auto Kern>
+int set_attributes_once(Ctx* c, int opt_in_smem, bool cluster) {
+    if (opt_in_smem == 0 && !cluster) return LQ_OK;
+    static DeviceLatch configured;
+    if (configured.test(c->device)) return LQ_OK;
+    if (opt_in_smem == SMEM_OPT_IN_REST) {
+        cudaFuncAttributes fa{};
+        LQ_CUDA(c, cudaFuncGetAttributes(&fa, Kern));
+        opt_in_smem = c->max_smem - (int)fa.sharedSizeBytes;
+    }
+    if (opt_in_smem != 0)
+        LQ_CUDA(c, cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, opt_in_smem));
+    if (cluster) LQ_CUDA(c, cudaFuncSetAttribute(Kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    configured.set(c->device);
+    return LQ_OK;
+}
+
+template <auto Kern, typename... Args>
+int launch(Ctx* c, dim3 grid, dim3 block, size_t smem, cudaStream_t st, int opt_in_smem, Args... args) {
+    LQ_TRY(set_attributes_once<Kern>(c, opt_in_smem, false));
+    Kern<<<grid, block, smem, st>>>(args...);
     LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    c->launches++;
+    return LQ_OK;
+}
+
+// one cluster of cs CTAs (threads each, no dynamic shared memory) on the context stream
+template <auto Kern, typename... Args>
+int launch_cluster(Ctx* c, int cs, int threads, Args... args) {
+    LQ_TRY(set_attributes_once<Kern>(c, 0, true));
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(cs);
+    cfg.blockDim = dim3(threads);
+    cfg.dynamicSmemBytes = 0;
+    cfg.stream = c->stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = cs;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    LQ_CUDA(c, cudaLaunchKernelEx(&cfg, Kern, args...));
+    c->launches++;
     return LQ_OK;
 }
 

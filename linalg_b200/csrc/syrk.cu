@@ -163,22 +163,14 @@ bool syrk_tn_supported(const double* A, int lda, long long m, int n) {
 // G (n x n, ldg, both triangles) = A^T A, A m x n with row stride lda
 int syrk_tn(Ctx* c, const double* A, int lda, long long m, int n, double* G, int ldg) {
     if (!syrk_tn_supported(A, lda, m, n)) return LQ_ERR_UNSUPPORTED;
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(syrk_tn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SYRK_SMEM));
-        configured.set(c->device);
-    }
     const int KT = (int)(m / SBK);
     const int splits = (int)std::min<long long>(c->sm_count, std::max(1, KT / 4));
     DevBuf W;
     LQ_TRY(W.alloc(c, sizeof(double) * (size_t)splits * 128 * 128));
-    syrk_tn_kernel<<<splits, SYRK_THREADS, SYRK_SMEM, c->stream>>>(A, lda, n, KT, W.as<double>());
-    LQ_CHECK_LAUNCH(c);
+    LQ_TRY(launch<syrk_tn_kernel>(c, splits, SYRK_THREADS, SYRK_SMEM, c->stream, (int)SYRK_SMEM, A, lda, n, KT, W.as<double>()));
     const int tail = (int)(m - (long long)KT * SBK);
-    syrk_reduce_kernel<<<n, 128, 0, c->stream>>>(W.as<double>(), splits, A + (size_t)KT * SBK * lda, lda, tail, n, G, ldg);
-    LQ_CHECK_LAUNCH(c);
-    c->launches += 2;
-    return LQ_OK;
+    return launch<syrk_reduce_kernel>(c, n, 128, 0, c->stream, 0, W.as<double>(), splits, A + (size_t)KT * SBK * lda, lda, tail, n,
+                                      G, ldg);
 }
 
 }  // namespace lq

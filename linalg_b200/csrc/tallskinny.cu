@@ -685,14 +685,7 @@ __global__ void __launch_bounds__(1024) chol_upper128_kernel(const double* __res
 
 int launch_triu_inverse(Ctx* c, const double* R, int n, double* Rinv) {
     LQ_REQUIRE(c, n <= 128, LQ_ERR_UNSUPPORTED, "triangular inverse supports n <= 128 (got %d)", n);
-    static DeviceLatch configured;
-    if (!configured.test(c->device)) {
-        LQ_CUDA(c, cudaFuncSetAttribute(triu_inverse128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 129 * 8));
-        configured.set(c->device);
-    }
-    triu_inverse128_kernel<<<8, 128, 128 * 129 * 8, c->stream>>>(R, n, Rinv);
-    LQ_CHECK_LAUNCH(c);
-    return LQ_OK;
+    return launch<triu_inverse128_kernel>(c, 8, 128, 128 * 129 * 8, c->stream, 128 * 129 * 8, R, n, Rinv);
 }
 
 
@@ -701,22 +694,6 @@ __global__ void __launch_bounds__(256) scale_cols_tall_kernel(double* __restrict
     const long long total = rows * n;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x)
         M[e] *= sgn[e % n];
-}
-
-int eigh_configure(Ctx* c) {
-    static DeviceLatch done;
-    if (done.test(c->device)) return LQ_OK;
-    cudaFuncAttributes fa{};
-    LQ_CUDA(c, cudaFuncGetAttributes(&fa, jacobi_kernel));
-    LQ_CUDA(c, cudaFuncSetAttribute(jacobi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    c->max_smem - (int)fa.sharedSizeBytes));
-    LQ_CUDA(c, cudaFuncSetAttribute(jacobi1s_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 128 * 8));
-    LQ_CUDA(c, cudaFuncSetAttribute(jacobi1s_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 128 * 8));
-    LQ_CUDA(c, cudaFuncGetAttributes(&fa, tsqr_leaf_kernel<16, 8>));
-    LQ_CUDA(c, cudaFuncSetAttribute(tsqr_leaf_kernel<16, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    c->max_smem - (int)fa.sharedSizeBytes));
-    done.set(c->device);
-    return LQ_OK;
 }
 
 // R factor (n x n upper) of A (m x n, lda) by a tree of streaming Householder reductions
@@ -743,9 +720,8 @@ int tsqr_rfactor(Ctx* c, const double* A, int lda, long long m, int n, double* R
             LQ_TRY(bufs[flip].alloc(c, sizeof(double) * (size_t)ctas * n * n));
             out = bufs[flip].as<double>();
         }
-        tsqr_leaf_kernel<16, 8><<<(unsigned)ctas, 256, smem, c->stream>>>(cur, cur_ld, cur_m, n, rpc, out);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
+        LQ_TRY((launch<tsqr_leaf_kernel<16, 8>>(c, (unsigned)ctas, 256, smem, c->stream, SMEM_OPT_IN_REST, cur, cur_ld, cur_m, n,
+                                                rpc, out)));
         if (ctas == 1) return LQ_OK;
         cur = out;
         cur_ld = n;
@@ -776,7 +752,6 @@ static unsigned small_grid(Ctx* c, int n) {
 
 int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, bool psd) {
     LQ_REQUIRE(c, n >= 1 && n <= 2048, LQ_ERR_UNSUPPORTED, "eigen-solver supports n <= 2048 (got %d)", n);
-    LQ_TRY(eigh_configure(c));
     const int max_sweeps = 40;
     // a pair is rotated while |a_pq| > rel_tol * sqrt(a_pp a_qq); 4 eps stops the tail of sweeps that only chase
     // rounding noise (eigenvalues move by O(a_pq^2 / gap), the eigenvector basis stays a product of exact rotations)
@@ -792,25 +767,24 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
         LQ_TRY(rot.alloc(c, sizeof(double2) * (size_t)(max_sweeps + 1) * jacobi1s_steps_per_sweep(ne) * 64));
         LQ_TRY(ptab.alloc(c, sizeof(unsigned short) * (size_t)jacobi1s_steps_per_sweep(ne) * 64));
         const int direct = psd ? 1 : 0;
+        const size_t smem = sizeof(double) * (size_t)ne * ne;
         if (ne == 128)
-            jacobi1s_kernel<8><<<1, 512, sizeof(double) * (size_t)ne * ne, c->stream>>>(G, n, ne, rot.as<double2>(), max_sweeps, rel_tol,
-                                                                                       nr.as<int>(), Aw.as<double>(), ptab.as<unsigned short>(), lam.as<double>(), direct);
+            LQ_TRY(launch<jacobi1s_kernel<8>>(c, 1, 512, smem, c->stream, 128 * 128 * 8, G, n, ne, rot.as<double2>(), max_sweeps,
+                                              rel_tol, nr.as<int>(), Aw.as<double>(), ptab.as<unsigned short>(), lam.as<double>(),
+                                              direct));
         else
-            jacobi1s_kernel<0><<<1, 512, sizeof(double) * (size_t)ne * ne, c->stream>>>(G, n, ne, rot.as<double2>(), max_sweeps, rel_tol,
-                                                                                       nr.as<int>(), Aw.as<double>(), ptab.as<unsigned short>(), lam.as<double>(), direct);
-        LQ_CHECK_LAUNCH(c);
-        jacobi1s_apply_kernel<<<(n + 3) / 4, 128, 0, c->stream>>>(rot.as<double2>(), nr.as<int>(), ptab.as<unsigned short>(), n, ne,
-                                                                   Vraw.as<double>());
-        LQ_CHECK_LAUNCH(c);
+            LQ_TRY(launch<jacobi1s_kernel<0>>(c, 1, 512, smem, c->stream, 128 * 128 * 8, G, n, ne, rot.as<double2>(), max_sweeps,
+                                              rel_tol, nr.as<int>(), Aw.as<double>(), ptab.as<unsigned short>(), lam.as<double>(),
+                                              direct));
+        LQ_TRY(launch<jacobi1s_apply_kernel>(c, (n + 3) / 4, 128, 0, c->stream, 0, rot.as<double2>(), nr.as<int>(),
+                                             ptab.as<unsigned short>(), n, ne, Vraw.as<double>()));
         if (direct)
-            eigvec_from_b_kernel<<<small_grid(c, n), 256, 0, c->stream>>>(Aw.as<double>(), ne, lam.as<double>(), nr.as<int>(), n, Vraw.as<double>());
-        LQ_CHECK_LAUNCH(c);
-        eig_rayleigh_kernel<<<(n + 7) / 8, 256, 0, c->stream>>>(Aw.as<double>(), ne, Vraw.as<double>(), n, lam.as<double>());
-        LQ_CHECK_LAUNCH(c);
-        eig_sort_kernel<<<small_grid(c, n), 256, sizeof(int) * n, c->stream>>>(lam.as<double>(), Vraw.as<double>(), n, lambda_desc, V);
-        LQ_CHECK_LAUNCH(c);
-        c->launches += direct ? 5 : 4;
-        return LQ_OK;
+            LQ_TRY(launch<eigvec_from_b_kernel>(c, small_grid(c, n), 256, 0, c->stream, 0, Aw.as<double>(), ne, lam.as<double>(),
+                                                nr.as<int>(), n, Vraw.as<double>()));
+        LQ_TRY(launch<eig_rayleigh_kernel>(c, (n + 7) / 8, 256, 0, c->stream, 0, Aw.as<double>(), ne, Vraw.as<double>(), n,
+                                           lam.as<double>()));
+        return launch<eig_sort_kernel>(c, small_grid(c, n), 256, sizeof(int) * n, c->stream, 0, lam.as<double>(), Vraw.as<double>(),
+                                       n, lambda_desc, V);
     }
     const int ne = (n + 1) & ~1, ld = ne | 1, half = ne / 2;
     const size_t need = ((size_t)ne * ld + 4) * sizeof(double) + (size_t)half * sizeof(double2) + 64;
@@ -818,15 +792,12 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
     LQ_TRY(Aw.alloc(c, use_global ? sizeof(double) * (size_t)ne * ld : 16));
     LQ_TRY(rot.alloc(c, sizeof(double2) * (size_t)max_sweeps * (ne - 1 > 0 ? ne - 1 : 1) * (half > 0 ? half : 1)));
     const size_t smem = use_global ? (size_t)half * sizeof(double2) + 64 : need;
-    jacobi_kernel<<<1, 1024, smem, c->stream>>>(G, n, Aw.as<double>(), use_global, rot.as<double2>(), max_sweeps, rel_tol,
-                                               nr.as<int>(), lam.as<double>());
-    LQ_CHECK_LAUNCH(c);
-    jacobi_apply_kernel<<<n, 256, sizeof(double) * (ne + 2), c->stream>>>(rot.as<double2>(), nr.as<int>(), n, ne, Vraw.as<double>());
-    LQ_CHECK_LAUNCH(c);
-    eig_sort_kernel<<<small_grid(c, n), 256, sizeof(int) * n, c->stream>>>(lam.as<double>(), Vraw.as<double>(), n, lambda_desc, V);
-    LQ_CHECK_LAUNCH(c);
-    c->launches += 3;
-    return LQ_OK;
+    LQ_TRY(launch<jacobi_kernel>(c, 1, 1024, smem, c->stream, SMEM_OPT_IN_REST, G, n, Aw.as<double>(), use_global,
+                                 rot.as<double2>(), max_sweeps, rel_tol, nr.as<int>(), lam.as<double>()));
+    LQ_TRY(launch<jacobi_apply_kernel>(c, n, 256, sizeof(double) * (ne + 2), c->stream, 0, rot.as<double2>(), nr.as<int>(), n, ne,
+                                       Vraw.as<double>()));
+    return launch<eig_sort_kernel>(c, small_grid(c, n), 256, sizeof(int) * n, c->stream, 0, lam.as<double>(), Vraw.as<double>(), n,
+                                   lambda_desc, V);
 }
 
 int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, double* U, double* s, double* Vt,
@@ -842,10 +813,8 @@ int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, doub
     LQ_TRY(gram(c, A, m, n, G.as<double>()));                                  // svd.py:42
     if (sharded) LQ_TRY(comm_allreduce_sum(c, G.as<double>(), (long long)n * n));
     LQ_TRY(eigh_jacobi(c, G.as<double>(), n, lam.as<double>(), V.as<double>(), true)); // svd.py:46-51 (G = A^T A is PSD)
-    svd_post_kernel<<<small_grid(c, n), 256, sizeof(double) * n, c->stream>>>(lam.as<double>(), V.as<double>(), n, tol, s, M2.as<double>(), Vt,
-                                                                             rk.as<int>());
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
+    LQ_TRY(launch<svd_post_kernel>(c, small_grid(c, n), 256, sizeof(double) * n, c->stream, 0, lam.as<double>(), V.as<double>(), n,
+                                   tol, s, M2.as<double>(), Vt, rk.as<int>()));
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, n, M2.as<double>(), n, 0.0, U, n));  // svd.py:61-64
     if (rank_host) {
         LQ_CUDA(c, cudaMemcpyAsync(rank_host, rk.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
@@ -858,7 +827,6 @@ int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, doub
 // Q = A R^{-1} followed by one TSQR refinement pass (restores orthogonality to O(eps) whenever
 // cond(A) * eps << 1), signs normalised so that diag(R) > 0 -- the MGS convention (qr.py:39-42).
 static int tsqr_householder(Ctx* c, const double* A, long long m, int n, double* Q, double* R, bool sharded) {
-    LQ_TRY(eigh_configure(c));
     DevBuf R1, R2, Rinv, Rall, sgn, Q1;
     const size_t nn = sizeof(double) * (size_t)n * n;
     LQ_TRY(R1.alloc(c, nn));
@@ -880,22 +848,18 @@ static int tsqr_householder(Ctx* c, const double* A, long long m, int n, double*
     // pass 1
     LQ_TRY(reduce_R(A, R1.as<double>()));
     LQ_TRY(launch_triu_inverse(c, R1.as<double>(), n, Rinv.as<double>()));
-    LQ_CHECK_LAUNCH(c);
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, n, Rinv.as<double>(), n, 0.0, Q1.as<double>(), n));
     // pass 2 (refinement)
     LQ_TRY(reduce_R(Q1.as<double>(), R2.as<double>()));
-    sign_fix_R_kernel<<<1, 256, 0, c->stream>>>(R2.as<double>(), n, sgn.as<double>());   // R2 <- S R2 (temporarily, S folded below)
-    LQ_CHECK_LAUNCH(c);
+    LQ_TRY(launch<sign_fix_R_kernel>(c, 1, 256, 0, c->stream, 0, R2.as<double>(), n, sgn.as<double>()));  // R2 <- S R2 (temporarily, S folded below)
     // we want R = S' (R2 R1) with diag > 0.  Compute R = R2 R1 first with the unsigned R2:
     //   sign_fix made diag(R2) > 0; R1's diagonal sign decides the final flip.
     LQ_TRY(gemm(c, false, false, n, n, n, 1.0, R2.as<double>(), n, R1.as<double>(), n, 0.0, R, n));
     // Q = Q1 (S R2)^{-1} ... then flip so that diag(R) > 0
     LQ_TRY(launch_triu_inverse(c, R2.as<double>(), n, Rinv.as<double>()));
-    LQ_CHECK_LAUNCH(c);
-    sign_fix_R_kernel<<<1, 256, 0, c->stream>>>(R, n, sgn.as<double>());                  // R <- S2 R
-    scale_cols_kernel<<<grid_for(c, (long long)n * n), 256, 0, c->stream>>>(Rinv.as<double>(), n, sgn.as<double>());  // Rinv <- Rinv S2
-    LQ_CHECK_LAUNCH(c);
-    c->launches += 5;
+    LQ_TRY(launch<sign_fix_R_kernel>(c, 1, 256, 0, c->stream, 0, R, n, sgn.as<double>()));  // R <- S2 R
+    LQ_TRY(launch<scale_cols_kernel>(c, grid_for(c, (long long)n * n), 256, 0, c->stream, 0, Rinv.as<double>(), n,
+                                     sgn.as<double>()));  // Rinv <- Rinv S2
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, Q1.as<double>(), n, Rinv.as<double>(), n, 0.0, Q, n));
     return LQ_OK;
 }
@@ -940,24 +904,18 @@ static int cholqr2_enqueue(Ctx* c, const double* A, int lda, long long m, int n,
                            bool sharded, CholQrScratch& w, double* stat, double short_flag) {
     double* G = w.G.as<double>();
     const bool carry = short_flag >= 0.0;
-    if (carry) {
-        tsqr_flags_kernel<<<1, 1, 0, c->stream>>>(G + (size_t)n * n, short_flag, 0.0);
-        LQ_CHECK_LAUNCH(c);
-    }
+    if (carry) LQ_TRY(launch<tsqr_flags_kernel>(c, 1, 1, 0, c->stream, 0, G + (size_t)n * n, short_flag, 0.0));
     // pass 1
     LQ_TRY(gram_ld(c, A, lda, m, n, G));
     if (sharded) LQ_TRY(comm_allreduce_sum(c, G, (long long)n * n + (carry ? 2 : 0)));
-    chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R1.as<double>(), stat);
-    LQ_CHECK_LAUNCH(c);
+    LQ_TRY(launch<chol_upper128_kernel>(c, 1, 1024, 0, c->stream, 0, G, n, w.R1.as<double>(), stat));
     LQ_TRY(launch_triu_inverse(c, w.R1.as<double>(), n, w.Rinv.as<double>()));
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, lda, w.Rinv.as<double>(), n, 0.0, w.Q1.as<double>(), n));
     // pass 2
     LQ_TRY(gram_ld(c, w.Q1.as<double>(), n, m, n, G));
     if (sharded) LQ_TRY(comm_allreduce_sum(c, G, (long long)n * n));
-    chol_upper128_kernel<<<1, 1024, 0, c->stream>>>(G, n, w.R2.as<double>(), stat + 2);
-    LQ_CHECK_LAUNCH(c);
+    LQ_TRY(launch<chol_upper128_kernel>(c, 1, 1024, 0, c->stream, 0, G, n, w.R2.as<double>(), stat + 2));
     LQ_TRY(launch_triu_inverse(c, w.R2.as<double>(), n, w.Rinv.as<double>()));
-    c->launches += 4 + (carry ? 1 : 0);
     LQ_TRY(gemm(c, false, false, n, n, n, 1.0, w.R2.as<double>(), n, w.R1.as<double>(), n, 0.0, R, ldr));
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, w.Q1.as<double>(), n, w.Rinv.as<double>(), n, 0.0, Q, ldq));
     return LQ_OK;
@@ -968,7 +926,6 @@ static int tsqr_cholqr2(Ctx* c, const double* A, long long m, int n, double* Q, 
     // the first Cholesky to look at the cond^2 estimate: a bubble in the middle of a 4 ms call).  The status words and the
     // "short rank" count ride in the first all-reduce / are computed from all-reduced data, so every rank reaches the same
     // verdict and a fallback is taken by all ranks together (ADVICE r1: the path decision must be collective).
-    LQ_TRY(eigh_configure(c));
     CholQrScratch w;
     DevBuf stat;
     LQ_TRY(w.alloc(c, m, n));
@@ -1009,7 +966,6 @@ static int tsqr_wide(Ctx* c, const double* A, long long m, int n, double* Q, dou
     const int np = (n + PB - 1) / PB;
     bool ok = !c->env_tsqr_householder && (sh || m >= 2LL * n);
     if (ok) {
-        LQ_TRY(eigh_configure(c));
         CholQrScratch w;
         DevBuf stat, S;
         LQ_TRY(w.alloc(c, m, PB));
@@ -1024,9 +980,8 @@ static int tsqr_wide(Ctx* c, const double* A, long long m, int n, double* Q, dou
                 LQ_TRY(gemm(c, true, false, c0, bk, (int)m, 1.0, Q, n, Qk, n, 0.0, S.as<double>(), bk));
                 if (sh) LQ_TRY(comm_allreduce_sum(c, S.as<double>(), (long long)c0 * bk));
                 LQ_TRY(gemm(c, false, false, m, bk, c0, -1.0, Q, n, S.as<double>(), bk, 1.0, Qk, n));
-                add_inplace_kernel<<<grid_for(c, (long long)c0 * bk), 256, 0, c->stream>>>(R + c0, n, S.as<double>(), bk, c0, bk);
-                LQ_CHECK_LAUNCH(c);
-                LQ_COUNT_LAUNCH(c);
+                LQ_TRY(launch<add_inplace_kernel>(c, grid_for(c, (long long)c0 * bk), 256, 0, c->stream, 0, R + c0, n, S.as<double>(),
+                                                  bk, c0, bk));
             }
             LQ_TRY(cholqr2_enqueue(c, Qk, n, m, bk, Qk, n, R + (size_t)c0 * n + c0, n, sh, w, stat.as<double>() + 4 * k, -1.0));
         }
@@ -1044,11 +999,8 @@ static int tsqr_wide(Ctx* c, const double* A, long long m, int n, double* Q, dou
     DevBuf sgn;
     LQ_TRY(sgn.alloc(c, sizeof(double) * n));
     LQ_TRY(blocked_householder_qr(c, A, (int)m, n, Q, R));
-    sign_fix_R_kernel<<<1, 256, 0, c->stream>>>(R, n, sgn.as<double>());
-    scale_cols_tall_kernel<<<grid_for(c, m * n), 256, 0, c->stream>>>(Q, m, n, sgn.as<double>());
-    LQ_CHECK_LAUNCH(c);
-    c->launches += 2;
-    return LQ_OK;
+    LQ_TRY(launch<sign_fix_R_kernel>(c, 1, 256, 0, c->stream, 0, R, n, sgn.as<double>()));
+    return launch<scale_cols_tall_kernel>(c, grid_for(c, m * n), 256, 0, c->stream, 0, Q, m, n, sgn.as<double>());
 }
 
 // a7: thin QR of a tall-skinny matrix with diag(R) > 0.
@@ -1072,19 +1024,15 @@ int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R
         DevBuf sgn;
         LQ_TRY(sgn.alloc(c, sizeof(double) * n));
         LQ_TRY(blocked_householder_qr(c, A, (int)m, n, Q, R));
-        sign_fix_R_kernel<<<1, 256, 0, c->stream>>>(R, n, sgn.as<double>());
-        scale_cols_tall_kernel<<<grid_for(c, m * n), 256, 0, c->stream>>>(Q, m, n, sgn.as<double>());
-        LQ_CHECK_LAUNCH(c);
-        c->launches += 2;
-        return LQ_OK;
+        LQ_TRY(launch<sign_fix_R_kernel>(c, 1, 256, 0, c->stream, 0, R, n, sgn.as<double>()));
+        return launch<scale_cols_tall_kernel>(c, grid_for(c, m * n), 256, 0, c->stream, 0, Q, m, n, sgn.as<double>());
     }
     // row-sharded and ill-conditioned: Householder reduction tree + Q = A R^{-1} with one refinement pass
     // (orthogonality O(eps), residual O(cond(A) eps)); its leaves need at least n rows on every rank
     if (!have_status) {
         DevBuf f;
         LQ_TRY(f.alloc(c, 2 * sizeof(double)));
-        tsqr_flags_kernel<<<1, 1, 0, c->stream>>>(f.as<double>(), m < n ? 1.0 : 0.0, 0.0);
-        LQ_CHECK_LAUNCH(c);
+        LQ_TRY(launch<tsqr_flags_kernel>(c, 1, 1, 0, c->stream, 0, f.as<double>(), m < n ? 1.0 : 0.0, 0.0));
         LQ_TRY(comm_allreduce_sum(c, f.as<double>(), 2));
         double h[2] = {0, 0};
         LQ_CUDA(c, cudaMemcpyAsync(h, f.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
@@ -1212,9 +1160,7 @@ static int svd_complete_impl(lq_ctx* h, double* U, int64_t m, int n, int rank, c
     LQ_CUDA(c, cudaMemcpyAsync(dU.p, U, sizeof(double) * (size_t)m * n, cudaMemcpyHostToDevice, c->stream));
     if (seeded) {
         const long long count = (long long)m * k;
-        philox_normal_kernel<<<grid_for(c, (count + 3) / 4), 256, 0, c->stream>>>(dZ.as<double>(), count, seed);
-        LQ_CHECK_LAUNCH(c);
-        LQ_COUNT_LAUNCH(c);
+        LQ_TRY(launch<philox_normal_kernel>(c, grid_for(c, (count + 3) / 4), 256, 0, c->stream, 0, dZ.as<double>(), count, seed));
     } else {
         LQ_CUDA(c, cudaMemcpyAsync(dZ.p, Z, sizeof(double) * (size_t)m * k, cudaMemcpyHostToDevice, c->stream));
     }
@@ -1243,10 +1189,8 @@ int lq_random_normal_dev(lq_ctx* h, double* out, int64_t count, uint64_t seed) {
     LQ_REQUIRE(c, count >= 0 && (count == 0 || out), LQ_ERR_ARG, "random_normal: bad arguments");
     if (count == 0) return LQ_OK;
     LQ_CUDA(c, cudaSetDevice(c->device));
-    philox_normal_kernel<<<grid_for(c, (count + 3) / 4), 256, 0, c->stream>>>(out, count, (unsigned long long)seed);
-    LQ_CHECK_LAUNCH(c);
-    LQ_COUNT_LAUNCH(c);
-    return LQ_OK;
+    return launch<philox_normal_kernel>(c, grid_for(c, (count + 3) / 4), 256, 0, c->stream, 0, out, count,
+                                        (unsigned long long)seed);
 }
 
 int lq_tsqr_dev(lq_ctx* h, const double* A, int64_t m, int n, double* Q, double* R) {

@@ -308,6 +308,18 @@ def test_householder_qr_single_matrix_routes(ctx, smem, m, n):
         check_householder(label, Ai, Q, R)
 
 
+def test_max_cluster_is_measured_when_the_context_is_created(ctx):
+    """A fresh context reports the panel kernel's largest cluster from the start, the same as one that has just run a
+    blocked QR (1000 x 1000, beyond the one-CTA kernel), and a B200 holds clusters of at least 2 CTAs."""
+    A = np.random.default_rng(1000).standard_normal((1000, 1000))
+    lb.householder_qr(A, ctx=ctx)
+    fresh = _native.Context(ctx.device)
+    try:
+        assert fresh.props()["max_cluster"] == ctx.props()["max_cluster"] >= 2
+    finally:
+        fresh.close()
+
+
 def test_householder_qr_two_column_ranges_unpadded(ctx, smem):
     """2100 x 2017: 2048 padded columns, so Q is formed in two column ranges on two streams and then unpadded.  R against
     LAPACK (mode "r"; the reference's convention equals LAPACK's here because m > n, so no last row is negated), every

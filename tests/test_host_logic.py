@@ -184,3 +184,32 @@ def test_native_environment_switches_are_the_documented_ones():
         with open(path) as fh:
             found |= set(re.findall(r"LINALG_B200_([A-Z_]+)", fh.read()))
     assert found == {"TRACE_BLOCKS", "NO_GRAPH", "TSQR_HOUSEHOLDER", "JACOBI_TWO_SIDED", "NCCL_LIB"}
+
+
+def test_every_kernel_launch_goes_through_the_counted_helper():
+    """launch / launch_cluster (ops.cuh) set a kernel's attributes once per device, launch it, check the launch and count
+    it, so lq_kernel_launches counts exactly the kernels that ran.  Only the uncounted measurement utilities of api_core.cu
+    launch directly; the launch count is otherwise written by the CUDA-graph replay alone; per-device state lives in the
+    helper's bounds-checked, atomic DeviceLatch or in the context, never in a static table indexed by the device."""
+    import glob
+    import re
+
+    src = {}
+    for path in glob.glob(os.path.join(ROOT, "linalg_b200", "csrc", "*.cu*")):
+        with open(path) as fh:
+            src[os.path.basename(path)] = fh.read()
+
+    def files_with(pattern):
+        return {name for name, text in src.items() if re.search(pattern, text)}
+
+    assert files_with(r"<<<|cudaLaunchKernelEx") == {"ops.cuh", "api_core.cu"}
+    assert files_with(r"cudaFuncSetAttribute|DeviceLatch") == {"ops.cuh"}
+    writes = {(name, m.group(0)) for name, text in src.items()
+              for m in re.finditer(r"\w+(?:->|\.)launches\s*(?:\+\+|--|[-+]=|=(?!=))[^;]*", text)}
+    assert writes == {
+        ("ops.cuh", "c->launches++"),
+        ("blocked_qr.cu", "c->launches += e->launches"),    # graph replay
+        ("blocked_qr.cu", "e->launches = c->launches - l0"),  # graph capture
+        ("blocked_qr.cu", "c->launches = l0"),              # capture failed: the plain path counts again
+    }
+    assert not files_with(r"static\s[^;(){}]*\[\s*64\s*\]")
