@@ -128,7 +128,10 @@ int lq_gram_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double* G);     
 /* Eigen-decomposition of a symmetric POSITIVE SEMI-DEFINITE matrix (the Gram / covariance matrices of svd.py:42,46 and
  * pca): eigenvalues descending, eigenvectors in the columns of V.  n <= 128: one-sided Jacobi on the columns of G (it
  * orthogonalises them, i.e. diagonalises G^2: eigenvalues of equal magnitude and opposite sign would not be separated,
- * which cannot happen for PSD input); 128 < n <= 2048: two-sided Jacobi (any symmetric matrix). */
+ * which cannot happen for PSD input); 128 < n <= 2048: two-sided Jacobi (any symmetric matrix).  Input range: any finite
+ * G whose largest |diagonal| entry is normal (2^-1022 to 2^1024); both kernels work on G scaled by a power of two to a
+ * largest diagonal entry in [1, 2), so the result scales with G, bit for bit, as long as no entry of the scaled G is
+ * subnormal. */
 int lq_eigh_dev(lq_ctx* ctx, const double* G, int n, double* lambda_desc, double* V);
 int lq_gemm_dev(lq_ctx* ctx, int transa, int transb, int64_t m, int n, int k, double alpha, const double* A,
                 int lda, const double* B, int ldb, double beta, double* C, int ldc); /* row-major C = a op(A) op(B) + b C */

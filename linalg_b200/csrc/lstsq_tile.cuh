@@ -184,7 +184,8 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                 }
                 if (t == 0 && g < j) Gs[(j & 1) * 8 + g] = d;
 
-                const double ssc = fma(x0, x0, q) + 1e-300;
+                const double ss = fma(x0, x0, q);
+                const double ssc = ss + 1e-300;
                 // y = 1 / ||[x0 ; x]||, beta = 2 / v^T v = y^2 / (1 + |x0| y); the reciprocal is seeded from the UNREFINED y
                 const double ax0 = fabs(x0);
                 double y = rsqrt_seed(ssc);
@@ -202,7 +203,10 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
                     const double e = fma(-Dn, u, 1.0);
                     u = fma(u, e, u);
                 }
-                const bool skip = nrm < kEps;  // zero column (linalg/qr.py:79-80): H = I
+                // skip only an exactly zero column: this block holds part of the column, and the rows of a skipped
+                // block would be lost (see stream_factor_block); |R_jj| ends as the full remaining norm, which the
+                // report below compares with 1e-12 (MGS) or 0 (Householder)
+                const bool skip = ss == 0.0;
                 const double alpha = copysign(nrm, x0);
                 const double v0 = skip ? 0.0 : x0 + alpha;
                 const double beta = skip ? 0.0 : (y * y) * u;

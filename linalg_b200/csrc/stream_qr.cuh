@@ -28,7 +28,12 @@ struct StreamCfg {
 };
 
 // One block step-loop over the factored columns.  r: block registers; Rs: shared R.
-template <int C, int RPT, int WARPS>
+// EXACT_ZERO_SKIP: skip a reflector only when the carried column [R_jj ; x] is exactly zero.  A block sees only part of the
+// remaining column, so it cannot apply the reference's test (remaining norm < 1e-12, linalg/qr.py:79-80) to the whole
+// column, and the rows of a skipped block would be dropped with the block: a column of norm 1.5e-12 spread over several
+// blocks would end with R_jj = 0.  Without the skip, |R_jj| ends as the full remaining norm, on which the least-squares
+// kernel's singularity report acts.
+template <int C, int RPT, int WARPS, bool EXACT_ZERO_SKIP = false>
 __device__ __forceinline__ void stream_factor_block(double (&r)[C][RPT], double* __restrict__ Rs, double* __restrict__ part,
                                                     double* __restrict__ vbuf, int nf, int lane, int warp) {
     using Cfg = StreamCfg<C, RPT, WARPS>;
@@ -96,7 +101,7 @@ __device__ __forceinline__ void stream_factor_block(double (&r)[C][RPT], double*
         const double ss = fma(x0, x0, ssb);
         double rinv;
         const double nrm = sqrt_nr_t<2>(fmax(ss, 1e-300), rinv);
-        const bool skip = nrm < kEps;  // qr.py:79-80
+        const bool skip = EXACT_ZERO_SKIP ? (ss == 0.0) : (nrm < kEps);  // qr.py:79-80
         const double alpha = copysign(nrm, x0);
         const double v0 = x0 + alpha;
         const double beta = skip ? 0.0 : rcp_nr_t<2>(nrm * fabs(v0));
@@ -164,7 +169,7 @@ __global__ void __launch_bounds__(WARPS * 32)
             const int cb = colv[2] - 64;
             r[2][ii] = (ok && cb < nrhs) ? ld_stream(Bg + (long long)row * nrhs + cb) : 0.0;
         }
-        stream_factor_block<C, RPT, WARPS>(r, Rs, part, vbuf, n, lane, warp);
+        stream_factor_block<C, RPT, WARPS, true>(r, Rs, part, vbuf, n, lane, warp);
     }
 
     if (info != nullptr && threadIdx.x == 0) {

@@ -45,7 +45,7 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
     double2* cs = reinterpret_cast<double2*>(use_global ? sm : sm + (size_t)ne * ld + (ne & 1 ? 1 : 0) + 1);
     // align cs to 16 bytes
     cs = reinterpret_cast<double2*>((reinterpret_cast<uintptr_t>(cs) + 15) & ~(uintptr_t)15);
-    __shared__ int s_rot;
+    __shared__ int s_rot, s_exp;
     __shared__ double s_scale;
     __shared__ int2 pq[1024];  // pairs of the current round (n <= 2048)
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -56,11 +56,22 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
         Am[(size_t)i * ld + j] = (i < n && j < n) ? G[(size_t)i * n + j] : 0.0;
     }
     __syncthreads();
+    // work on 2^-e G with max|diag| in [1, 2): the rotation test forms app * aqq, which would overflow from max|diag| ~ 2^512.
+    // The scaling is exact; lambda is scaled back by 2^e below.
     if (tid == 0) {
         double g = 0.0;
         for (int i = 0; i < n; ++i) g = fmax(g, fabs(Am[(size_t)i * ld + i]));
-        s_scale = g;
+        const int e = (g > 0.0 && isfinite(g)) ? ilogb(g) : 0;
+        s_exp = e;
+        s_scale = scalbn(g, -e);
     }
+    __syncthreads();
+    const int gexp = s_exp;
+    if (gexp != 0)
+        for (int e = tid; e < ne * ne; e += nt) {
+            double* a = Am + (size_t)(e / ne) * ld + e % ne;
+            *a = scalbn(*a, -gexp);
+        }
     __syncthreads();
     const double floor_abs = 4.9303806576313238e-32 * s_scale;  // eps^2 * max|diag|
 
@@ -153,7 +164,7 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
         if (nrot == 0) break;
     }
     if (tid == 0) *nrounds_out = rounds;
-    for (int i = tid; i < n; i += nt) lambda[i] = Am[(size_t)i * ld + i];
+    for (int i = tid; i < n; i += nt) lambda[i] = scalbn(Am[(size_t)i * ld + i], gexp);
 }
 
 
@@ -245,7 +256,7 @@ __global__ void __launch_bounds__(512) jacobi1s_kernel(const double* __restrict_
                                                        double* __restrict__ colnorm, int allow_direct) {
     constexpr int NUMAX = 8;
     extern __shared__ __align__(16) double Bm[];  // ne x ne, column-major
-    __shared__ int s_rot;
+    __shared__ int s_rot, s_exp;
     __shared__ double s_scale;
     const int tid = threadIdx.x, nt = blockDim.x;
     const int wid = tid >> 5, ln = tid & 31, g = ln >> 3, r8 = ln & 7;
@@ -257,11 +268,20 @@ __global__ void __launch_bounds__(512) jacobi1s_kernel(const double* __restrict_
         Bm[e] = (i < n && j < n) ? G[(size_t)j * n + i] : 0.0;  // G is symmetric: read it row-wise
     }
     __syncthreads();
+    // B = 2^-e G with max|diag| in [1, 2): the rotation test multiplies four entries (alpha beta, gamma^2), which would
+    // overflow from max|diag| ~ 2^256 and underflow below ~ 2^-256.  The scaling is exact; eig_rayleigh_kernel scales
+    // lambda back by 2^e (nsteps_out[2]).
     if (tid == 0) {
         double gmax = 0.0;
         for (int i = 0; i < n; ++i) gmax = fmax(gmax, fabs(Bm[i * ne + i]));
-        s_scale = gmax;
+        const int e = (gmax > 0.0 && isfinite(gmax)) ? ilogb(gmax) : 0;
+        s_exp = e;
+        s_scale = scalbn(gmax, -e);
+        nsteps_out[2] = e;
     }
+    __syncthreads();
+    if (s_exp != 0)
+        for (int e = tid; e < ne * ne; e += nt) Bm[e] = scalbn(Bm[e], -s_exp);
     __syncthreads();
     const double floor_abs = 4.9303806576313238e-32 * s_scale * s_scale;  // (eps * max|diag|)^2
     // the pair schedule of one sweep for the eigenvector replay: p | q << 8, 0xffff = idle slot
@@ -439,15 +459,17 @@ __global__ void __launch_bounds__(128) jacobi1s_apply_kernel(const double2* __re
     for (int j = ln; j < n; j += 32) V[(size_t)b * n + j] = row[j];
 }
 
-// lambda_i = v_i^T (G v_i) = v_i . b_i   (B = G V column-major with pitch ne; V row-major n x n, eigenvectors in columns)
+// lambda_i = 2^e v_i^T (2^-e G v_i) = 2^e v_i . b_i   (B = 2^-e G V column-major with pitch ne, e = flags[2]; V row-major
+// n x n, eigenvectors in columns)
 __global__ void __launch_bounds__(256) eig_rayleigh_kernel(const double* __restrict__ B, int ne, const double* __restrict__ V, int n,
-                                                           double* __restrict__ lambda) {
+                                                           const int* __restrict__ flags, double* __restrict__ lambda) {
     const int wid = threadIdx.x >> 5, ln = threadIdx.x & 31;
+    const int e = flags[2];
     for (int i = blockIdx.x * (blockDim.x >> 5) + wid; i < n; i += gridDim.x * (blockDim.x >> 5)) {
         double acc = 0.0;
         for (int j = ln; j < n; j += 32) acc = fma(V[(size_t)j * n + i], B[(size_t)i * ne + j], acc);
         acc = warp_sum(acc);
-        if (ln == 0) lambda[i] = acc;
+        if (ln == 0) lambda[i] = scalbn(acc, e);
     }
 }
 
@@ -782,7 +804,7 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
             LQ_TRY(launch<eigvec_from_b_kernel>(c, small_grid(c, n), 256, 0, c->stream, 0, Aw.as<double>(), ne, lam.as<double>(),
                                                 nr.as<int>(), n, Vraw.as<double>()));
         LQ_TRY(launch<eig_rayleigh_kernel>(c, (n + 7) / 8, 256, 0, c->stream, 0, Aw.as<double>(), ne, Vraw.as<double>(), n,
-                                           lam.as<double>()));
+                                           nr.as<int>(), lam.as<double>()));
         return launch<eig_sort_kernel>(c, small_grid(c, n), 256, sizeof(int) * n, c->stream, 0, lam.as<double>(), Vraw.as<double>(),
                                        n, lambda_desc, V);
     }

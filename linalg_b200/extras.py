@@ -48,6 +48,11 @@ def project_onto_colspace(A, b, *, ctx=None) -> np.ndarray:
     if b.ndim == 1:
         b = b[:, None]  # projections.py:31-32
     m, n = A.shape
+    # scale every column by a power of two to a largest entry in [0.5, 1): exact, the column space is the same, and the
+    # QR's absolute 1e-12 skip and the relative rank checks below then see a matrix of unit scale (the projection, like
+    # the reference's normal equations, does not depend on the scale of A)
+    if A.size:
+        A = np.ldexp(A, -np.frexp(np.max(np.abs(A), axis=0))[1])
     if m >= n:
         Q, R = householder_qr(A, ctx=ctx)
         d = np.abs(np.diag(R))

@@ -173,17 +173,17 @@ else:  # long double is plain double on this platform: 40 significant digits thr
     _hp_sqrt = mpmath.sqrt
 
 
-def hp_householder(A, B=None, want_q=False):
+def hp_householder(A, B=None, want_q=False, eps=orc.EPS):
     """Householder QR of A (m >= n) in extended precision with the reference's conventions (linalg/qr.py:75-97):
-    R[j, j] = -copysign(||x||, x[0]), a column with ||x|| < 1e-12 is skipped.  Returns (Q or None, R, X), X = R^-1 (Q^T B)
-    for a B, else None; rounded to float64."""
+    R[j, j] = -copysign(||x||, x[0]), a column with ||x|| < eps (the reference's 1e-12) or ||x|| == 0 is skipped.  Returns
+    (Q or None, R, X), X = R^-1 (Q^T B) for a B, else None; rounded to float64."""
     m, n = A.shape
     W = _hp(A if B is None else np.hstack([A, B]))
     refl = [None] * n
     for j in range(n):
         x = W[j:, j]
         nx = _hp_sqrt(np.sum(x * x))
-        if nx < orc.EPS:
+        if nx < eps or nx == 0:
             continue
         v = x.copy()
         v[0] += -nx if np.signbit(np.float64(x[0])) else nx
