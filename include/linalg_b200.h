@@ -139,6 +139,13 @@ int lq_gemm_dev(lq_ctx* ctx, int transa, int transb, int64_t m, int n, int k, do
 /* ---- a7: TSQR for tall-skinny matrices, diag(R) > 0 (the MGS convention) ------------------------ */
 int lq_tsqr_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double* Q, double* R);
 int lq_tsqr(lq_ctx* ctx, const double* A, int64_t m, int n, double* Q, double* R);
+/* least squares on the same pipeline: X (n, nrhs) = argmin ||A X - B||_F for A (m, n), B (m, nrhs); m < 2^31 per device.
+ * info: 0, or 1 + the first column whose R[j][j] is exactly 0 (the contract of lq_lstsq_householder_batched_info).
+ * Routes: n <= 128 and m >= 4n: CholeskyQR2 that never forms Q (G1 = A^T A -> R1, Q1 = A R1^-1, [G2 | C] = Q1^T [Q1 | B] in one
+ * pass for even n, nrhs <= 32, m >= 1024 -> R2, X = (R2 R1)^-1 R2^-T C), accepted under TSQR's cond(A)^2 < 1e10 verdict.
+ * Otherwise (ill-conditioned, m < 4n, n > 128 or TSQR_HOUSEHOLDER set) the lq_lstsq_householder_batched_info route. */
+int lq_lstsq_tsqr_dev(lq_ctx* ctx, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info);
+int lq_lstsq_tsqr(lq_ctx* ctx, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info);
 
 /* ---- multi-GPU: one process (context) per GPU, NCCL over NVLink ---------------------------------- */
 int lq_comm_unique_id(void* id128);                                     /* 128 bytes, from rank 0 */
@@ -150,6 +157,13 @@ int lq_comm_allgather(lq_ctx* ctx, const double* dsend, double* drecv, int64_t c
 int lq_tsqr_sharded_dev(lq_ctx* ctx, const double* A_local, int64_t m_local, int n, double* Q_local, double* R);
 int lq_svd_gram_sharded_dev(lq_ctx* ctx, const double* A_local, int64_t m_local, int n, double tol, double* U_local,
                             double* s, double* Vt, int* rank_host);
+/* row-sharded least squares, n <= 128: every rank passes its (m_local, n) block of A and (m_local, nrhs) block of B; X (n, nrhs)
+ * and info come back replicated, bitwise identical on every rank.  CholeskyQR2 as in lq_lstsq_tsqr_dev (one all-reduce per
+ * pass); when its verdict fails or TSQR_HOUSEHOLDER is set, the Householder reduction tree of [A_local | B_local] with an
+ * all-gather of the local R factors, whose top n rows are [R | Q^T B] (needs n + nrhs <= 128 and m_local >= n + nrhs on every
+ * rank; otherwise every rank returns the same error). */
+int lq_lstsq_tsqr_sharded_dev(lq_ctx* ctx, const double* A_local, int64_t m_local, int n, const double* B_local, int nrhs,
+                              double* X, int32_t* info);
 
 /* ---- roofline probes (bench.py) --------------------------------------------------------------------- */
 /* kind 0: FP64 FMA (DFMA) peak, 1: FP64 tensor (DMMA m16n8k8) peak, 3: both pipes mixed [TFLOP/s];

@@ -16,6 +16,7 @@ from .qr import (
     least_squares_householder_qr_batched,
     least_squares_qr,
     least_squares_qr_batched,
+    least_squares_tsqr,
     qr,
     qr_batched,
     random_nonsingular_qr,
@@ -38,6 +39,7 @@ __all__ = [
     "least_squares_qr_batched",
     "least_squares_householder_qr_batched",
     "tsqr",
+    "least_squares_tsqr",
     "Context",
     "default_context",
     "pinned_empty",

@@ -68,6 +68,8 @@ SIGNATURES = {
                               C.c_int, C.c_double, _DP, C.c_int]),
     "lq_tsqr_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, _DP]),
     "lq_tsqr": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, _DP]),
+    "lq_lstsq_tsqr_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, C.c_int, _DP, C.c_void_p]),
+    "lq_lstsq_tsqr": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, C.c_int, _DP, C.c_void_p]),
     "lq_comm_unique_id": (C.c_int, [C.c_void_p]),
     "lq_comm_init": (C.c_int, [_CTX, C.c_int, C.c_int, C.c_void_p]),
     "lq_comm_destroy": (C.c_int, [_CTX]),
@@ -76,6 +78,7 @@ SIGNATURES = {
     "lq_tsqr_sharded_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, _DP]),
     "lq_svd_gram_sharded_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_double, _DP, _DP, _DP,
                                           C.POINTER(C.c_int)]),
+    "lq_lstsq_tsqr_sharded_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, _DP, C.c_int, _DP, C.c_void_p]),
     "lq_probe": (C.c_int, [_CTX, C.c_int, C.POINTER(C.c_double)]),
     "lq_debug_panel_trace": (C.c_int, [_CTX, _DP, C.c_int, _DP, C.c_int, _DP, C.c_int, C.c_int, C.c_void_p]),
     "lq_debug_panel": (C.c_int, [_CTX, _DP, C.c_int, _DP, C.c_int, _DP, C.c_int, C.c_int, C.c_int, C.c_int]),

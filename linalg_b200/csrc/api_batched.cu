@@ -54,7 +54,7 @@ int mgs_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long ba
 // info (device, may be null): per system 0, or 1 + the first column whose R[j][j] is exactly 0 (np.linalg.solve raises
 // LinAlgError("Singular matrix") there, linalg/qr.py:134); every route writes it
 int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
-                            int nrhs, double* X, int* info = nullptr) {
+                            int nrhs, double* X, int* info) {
     if (batch == 0) return LQ_OK;
     int rc = lstsq_tile_kernel_launch(c, st, A, B, batch, m, n, nrhs, X, info, 2);
     if (rc != LQ_ERR_UNSUPPORTED) return rc;

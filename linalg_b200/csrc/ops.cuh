@@ -51,6 +51,10 @@ int lstsq_tile_kernel_launch(Ctx* c, cudaStream_t st, const double* A, const dou
 
 // ---- syrk.cu: G (n x n, both triangles) = A^T A for n <= 128, upper-triangle blocks only; LQ_ERR_UNSUPPORTED otherwise
 int syrk_tn(Ctx* c, const double* A, int lda, long long m, int n, double* G, int ldg);
+// G (n x n, both triangles) = Q^T Q and C (n x nrhs) = Q^T B in one pass (Q m x n, B m x nrhs, densely packed).  Taken for
+// even n <= 128, even nrhs <= 32, m >= 1024 and 16-byte aligned Q and B (syrk_strip_supported); LQ_ERR_UNSUPPORTED otherwise.
+bool syrk_strip_supported(const double* Q, long long m, int n, const double* B, int nrhs);
+int syrk_strip_tn(Ctx* c, const double* Q, long long m, int n, const double* B, int nrhs, double* G, double* C);
 
 // ---- tallskinny.cu
 int gram(Ctx* c, const double* A, long long m, int n, double* G);  // G = A^T A
@@ -60,11 +64,17 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
 int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, double* U, double* s, double* Vt,
                    int* rank_host, bool sharded);
 int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R, bool sharded);
+// min ||A X - B|| for a tall-skinny A (m x n) and B (m x nrhs): CholeskyQR2 pipeline, Householder fallbacks.  info (device):
+// 0, or 1 + the first column whose R[j][j] is exactly 0
+int lstsq_tsqr_local(Ctx* c, const double* A, long long m, int n, const double* B, int nrhs, double* X, int* info, bool sharded);
 
 // ---- batched (api_batched.cu).  qr32: 32 x 32 matrices go to the batched 32 x 32 kernel; false keeps them on the
 // one-CTA kernel (the single-matrix entry point)
 int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double* Q,
                          double* R, bool qr32);
+// info (device, may be null): per system 0, or 1 + the first column whose R[j][j] is exactly 0
+int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
+                            int nrhs, double* X, int* info = nullptr);
 
 // ---- kernel launches.  Every kernel of the linear-algebra entry points goes through launch<Kern> (launch_cluster<Kern>
 // for one cluster of CTAs), which in this order

@@ -1,5 +1,6 @@
-// K5: tall-skinny paths -- Gram matrix, symmetric eigen-solver, economy SVD (linalg/svd.py:10-82)
-// and TSQR (SURVEY.md section 8 row a7), with the NCCL exchange steps of the row-sharded variants.
+// K5: tall-skinny paths -- Gram matrix, symmetric eigen-solver, economy SVD (linalg/svd.py:10-82),
+// TSQR (SURVEY.md section 8 row a7) and least squares on the TSQR pipeline, with the NCCL exchange steps of the row-sharded
+// variants.
 #include <algorithm>
 #include <vector>
 
@@ -1066,6 +1067,169 @@ int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R
     return tsqr_householder(c, A, m, n, Q, R, sharded);
 }
 
+// ------------------------------------------------------------------ least squares on the tall-skinny pipeline
+// Bp (m x (nrhs + 1)) = [B | 0]: an odd right-hand-side count padded to the even width of the strip kernel's bulk copies
+__global__ void __launch_bounds__(256) pad_rhs_kernel(const double* __restrict__ B, int nrhs, long long m, double* __restrict__ Bp) {
+    const int kp = nrhs + 1;
+    const long long total = m * kp;
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        const long long i = e / kp;
+        const int k = (int)(e - i * kp);
+        Bp[e] = k < nrhs ? B[i * nrhs + k] : 0.0;
+    }
+}
+
+// X (n x nrhs) = R^-1 y from the top n rows [R | y] (pitch ld) of the R factor of [A | B]; info = 0, or 1 + the first j with
+// R[j][j] exactly 0 (X is then not meaningful)
+__global__ void __launch_bounds__(128) backsub_aug_kernel(const double* __restrict__ Rf, int ld, int n, int nrhs,
+                                                          double* __restrict__ X, int* __restrict__ info) {
+    if (threadIdx.x == 0) {
+        int bad = 0;
+        for (int j = 0; j < n && !bad; ++j)
+            if (Rf[(size_t)j * ld + j] == 0.0) bad = j + 1;
+        *info = bad;
+    }
+    for (int k = threadIdx.x; k < nrhs; k += blockDim.x)
+        for (int i = n - 1; i >= 0; --i) {
+            double s = Rf[(size_t)i * ld + n + k];
+            for (int j = i + 1; j < n; ++j) s = fma(-Rf[(size_t)i * ld + j], X[(size_t)j * nrhs + k], s);
+            X[(size_t)i * nrhs + k] = s / Rf[(size_t)i * ld + i];
+        }
+}
+
+// [G | C] = Q^T [Q | B] (G n x n, C n x nrhs): the strip kernel where its shape rules allow it (an odd nrhs < 32 is padded with a
+// zero column first), the SYRK or GEMM Gram matrix and a TN GEMM otherwise
+static int gram_rhs(Ctx* c, const double* Q, long long m, int n, const double* B, int nrhs, double* G, double* C) {
+    // (Q stands in for the padded copy of B in the check: both are 16-byte aligned workspace)
+    if (nrhs % 2 == 1 && syrk_strip_supported(Q, m, n, Q, nrhs + 1)) {
+        const int kp = nrhs + 1;
+        DevBuf Bp, Cp;
+        LQ_TRY(Bp.alloc(c, sizeof(double) * (size_t)m * kp));
+        LQ_TRY(Cp.alloc(c, sizeof(double) * (size_t)n * kp));
+        LQ_TRY(launch<pad_rhs_kernel>(c, grid_for(c, m * kp), 256, 0, c->stream, 0, B, nrhs, m, Bp.as<double>()));
+        LQ_TRY(syrk_strip_tn(c, Q, m, n, Bp.as<double>(), kp, G, Cp.as<double>()));
+        LQ_CUDA(c, cudaMemcpy2DAsync(C, sizeof(double) * nrhs, Cp.p, sizeof(double) * kp, sizeof(double) * nrhs, (size_t)n,
+                                     cudaMemcpyDeviceToDevice, c->stream));
+        return LQ_OK;
+    }
+    const int rc = syrk_strip_tn(c, Q, m, n, B, nrhs, G, C);
+    if (rc != LQ_ERR_UNSUPPORTED) return rc;
+    LQ_TRY(gram_ld(c, Q, n, m, n, G));
+    return gemm(c, true, false, n, nrhs, (int)m, 1.0, Q, n, B, nrhs, 0.0, C, nrhs);
+}
+
+// CholeskyQR2 least squares (n <= 128), never forming Q:
+//   G1 = A^T A (+ all-reduce) -> R1 = chol(G1) -> Q1 = A R1^-1
+//   [G2 | C] = Q1^T [Q1 | B] (+ one all-reduce of the packed buffer) -> R2 = chol(G2)
+//   X = (R2 R1)^-1 R2^-T C = R1^-1 R2^-1 R2^-T C
+// Everything is queued before the one read-back of the status words (cholqr2_enqueue's verdict).  CholeskyQR2 of [A | B] would
+// break down for every consistent system (zero residual: [A | B] is rank deficient), so B only enters the second pass.
+static int lstsq_cholqr2(Ctx* c, const double* A, long long m, int n, const double* B, int nrhs, double* X, bool sh,
+                         double short_flag, CholQrStatus* st) {
+    const size_t nn = sizeof(double) * (size_t)n * n, nk = sizeof(double) * (size_t)n * nrhs;
+    DevBuf G1, GC, R1, R2, R1inv, R2inv, Q1, Y, Z, stat;
+    LQ_TRY(G1.alloc(c, nn + 2 * sizeof(double)));
+    LQ_TRY(GC.alloc(c, nn + nk));
+    LQ_TRY(R1.alloc(c, nn));
+    LQ_TRY(R2.alloc(c, nn));
+    LQ_TRY(R1inv.alloc(c, nn));
+    LQ_TRY(R2inv.alloc(c, nn));
+    LQ_TRY(Q1.alloc(c, sizeof(double) * (size_t)m * n));
+    LQ_TRY(Y.alloc(c, nk));
+    LQ_TRY(Z.alloc(c, nk));
+    LQ_TRY(stat.alloc(c, 4 * sizeof(double)));
+    double* G = G1.as<double>();
+    double* G2 = GC.as<double>();
+    double* C = G2 + (size_t)n * n;
+    // pass 1; the short-rank flag rides in the two spare words behind G1
+    LQ_TRY(launch<tsqr_flags_kernel>(c, 1, 1, 0, c->stream, 0, G + (size_t)n * n, short_flag, 0.0));
+    LQ_TRY(gram_ld(c, A, n, m, n, G));
+    if (sh) LQ_TRY(comm_allreduce_sum(c, G, (long long)n * n + 2));
+    LQ_TRY(launch<chol_upper128_kernel>(c, 1, 1024, 0, c->stream, 0, G, n, R1.as<double>(), stat.as<double>()));
+    LQ_TRY(launch_triu_inverse(c, R1.as<double>(), n, R1inv.as<double>()));
+    LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, n, R1inv.as<double>(), n, 0.0, Q1.as<double>(), n));
+    // pass 2
+    LQ_TRY(gram_rhs(c, Q1.as<double>(), m, n, B, nrhs, G2, C));
+    if (sh) LQ_TRY(comm_allreduce_sum(c, G2, (long long)n * (n + nrhs)));
+    LQ_TRY(launch<chol_upper128_kernel>(c, 1, 1024, 0, c->stream, 0, G2, n, R2.as<double>(), stat.as<double>() + 2));
+    LQ_TRY(launch_triu_inverse(c, R2.as<double>(), n, R2inv.as<double>()));
+    // the n x nrhs tail
+    LQ_TRY(gemm(c, true, false, n, nrhs, n, 1.0, R2inv.as<double>(), n, C, nrhs, 0.0, Y.as<double>(), nrhs));
+    LQ_TRY(gemm(c, false, false, n, nrhs, n, 1.0, R2inv.as<double>(), n, Y.as<double>(), nrhs, 0.0, Z.as<double>(), nrhs));
+    LQ_TRY(gemm(c, false, false, n, nrhs, n, 1.0, R1inv.as<double>(), n, Z.as<double>(), nrhs, 0.0, X, nrhs));
+    double h[6] = {0, 0, 0, 0, 0, 0};
+    LQ_CUDA(c, cudaMemcpyAsync(h, stat.p, 4 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    LQ_CUDA(c, cudaMemcpyAsync(h + 4, G + (size_t)n * n, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
+    st->chol1_bad = h[0];
+    st->cond2 = (h[1] == h[1]) ? h[1] : 1e300;  // NaN -> ill-conditioned
+    st->chol2_bad = h[2];
+    st->cond2_pass2 = h[3];
+    st->ranks_short = h[4];
+    return LQ_OK;
+}
+
+// Row-sharded fallback (communication-avoiding least squares): the Householder reduction tree of [A_local | B_local], the
+// all-gathered local R factors reduced again; the top n rows of the result are [R | Q^T B].  Backward stable for any cond(A).
+static int lstsq_tree_sharded(Ctx* c, const double* A, long long m, int n, const double* B, int nrhs, double* X, int* info) {
+    const int w = n + nrhs;
+    const size_t ww = sizeof(double) * (size_t)w * w;
+    DevBuf AB, Rloc, Rall, Rf;
+    LQ_TRY(AB.alloc(c, sizeof(double) * (size_t)m * w));
+    LQ_TRY(Rloc.alloc(c, ww));
+    LQ_TRY(Rall.alloc(c, ww * c->nranks));
+    LQ_TRY(Rf.alloc(c, ww));
+    LQ_CUDA(c, cudaMemcpy2DAsync(AB.p, sizeof(double) * w, A, sizeof(double) * n, sizeof(double) * n, (size_t)m,
+                                 cudaMemcpyDeviceToDevice, c->stream));
+    LQ_CUDA(c, cudaMemcpy2DAsync(AB.as<double>() + n, sizeof(double) * w, B, sizeof(double) * nrhs, sizeof(double) * nrhs,
+                                 (size_t)m, cudaMemcpyDeviceToDevice, c->stream));
+    LQ_TRY(tsqr_rfactor(c, AB.as<double>(), w, m, w, Rloc.as<double>()));
+    LQ_TRY(comm_allgather(c, Rloc.as<double>(), Rall.as<double>(), (long long)w * w));
+    LQ_TRY(tsqr_rfactor(c, Rall.as<double>(), w, (long long)c->nranks * w, w, Rf.as<double>()));
+    return launch<backsub_aug_kernel>(c, 1, 128, 0, c->stream, 0, Rf.as<double>(), w, n, nrhs, X, info);
+}
+
+int lstsq_tsqr_local(Ctx* c, const double* A, long long m, int n, const double* B, int nrhs, double* X, int* info, bool sharded) {
+    const bool sh = sharded && c->nranks > 1;
+    // as in tsqr_local, a row-sharded call validates only what every rank sees alike; the rank-local row count goes through the
+    // all-reduced "short rank" count
+    LQ_REQUIRE(c, n >= 1 && nrhs >= 1 && m >= 1 && (sh || m >= n), LQ_ERR_SHAPE,
+               "lstsq_tsqr needs m >= n >= 1 and nrhs >= 1 (got %lld x %d, %d rhs)", m, n, nrhs);
+    LQ_REQUIRE(c, m < (1LL << 31), LQ_ERR_SHAPE, "lstsq_tsqr: more than 2^31 rows per device not supported");
+    LQ_REQUIRE(c, A && B && X && info, LQ_ERR_ARG, "lstsq_tsqr: null pointer");
+    LQ_REQUIRE(c, !sh || n <= 128, LQ_ERR_UNSUPPORTED, "lstsq_tsqr (sharded) supports n <= 128 (got %d)", n);
+    const int w = n + nrhs;
+    CholQrStatus st;
+    bool have_status = false;
+    if (n <= 128 && !c->env_tsqr_householder && (sh || m >= 4LL * n)) {
+        LQ_TRY(lstsq_cholqr2(c, A, m, n, B, nrhs, X, sh, m < w ? 1.0 : 0.0, &st));
+        if (st.ok()) {
+            LQ_CUDA(c, cudaMemsetAsync(info, 0, sizeof(int), c->stream));
+            return LQ_OK;
+        }
+        have_status = true;
+    }
+    // one GPU: the Householder least-squares route of lq_lstsq_householder_batched_info (any n, any conditioning)
+    if (!sh) return lstsq_hh_batched_stream(c, c->stream, A, B, 1, (int)m, n, nrhs, X, info);
+    LQ_REQUIRE(c, w <= 128, LQ_ERR_UNSUPPORTED,
+               "lstsq_tsqr (sharded, n + nrhs = %d > 128): too ill-conditioned for CholeskyQR2, and the reflector tree of [A | B] "
+               "supports n + nrhs <= 128", w);
+    if (!have_status) {
+        DevBuf f;
+        LQ_TRY(f.alloc(c, 2 * sizeof(double)));
+        LQ_TRY(launch<tsqr_flags_kernel>(c, 1, 1, 0, c->stream, 0, f.as<double>(), m < w ? 1.0 : 0.0, 0.0));
+        LQ_TRY(comm_allreduce_sum(c, f.as<double>(), 2));
+        double h[2] = {0, 0};
+        LQ_CUDA(c, cudaMemcpyAsync(h, f.p, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+        LQ_CUDA(c, cudaStreamSynchronize(c->stream));
+        st.ranks_short = h[0];
+    }
+    LQ_REQUIRE(c, st.ranks_short == 0.0, LQ_ERR_SHAPE,
+               "lstsq_tsqr (sharded, reflector path): %d rank(s) hold fewer than n + nrhs = %d rows; re-shard the rows",
+               (int)st.ranks_short, w);
+    return lstsq_tree_sharded(c, A, m, n, B, nrhs, X, info);
+}
+
 
 // ------------------------------------------------------------------ counter-based standard-normal generator
 // Philox4x32-10 (Salmon et al., SC'11: counter = element group, key = seed) + Box-Muller; four doubles per counter.
@@ -1241,6 +1405,40 @@ int lq_tsqr(lq_ctx* h, const double* A, int64_t m, int n, double* Q, double* R) 
     LQ_TRY(tsqr_local(c, dA.as<double>(), m, n, dQ.as<double>(), dR.as<double>(), false));
     LQ_CUDA(c, cudaMemcpyAsync(Q, dQ.p, mn, cudaMemcpyDeviceToHost, c->stream));
     LQ_CUDA(c, cudaMemcpyAsync(R, dR.p, nn, cudaMemcpyDeviceToHost, c->stream));
+    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
+    return LQ_OK;
+}
+
+int lq_lstsq_tsqr_dev(lq_ctx* h, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info) {
+    Ctx* c = as_ctx(h);
+    if (!c) return LQ_ERR_ARG;
+    LQ_CUDA(c, cudaSetDevice(c->device));
+    return lstsq_tsqr_local(c, A, m, n, B, nrhs, X, info, false);
+}
+int lq_lstsq_tsqr_sharded_dev(lq_ctx* h, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info) {
+    Ctx* c = as_ctx(h);
+    if (!c) return LQ_ERR_ARG;
+    LQ_CUDA(c, cudaSetDevice(c->device));
+    return lstsq_tsqr_local(c, A, m, n, B, nrhs, X, info, true);
+}
+int lq_lstsq_tsqr(lq_ctx* h, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info) {
+    Ctx* c = as_ctx(h);
+    if (!c) return LQ_ERR_ARG;
+    LQ_REQUIRE(c, m >= n && n >= 1 && nrhs >= 1 && m < (1LL << 31), LQ_ERR_SHAPE,
+               "lstsq_tsqr needs 2^31 > m >= n >= 1 and nrhs >= 1 (got %lld x %d, %d rhs)", (long long)m, n, nrhs);
+    LQ_REQUIRE(c, A && B && X && info, LQ_ERR_ARG, "lstsq_tsqr: null pointer");
+    LQ_CUDA(c, cudaSetDevice(c->device));
+    const size_t mn = sizeof(double) * (size_t)m * n, mk = sizeof(double) * (size_t)m * nrhs, nk = sizeof(double) * (size_t)n * nrhs;
+    DevBuf dA, dB, dX, dI;
+    LQ_TRY(dA.alloc(c, mn));
+    LQ_TRY(dB.alloc(c, mk));
+    LQ_TRY(dX.alloc(c, nk));
+    LQ_TRY(dI.alloc(c, 16));
+    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
+    LQ_CUDA(c, cudaMemcpyAsync(dB.p, B, mk, cudaMemcpyHostToDevice, c->stream));
+    LQ_TRY(lstsq_tsqr_local(c, dA.as<double>(), m, n, dB.as<double>(), nrhs, dX.as<double>(), dI.as<int>(), false));
+    LQ_CUDA(c, cudaMemcpyAsync(X, dX.p, nk, cudaMemcpyDeviceToHost, c->stream));
+    LQ_CUDA(c, cudaMemcpyAsync(info, dI.p, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
     LQ_CUDA(c, cudaStreamSynchronize(c->stream));
     return LQ_OK;
 }

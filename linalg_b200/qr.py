@@ -221,6 +221,26 @@ def tsqr(A, *, ctx=None) -> Tuple[np.ndarray, np.ndarray]:
     return Q, R
 
 
+def least_squares_tsqr(A, b, *, ctx=None) -> np.ndarray:
+    """min ||Ax - b||_2 for a tall-skinny A on the TSQR pipeline (CholeskyQR2 that never forms Q, Householder least squares
+    when A is ill-conditioned, nearly square or wider than 128 columns).  The contract of ``least_squares_householder_qr``:
+    (n,) for a vector b, (n, k) for a matrix; m < n raises ``ValueError``; an exactly singular R raises
+    ``np.linalg.LinAlgError("Singular matrix")``."""
+    A = as_f64_matrix(A)
+    m, n = A.shape
+    if m < n:
+        raise ValueError(f"least_squares_tsqr needs m >= n, got {m} x {n}")
+    B, was_vec = _rhs_2d(b, m)
+    k = B.shape[1]
+    X = np.empty((n, k))
+    info = np.zeros(1, dtype=np.int32)
+    if n and k:
+        _ctx(ctx).call("lq_lstsq_tsqr", _ptr(A), m, n, _ptr(B), k, _ptr(X), _ptr(info))
+    if info[0] != 0:
+        raise np.linalg.LinAlgError("Singular matrix")
+    return X.reshape(n) if was_vec else X
+
+
 def random_nonsingular_qr(n, seed=None, *, ctx=None) -> np.ndarray:
     """Random orthogonal x random non-zero column scales (reference linalg/qr.py:137-154)."""
     rng = np.random.default_rng(seed)
