@@ -114,6 +114,14 @@ int lq_svd_gram_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double tol, 
                     int* rank_host);
 int lq_svd_gram(lq_ctx* ctx, const double* A, int64_t m, int n, double tol, double* U, double* s, double* Vt,
                 int* rank_host);
+/* the same for every matrix of a batch: A (batch, m, n) -> U (batch, m, n), s (batch, n), Vt (batch, n, n), rank (batch)
+ * for m >= n >= 1; U columns beyond rank are left ZERO (completed by the shim, as for lq_svd_gram).  n <= 32 and
+ * m <= 4096: one warp per matrix (two-sided Jacobi on the scaled Gram matrix, the rotation test of the single path);
+ * other shapes: lq_svd_gram matrix by matrix, bit for bit.  The route depends on (m, n) only. */
+int lq_svd_gram_batched_dev(lq_ctx* ctx, const double* A, int64_t batch, int m, int n, double tol, double* U, double* s,
+                            double* Vt, int32_t* rank);            /* device pointers */
+int lq_svd_gram_batched(lq_ctx* ctx, const double* A, int64_t batch, int m, int n, double tol, double* U, double* s,
+                        double* Vt, int32_t* rank);                /* host pointers: the two-lane chunked pipeline */
 /* svd.py:67-76: complete U (HOST, m x n, first `rank` columns valid) with an orthonormal basis of the
  * complement built from the caller-drawn candidates Z (HOST, m x (n - rank)); all arithmetic on device. */
 int lq_svd_complete(lq_ctx* ctx, double* U, int64_t m, int n, int rank, const double* Z);

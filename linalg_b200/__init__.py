@@ -22,7 +22,7 @@ from .qr import (
     random_nonsingular_qr,
     tsqr,
 )
-from .svd import svd
+from .svd import svd, svd_batched
 from .extras import adj, adj_batched, det, det_batched, pca, project_onto_colspace, random_nonsingular_qr_batched
 from .utils import EPS, shard_bounds
 
@@ -33,6 +33,7 @@ __all__ = [
     "least_squares_householder_qr",
     "random_nonsingular_qr",
     "svd",
+    "svd_batched",
     "EPS",
     "qr_batched",
     "householder_qr_batched",

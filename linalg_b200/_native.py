@@ -59,6 +59,8 @@ SIGNATURES = {
     "lq_lstsq_mgs_batched": (C.c_int, [_CTX, _DP, _DP, C.c_int64, C.c_int, C.c_int, C.c_int, _DP, C.c_void_p]),
     "lq_svd_gram_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_int)]),
     "lq_svd_gram": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_int)]),
+    "lq_svd_gram_batched_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.c_void_p]),
+    "lq_svd_gram_batched": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.c_void_p]),
     "lq_svd_complete": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_int, _DP]),
     "lq_svd_complete_seeded": (C.c_int, [_CTX, _DP, C.c_int64, C.c_int, C.c_int, C.c_uint64]),
     "lq_random_normal_dev": (C.c_int, [_CTX, _DP, C.c_int64, C.c_uint64]),

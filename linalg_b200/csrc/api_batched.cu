@@ -1,10 +1,11 @@
-// Batched QR / least-squares entry points (a1-a4 of SURVEY.md section 8).
+// Batched QR / least-squares / SVD entry points (a1-a5 of SURVEY.md section 8).
 #include <algorithm>
 
 #include "../../include/linalg_b200.h"
 #include "batched_qr32.cuh"
 #include "batched_qr32_c8.cuh"
 #include "batched_small.cuh"
+#include "batched_svd_small.cuh"
 #include "ctx.cuh"
 #include "ops.cuh"
 
@@ -88,6 +89,24 @@ int lstsq_mgs_batched_stream(Ctx* c, cudaStream_t st, const double* A, const dou
     return LQ_OK;
 }
 
+// rank (device): #(s > tol) per matrix.  The route depends on (m, n) only, so a matrix's result does not depend on the batch
+// it is in: the warp-per-matrix kernel, or the single-matrix pipeline matrix by matrix (bitwise svd(A[b]); stream `st` must
+// then be the context stream).
+int svd_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double tol, double* U,
+                       double* s, double* Vt, int* rank) {
+    if (batch == 0) return LQ_OK;
+    if (svd_small_supported(m, n)) {
+        constexpr int WARPS = 4;
+        const size_t smem = (size_t)WARPS * SvdSmall::WARP_DOUBLES * sizeof(double);
+        return launch<svd_small_kernel<WARPS>>(c, (batch + WARPS - 1) / WARPS, WARPS * 32, smem, st, (int)smem, A, batch, m, n,
+                                               tol, U, s, Vt, rank);
+    }
+    for (long long b = 0; b < batch; ++b)
+        LQ_TRY(svd_gram_local(c, A + b * (long long)m * n, m, n, tol, U + b * (long long)m * n, s + b * (long long)n,
+                              Vt + b * (long long)n * n, nullptr, false, rank + b));
+    return LQ_OK;
+}
+
 // ------------------------------------------------------------------ host-pointer pipelines
 // Chunks of the batch flow through two lanes (stream + device buffers each): H2D, kernel and D2H
 // of neighbouring chunks overlap on the copy engines.  With pinned host buffers the copies are
@@ -98,19 +117,21 @@ static long long pick_chunk(long long batch, size_t bytes_per_item) {
     return std::min(batch, ch);
 }
 
+// out_c / hOc: a third floating-point output (the singular values of the SVD), 0 / nullptr for the others
 template <typename Fn>
 static int run_chunked(Ctx* c, long long batch, size_t in_a, size_t in_b, size_t out_a, size_t out_b, size_t out_i,
-                       const void* hA, const void* hB, void* hOa, void* hOb, void* hInfo, Fn&& fn) {
+                       const void* hA, const void* hB, void* hOa, void* hOb, void* hInfo, size_t out_c, void* hOc, Fn&& fn) {
     if (batch == 0) return LQ_OK;
     LQ_CUDA(c, cudaSetDevice(c->device));
-    const long long chunk = pick_chunk(batch, in_a + in_b + out_a + out_b + out_i);
-    DevBuf dA[2], dB[2], dOa[2], dOb[2], dI[2];
+    const long long chunk = pick_chunk(batch, in_a + in_b + out_a + out_b + out_i + out_c);
+    DevBuf dA[2], dB[2], dOa[2], dOb[2], dI[2], dOc[2];
     for (int l = 0; l < 2; ++l) {
         LQ_TRY(dA[l].alloc(c, in_a * chunk, c->lane[l]));
         LQ_TRY(dB[l].alloc(c, in_b * chunk, c->lane[l]));
         LQ_TRY(dOa[l].alloc(c, out_a * chunk, c->lane[l]));
         LQ_TRY(dOb[l].alloc(c, out_b * chunk, c->lane[l]));
         LQ_TRY(dI[l].alloc(c, out_i * chunk, c->lane[l]));
+        if (out_c) LQ_TRY(dOc[l].alloc(c, out_c * chunk, c->lane[l]));
     }
     int k = 0;
     for (long long off = 0; off < batch; off += chunk, ++k) {
@@ -120,13 +141,15 @@ static int run_chunked(Ctx* c, long long batch, size_t in_a, size_t in_b, size_t
         LQ_CUDA(c, cudaMemcpyAsync(dA[l].p, (const char*)hA + off * in_a, in_a * cnt, cudaMemcpyHostToDevice, st));
         if (in_b)
             LQ_CUDA(c, cudaMemcpyAsync(dB[l].p, (const char*)hB + off * in_b, in_b * cnt, cudaMemcpyHostToDevice, st));
-        LQ_TRY(fn(st, cnt, dA[l].p, dB[l].p, dOa[l].p, dOb[l].p, dI[l].p));
+        LQ_TRY(fn(st, cnt, dA[l].p, dB[l].p, dOa[l].p, dOb[l].p, dI[l].p, dOc[l].p));
         if (out_a)
             LQ_CUDA(c, cudaMemcpyAsync((char*)hOa + off * out_a, dOa[l].p, out_a * cnt, cudaMemcpyDeviceToHost, st));
         if (out_b)
             LQ_CUDA(c, cudaMemcpyAsync((char*)hOb + off * out_b, dOb[l].p, out_b * cnt, cudaMemcpyDeviceToHost, st));
         if (out_i && hInfo)
             LQ_CUDA(c, cudaMemcpyAsync((char*)hInfo + off * out_i, dI[l].p, out_i * cnt, cudaMemcpyDeviceToHost, st));
+        if (out_c)
+            LQ_CUDA(c, cudaMemcpyAsync((char*)hOc + off * out_c, dOc[l].p, out_c * cnt, cudaMemcpyDeviceToHost, st));
     }
     for (int l = 0; l < 2; ++l) LQ_CUDA(c, cudaStreamSynchronize(c->lane[l]));
     return LQ_OK;
@@ -168,8 +191,8 @@ int lq_householder_qr_batched(lq_ctx* h, const double* A, int64_t batch, int m, 
             LQ_TRY(lq_householder_qr(h, A + b * (size_t)m * n, m, n, Q + b * (size_t)m * n, R + b * (size_t)n * n));
         return LQ_OK;
     }
-    return run_chunked(c, batch, mn, 0, mn, nn, 0, A, nullptr, Q, R, nullptr,
-                       [&](cudaStream_t st, long long cnt, void* dA, void*, void* dQ, void* dR, void*) {
+    return run_chunked(c, batch, mn, 0, mn, nn, 0, A, nullptr, Q, R, nullptr, 0, nullptr,
+                       [&](cudaStream_t st, long long cnt, void* dA, void*, void* dQ, void* dR, void*, void*) {
                            return hh_qr_batched_stream(c, st, (const double*)dA, cnt, m, n, (double*)dQ, (double*)dR, true);
                        });
 }
@@ -193,8 +216,8 @@ int lq_mgs_qr_batched(lq_ctx* h, const double* A, int64_t batch, int m, int n, i
                              info ? info + b : nullptr));
         return LQ_OK;
     }
-    return run_chunked(c, batch, mn, 0, mn, nn, sizeof(int32_t), A, nullptr, Q, R, info,
-                       [&](cudaStream_t st, long long cnt, void* dA, void*, void* dQ, void* dR, void* dI) {
+    return run_chunked(c, batch, mn, 0, mn, nn, sizeof(int32_t), A, nullptr, Q, R, info, 0, nullptr,
+                       [&](cudaStream_t st, long long cnt, void* dA, void*, void* dQ, void* dR, void* dI, void*) {
                            return mgs_qr_batched_stream(c, st, (const double*)dA, cnt, m, n, reorth, (double*)dQ,
                                                         (double*)dR, (int*)dI);
                        });
@@ -258,8 +281,8 @@ static int lstsq_hh_host(lq_ctx* h, const double* A, const double* B, int64_t ba
         }
         return LQ_OK;
     }
-    return run_chunked(c, batch, mn, mk, nk, 0, info ? sizeof(int32_t) : 0, A, B, X, nullptr, info,
-                       [&](cudaStream_t st, long long cnt, void* dA, void* dB, void* dX, void*, void* dI) {
+    return run_chunked(c, batch, mn, mk, nk, 0, info ? sizeof(int32_t) : 0, A, B, X, nullptr, info, 0, nullptr,
+                       [&](cudaStream_t st, long long cnt, void* dA, void* dB, void* dX, void*, void* dI, void*) {
                            return lstsq_hh_batched_stream(c, st, (const double*)dA, (const double*)dB, cnt, m, n, nrhs,
                                                           (double*)dX, info ? (int*)dI : nullptr);
                        });
@@ -297,10 +320,39 @@ int lq_lstsq_mgs_batched(lq_ctx* h, const double* A, const double* B, int64_t ba
         }
         return LQ_OK;
     }
-    return run_chunked(c, batch, mn, mk, nk, 0, sizeof(int32_t), A, B, X, nullptr, info,
-                       [&](cudaStream_t st, long long cnt, void* dA, void* dB, void* dX, void*, void* dI) {
+    return run_chunked(c, batch, mn, mk, nk, 0, sizeof(int32_t), A, B, X, nullptr, info, 0, nullptr,
+                       [&](cudaStream_t st, long long cnt, void* dA, void* dB, void* dX, void*, void* dI, void*) {
                            return lstsq_mgs_batched_stream(c, st, (const double*)dA, (const double*)dB, cnt, m, n, nrhs,
                                                            (double*)dX, (int*)dI);
+                       });
+}
+
+int lq_svd_gram_batched_dev(lq_ctx* h, const double* A, int64_t batch, int m, int n, double tol, double* U, double* s,
+                            double* Vt, int32_t* rank) {
+    Ctx* c = as_ctx(h);
+    LQ_ARGS_QR(c, A, batch, m, n);
+    LQ_REQUIRE(c, m >= n, LQ_ERR_SHAPE, "svd_gram needs m >= n (got %d x %d; transpose on the host side, svd.py:37-39)", m, n);
+    LQ_CUDA(c, cudaSetDevice(c->device));
+    return svd_batched_stream(c, c->stream, A, batch, m, n, tol, U, s, Vt, rank);
+}
+
+int lq_svd_gram_batched(lq_ctx* h, const double* A, int64_t batch, int m, int n, double tol, double* U, double* s, double* Vt,
+                        int32_t* rank) {
+    Ctx* c = as_ctx(h);
+    LQ_ARGS_QR(c, A, batch, m, n);
+    LQ_REQUIRE(c, m >= n, LQ_ERR_SHAPE, "svd_gram needs m >= n (got %d x %d; transpose on the host side, svd.py:37-39)", m, n);
+    if (!svd_small_supported(m, n)) {
+        // the single-matrix pipeline, one matrix at a time on the context stream
+        for (int64_t b = 0; b < batch; ++b)
+            LQ_TRY(lq_svd_gram(h, A + b * (size_t)m * n, m, n, tol, U + b * (size_t)m * n, s + b * (size_t)n, Vt + b * (size_t)n * n,
+                               rank + b));
+        return LQ_OK;
+    }
+    const size_t mn = (size_t)m * n * 8, nn = (size_t)n * n * 8;
+    return run_chunked(c, batch, mn, 0, mn, nn, sizeof(int32_t), A, nullptr, U, Vt, rank, (size_t)n * 8, s,
+                       [&](cudaStream_t st, long long cnt, void* dA, void*, void* dU, void* dVt, void* dR, void* dS) {
+                           return svd_batched_stream(c, st, (const double*)dA, cnt, m, n, tol, (double*)dU, (double*)dS,
+                                                     (double*)dVt, (int*)dR);
                        });
 }
 

@@ -231,4 +231,21 @@ __device__ __forceinline__ double ld_cluster_f64(uint32_t addr) {
     return v;
 }
 
+// ------------------------------------------------------------------ Jacobi round-robin ("circle") ordering
+// Pair k (0 <= k < n_even / 2) of round `round` (0 <= round < n_even - 1): every index meets every other once per sweep.
+__device__ __forceinline__ void rr_pair(int n_even, int round, int k, int& p, int& q) {
+    // players 0..n_even-2 on a circle, player n_even-1 fixed
+    const int mod = n_even - 1;
+    int a, b;
+    if (k == 0) {
+        a = n_even - 1;
+        b = round % mod;
+    } else {
+        a = (round + k) % mod;
+        b = (round - k + mod) % mod;
+    }
+    p = min(a, b);
+    q = max(a, b);
+}
+
 }  // namespace lq

@@ -61,8 +61,9 @@ int gram(Ctx* c, const double* A, long long m, int n, double* G);  // G = A^T A
 // psd: the caller guarantees a positive semi-definite G (a Gram matrix): a well-conditioned one then gets its eigenvectors as
 // the normalised converged columns b_i = lambda_i v_i instead of replaying the rotation log
 int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, bool psd = false);
+// rank_dev (device, may be null) receives the rank too, stream-ordered
 int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, double* U, double* s, double* Vt,
-                   int* rank_host, bool sharded);
+                   int* rank_host, bool sharded, int* rank_dev = nullptr);
 int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R, bool sharded);
 // min ||A X - B|| for a tall-skinny A (m x n) and B (m x nrhs): CholeskyQR2 pipeline, Householder fallbacks.  info (device):
 // 0, or 1 + the first column whose R[j][j] is exactly 0

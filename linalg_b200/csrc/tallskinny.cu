@@ -20,21 +20,8 @@ inline int grid_for(Ctx* c, long long total) {
 // Two-sided cyclic Jacobi with the round-robin ("circle") parallel ordering.  One CTA owns the
 // matrix (shared memory when it fits, global memory otherwise); every round applies n/2 disjoint
 // rotations, first to the columns then to the rows.  The (c, s) pairs are logged so that the
-// eigenvectors can be accumulated afterwards by independent CTAs (one row of V each).
-__device__ __forceinline__ void rr_pair(int n_even, int round, int k, int& p, int& q) {
-    // players 0..n_even-2 on a circle, player n_even-1 fixed
-    const int mod = n_even - 1;
-    int a, b;
-    if (k == 0) {
-        a = n_even - 1;
-        b = round % mod;
-    } else {
-        a = (round + k) % mod;
-        b = (round - k + mod) % mod;
-    }
-    p = min(a, b);
-    q = max(a, b);
-}
+// eigenvectors can be accumulated afterwards by independent CTAs (one row of V each).  Pairs of a round: rr_pair
+// (common.cuh).
 
 __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__ G, int n, double* __restrict__ Awork,
                                                      int use_global, double2* __restrict__ rotlog, int max_sweeps, double rel_tol,
@@ -824,7 +811,7 @@ int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, 
 }
 
 int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, double* U, double* s, double* Vt,
-                   int* rank_host, bool sharded) {
+                   int* rank_host, bool sharded, int* rank_dev) {
     LQ_REQUIRE(c, m >= 1 && n >= 1, LQ_ERR_SHAPE, "svd: bad shape %lld x %d", m, n);
     LQ_REQUIRE(c, m < (1LL << 31), LQ_ERR_SHAPE, "svd: more than 2^31 rows per device not supported");
     DevBuf G, lam, V, M2, rk;
@@ -839,6 +826,7 @@ int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, doub
     LQ_TRY(launch<svd_post_kernel>(c, small_grid(c, n), 256, sizeof(double) * n, c->stream, 0, lam.as<double>(), V.as<double>(), n,
                                    tol, s, M2.as<double>(), Vt, rk.as<int>()));
     LQ_TRY(gemm(c, false, false, m, n, n, 1.0, A, n, M2.as<double>(), n, 0.0, U, n));  // svd.py:61-64
+    if (rank_dev) LQ_CUDA(c, cudaMemcpyAsync(rank_dev, rk.p, sizeof(int), cudaMemcpyDeviceToDevice, c->stream));
     if (rank_host) {
         LQ_CUDA(c, cudaMemcpyAsync(rank_host, rk.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         LQ_CUDA(c, cudaStreamSynchronize(c->stream));

@@ -12,6 +12,8 @@ import ctypes as C
 import numpy as np
 
 from . import _native as nat
+from .qr import _check_out, _run_batched
+from .utils import as_f64_batch
 
 
 def svd(A, tol: float = 1e-12, *, ctx=None, seed=None):
@@ -47,4 +49,52 @@ def svd(A, tol: float = 1e-12, *, ctx=None, seed=None):
             ctx.call("lq_svd_complete", U.ctypes.data, m, n, r, Z.ctypes.data)
         else:
             ctx.call("lq_svd_complete_seeded", U.ctypes.data, m, n, r, int(seed) & 0xFFFFFFFFFFFFFFFF)
+    return U, s, Vt
+
+
+def svd_batched(A, tol: float = 1e-12, *, seed=None, out=None, ctx=None, devices=None):
+    """``svd`` applied independently to every ``A[i]`` of a (batch, m, n) array: returns U (batch, m, k), s (batch, k)
+    descending, Vt (batch, k, n) with k = min(m, n).  Matrix i of the result is ``svd(A[i], tol, seed=seed)``: the rank
+    #(s > tol) is decided per matrix, and each rank-deficient matrix gets U's orthonormal completion.  With ``seed=None``
+    the candidates are drawn from the global ``np.random`` for the rank-deficient matrices in increasing i, leaving it in
+    the state a loop over ``svd`` leaves.
+
+    n <= 32 and m <= 4096 (after transposing a wide batch) run one warp per matrix; other shapes run the single-matrix
+    pipeline matrix by matrix, bit for bit ``svd(A[i])``.  The route depends on the shape alone, so a matrix's result does
+    not depend on the batch it is in.  ``out=(U, s, Vt)`` receives the result; ``devices=[0, 1, ...]`` splits the batch
+    contiguously over several GPUs of this process (bitwise the one-GPU result)."""
+    A = as_f64_batch(A)
+    b, m, n = A.shape
+    k = min(m, n)
+    if out is not None:
+        U, s, Vt = out
+        _check_out(U, (b, m, k))
+        _check_out(s, (b, k))
+        _check_out(Vt, (b, k, n))
+    if m < n:
+        Vt_, s_, Ut = svd_batched(np.ascontiguousarray(A.transpose(0, 2, 1)), tol, seed=seed, ctx=ctx, devices=devices)
+        U_, Vt_ = Ut.transpose(0, 2, 1), Vt_.transpose(0, 2, 1)
+        if out is None:
+            return U_, s_, Vt_
+        U[...], s[...], Vt[...] = U_, s_, Vt_
+        return U, s, Vt
+    if out is None:
+        U, s, Vt = np.empty((b, m, n)), np.empty((b, n)), np.empty((b, n, n))
+    if b == 0 or n == 0:
+        return U, s, Vt
+    rank = np.zeros(b, dtype=np.int32)
+    _run_batched(ctx, devices, b, lambda c, lo, hi: c.call("lq_svd_gram_batched", A[lo:hi].ctypes.data, hi - lo, m, n, float(tol),
+                                                           U[lo:hi].ctypes.data, s[lo:hi].ctypes.data, Vt[lo:hi].ctypes.data,
+                                                           rank[lo:hi].ctypes.data))
+    deficient = np.flatnonzero(rank < n)
+    if deficient.size:
+        # linalg/svd.py:67-76 for each rank-deficient matrix, in increasing i (the global np.random draws of a loop over svd)
+        cctx = ctx if ctx is not None else (nat.default_context() if devices is None else nat.device_context(devices[0]))
+        for i in deficient:
+            r = int(rank[i])
+            if seed is None:
+                Z = np.ascontiguousarray(np.random.randn(m, n - r))
+                cctx.call("lq_svd_complete", U[i].ctypes.data, m, n, r, Z.ctypes.data)
+            else:
+                cctx.call("lq_svd_complete_seeded", U[i].ctypes.data, m, n, r, int(seed) & 0xFFFFFFFFFFFFFFFF)
     return U, s, Vt
