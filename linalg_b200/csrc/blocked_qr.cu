@@ -262,10 +262,6 @@ int panel_factor(Ctx* c, double* A, int lda, double* V, int ldv, double* T, int 
     return panel_factor_v(c, A, lda, V, ldv, T, ldt, mp, nb, 0);
 }
 
-inline int grid_for(Ctx* c, long long total) {
-    return (int)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)c->sm_count * 8));
-}
-
 // apply the block reflector  C <- (I - V op(T) V^T) C   to C (mk x nc, ldc); V (mk x kb, ldv); T (kb x kb, ldt)
 // trans_t = true -> T^T (factorisation order H_kb ... H_1), false -> T (Q formation order H_1 ... H_kb)
 int apply_block_reflector(Ctx* c, const double* V, int ldv, const double* T, int ldt, bool trans_t, int mk, int kb,
@@ -571,7 +567,7 @@ __global__ void __launch_bounds__(256) singular_diag_kernel(const double* __rest
 
 // R X = Y in place (Y: n x k, ldy; k even when the tensor-core GEMM is to be used for the off-diagonal part)
 int back_substitute(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n, int k) {
-    if (n <= 256) return launch<backsub_kernel>(c, std::max(1, (k + 255) / 256), 256, 0, c->stream, 0, R, ldr, Y, ldy, n, k);
+    if (n <= 256) return backsub_per_column(c, R, ldr, Y, ldy, n, k);
     const int nblk = (n + 127) / 128;
     for (int b = nblk - 1; b >= 0; --b) {
         const int r0 = b * 128, nb = std::min(128, n - r0), after = n - (r0 + nb);
@@ -585,6 +581,15 @@ int back_substitute(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n,
 }
 
 }  // namespace
+
+int backsub_per_column(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n, int k) {
+    return launch<backsub_kernel>(c, std::max(1, (k + 255) / 256), 256, 0, c->stream, 0, R, ldr, Y, ldy, n, k);
+}
+
+int pad_columns(Ctx* c, const double* src, int lds, double* dst, int ldd, long long rows, int cols_src, int cols_dst) {
+    return launch<pad_copy_kernel>(c, grid_for(c, rows * cols_dst), 256, 0, c->stream, 0, src, lds, dst, ldd, rows, cols_src,
+                                   cols_dst);
+}
 
 int measure_max_cluster(Ctx* c) {
     constexpr auto kern = panel_cluster_kernel<4, 16>;
@@ -624,8 +629,7 @@ int blocked_householder_qr(Ctx* c, const double* A, int m, int n, double* Q, dou
     DevBuf Aw, Vw, Qw;
     LQ_TRY(Aw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Vw.alloc(c, sizeof(double) * (size_t)m * npad));
-    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * npad), 256, 0, c->stream, 0, A, n, Aw.as<double>(), npad, m, n,
-                                   npad));
+    LQ_TRY(pad_columns(c, A, n, Aw.as<double>(), npad, m, n, npad));
     LQ_CUDA(c, cudaMemsetAsync(Vw.p, 0, sizeof(double) * (size_t)m * npad, c->stream));
     Factored keep;
     LQ_TRY(factor_padded(c, Aw.as<double>(), npad, m, npad, n, Vw.as<double>(), npad, nullptr, 0, 0, &keep));
@@ -697,10 +701,8 @@ int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int
     LQ_TRY(Aw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Vw.alloc(c, sizeof(double) * (size_t)m * npad));
     LQ_TRY(Bw.alloc(c, sizeof(double) * (size_t)m * kpad));
-    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * npad), 256, 0, c->stream, 0, A, n, Aw.as<double>(), npad, m, n,
-                                   npad));
-    LQ_TRY(launch<pad_copy_kernel>(c, grid_for(c, (long long)m * kpad), 256, 0, c->stream, 0, B, nrhs, Bw.as<double>(), kpad, m,
-                                   nrhs, kpad));
+    LQ_TRY(pad_columns(c, A, n, Aw.as<double>(), npad, m, n, npad));
+    LQ_TRY(pad_columns(c, B, nrhs, Bw.as<double>(), kpad, m, nrhs, kpad));
     LQ_CUDA(c, cudaMemsetAsync(Vw.p, 0, sizeof(double) * (size_t)m * npad, c->stream));
     LQ_TRY(factor_padded(c, Aw.as<double>(), npad, m, npad, n, Vw.as<double>(), npad, Bw.as<double>(), kpad, kpad, nullptr));
     if (info) LQ_TRY(launch<singular_diag_kernel>(c, 1, 256, 0, c->stream, 0, Aw.as<double>(), npad, n, info));

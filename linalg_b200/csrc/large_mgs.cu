@@ -76,15 +76,6 @@ __global__ void __launch_bounds__(256) mgs_update_kernel(double* __restrict__ At
         for (int i = threadIdx.x; i < m; i += blockDim.x) a[i] = a[i] / nrm;  // true division, qr.py:42 (own writes)
     }
 }
-__global__ void __launch_bounds__(256) backsub_cols_kernel(const double* __restrict__ R, int n, double* __restrict__ Y, int k) {
-    for (int col = blockIdx.x * blockDim.x + threadIdx.x; col < k; col += gridDim.x * blockDim.x) {
-        for (int i = n - 1; i >= 0; --i) {
-            double acc = Y[(size_t)i * k + col];
-            for (int cc = i + 1; cc < n; ++cc) acc = fma(-R[(size_t)i * n + cc], Y[(size_t)cc * k + col], acc);
-            Y[(size_t)i * k + col] = acc / R[(size_t)i * n + i];
-        }
-    }
-}
 
 }  // namespace
 
@@ -110,7 +101,8 @@ int large_lstsq_mgs(Ctx* c, const double* A, const double* B, int m, int n, int 
     LQ_TRY(Rb.alloc(c, sizeof(double) * (size_t)n * n));
     LQ_TRY(large_mgs_qr(c, A, m, n, 0, Qb.as<double>(), Rb.as<double>(), info));
     LQ_TRY(gemm(c, true, false, n, nrhs, m, 1.0, Qb.as<double>(), n, B, nrhs, 0.0, X, nrhs));  // y = Q^T b  (qr.py:113)
-    return launch<backsub_cols_kernel>(c, (nrhs + 255) / 256, 256, 0, c->stream, 0, Rb.as<double>(), n, X, nrhs);
+    // one thread per right-hand side at every n (the blocked solve of back_substitute would reorder the sums)
+    return backsub_per_column(c, Rb.as<double>(), n, X, nrhs, n, nrhs);
 }
 
 }  // namespace lq

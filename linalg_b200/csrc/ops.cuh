@@ -1,11 +1,17 @@
 // Internal (device-pointer) operations shared between the translation units.
 #pragma once
 
+#include <algorithm>
 #include <atomic>
 
 #include "ctx.cuh"
 
 namespace lq {
+
+// CTAs of a grid-stride element-wise kernel over `total` elements: one element per thread, at most 8 CTAs of 256 per SM
+inline int grid_for(Ctx* c, long long total) {
+    return (int)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)c->sm_count * 8));
+}
 
 // ---- gemm.cu: row-major C = alpha * op(A) * op(B) + beta * C on the context stream.
 // FP64 tensor-core (DMMA) kernel fed by bulk-async (TMA engine) copies when shapes are aligned,
@@ -29,6 +35,10 @@ int blocked_householder_factor(Ctx* c, double* A, int lda, int m, int n, double*
                                int nrhs);
 // info (device, may be null): 0, or 1 + the first column whose R[j][j] is exactly 0 (the solve is singular)
 int large_lstsq_householder(Ctx* c, const double* A, const double* B, int m, int n, int nrhs, double* X, int* info);
+// dst (rows x cols_dst, ldd) = [src | 0] (src rows x cols_src, lds)
+int pad_columns(Ctx* c, const double* src, int lds, double* dst, int ldd, long long rows, int cols_src, int cols_dst);
+// R X = Y in place, one thread per right-hand side (R n x n upper triangular, ldr; Y n x k, ldy)
+int backsub_per_column(Ctx* c, const double* R, int ldr, double* Y, int ldy, int n, int k);
 // Largest cluster of the barrier.cluster panel kernel the device holds (16, 8, 4, 2 or 1) -> c->max_cluster.  One
 // occupancy query when the context is created; launches nothing.
 int measure_max_cluster(Ctx* c);
@@ -56,14 +66,22 @@ int syrk_tn(Ctx* c, const double* A, int lda, long long m, int n, double* G, int
 bool syrk_strip_supported(const double* Q, long long m, int n, const double* B, int nrhs);
 int syrk_strip_tn(Ctx* c, const double* Q, long long m, int n, const double* B, int nrhs, double* G, double* C);
 
-// ---- tallskinny.cu
-int gram(Ctx* c, const double* A, long long m, int n, double* G);  // G = A^T A
+// G = A^T A (A m x n, row stride lda): the symmetric rank-k kernel when the shape allows, the general TN GEMM otherwise
+inline int gram(Ctx* c, const double* A, int lda, long long m, int n, double* G) {
+    const int rc = syrk_tn(c, A, lda, m, n, G, n);
+    if (rc != LQ_ERR_UNSUPPORTED) return rc;
+    return gemm(c, true, false, n, n, (int)m, 1.0, A, lda, A, lda, 0.0, G, n);
+}
+
+// ---- eigh_svd.cu: the Jacobi eigen-solver and the economy SVD through the Gram matrix
 // psd: the caller guarantees a positive semi-definite G (a Gram matrix): a well-conditioned one then gets its eigenvectors as
 // the normalised converged columns b_i = lambda_i v_i instead of replaying the rotation log
 int eigh_jacobi(Ctx* c, const double* G, int n, double* lambda_desc, double* V, bool psd = false);
 // rank_dev (device, may be null) receives the rank too, stream-ordered
 int svd_gram_local(Ctx* c, const double* A, long long m, int n, double tol, double* U, double* s, double* Vt,
                    int* rank_host, bool sharded, int* rank_dev = nullptr);
+
+// ---- tsqr.cu: thin QR and least squares of tall-skinny matrices, on one GPU or row-sharded
 int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R, bool sharded);
 // min ||A X - B|| for a tall-skinny A (m x n) and B (m x nrhs): CholeskyQR2 pipeline, Householder fallbacks.  info (device):
 // 0, or 1 + the first column whose R[j][j] is exactly 0

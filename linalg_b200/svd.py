@@ -16,6 +16,17 @@ from .qr import _check_out, _run_batched
 from .utils import as_f64_batch
 
 
+def _complete(ctx, U, m, n, r, seed):
+    """linalg/svd.py:67-76: complete U (m, n; its first r columns valid) with an orthonormal basis of the complement, in
+    place.  ``seed=None`` draws the m x (n - r) candidate directions on the host exactly like upstream (global np.random);
+    an integer generates them on the device.  The projection and both orthonormalisations run on the device."""
+    if seed is None:
+        Z = np.ascontiguousarray(np.random.randn(m, n - r))
+        ctx.call("lq_svd_complete", U.ctypes.data, m, n, r, Z.ctypes.data)
+    else:
+        ctx.call("lq_svd_complete_seeded", U.ctypes.data, m, n, r, int(seed) & 0xFFFFFFFFFFFFFFFF)
+
+
 def svd(A, tol: float = 1e-12, *, ctx=None, seed=None):
     """Returns ``(U, s, Vt)``: U (m, n) orthonormal columns, s (n,) descending, Vt (n, n), for m >= n;
     a wide matrix is handled by transposing and swapping roles (linalg/svd.py:37-39).
@@ -41,14 +52,7 @@ def svd(A, tol: float = 1e-12, *, ctx=None, seed=None):
     ctx.call("lq_svd_gram", A.ctypes.data, m, n, float(tol), U.ctypes.data, s.ctypes.data, Vt.ctypes.data, C.byref(rank))
     r = int(rank.value)
     if r < n:
-        # linalg/svd.py:67-76 -- complete U with an orthonormal basis of the complement.  The
-        # candidate directions are drawn on the host exactly like upstream (global np.random);
-        # the projection and both orthonormalisations run on the device (lq_svd_complete).
-        if seed is None:
-            Z = np.ascontiguousarray(np.random.randn(m, n - r))
-            ctx.call("lq_svd_complete", U.ctypes.data, m, n, r, Z.ctypes.data)
-        else:
-            ctx.call("lq_svd_complete_seeded", U.ctypes.data, m, n, r, int(seed) & 0xFFFFFFFFFFFFFFFF)
+        _complete(ctx, U, m, n, r, seed)
     return U, s, Vt
 
 
@@ -91,10 +95,5 @@ def svd_batched(A, tol: float = 1e-12, *, seed=None, out=None, ctx=None, devices
         # linalg/svd.py:67-76 for each rank-deficient matrix, in increasing i (the global np.random draws of a loop over svd)
         cctx = ctx if ctx is not None else (nat.default_context() if devices is None else nat.device_context(devices[0]))
         for i in deficient:
-            r = int(rank[i])
-            if seed is None:
-                Z = np.ascontiguousarray(np.random.randn(m, n - r))
-                cctx.call("lq_svd_complete", U[i].ctypes.data, m, n, r, Z.ctypes.data)
-            else:
-                cctx.call("lq_svd_complete_seeded", U[i].ctypes.data, m, n, r, int(seed) & 0xFFFFFFFFFFFFFFFF)
+            _complete(cctx, U[i], m, n, int(rank[i]), seed)
     return U, s, Vt

@@ -1,7 +1,7 @@
 """least_squares_tsqr / lq_lstsq_tsqr*: tall-skinny least squares on the CholeskyQR2 pipeline, its Householder fallbacks,
 and the row-sharded form over NCCL with two ranks.
 
-Routes of one GPU (tallskinny.cu, lstsq_tsqr_local):
+Routes of one GPU (tsqr.cu, lstsq_tsqr_local):
 - "fused":  n <= 128, m >= 4n, even n, nrhs <= 32, m >= 1024: pass 2 forms [G2 | C] = Q1^T [Q1 | B] in the strip SYRK kernel
   (an odd nrhs is padded to even);
 - "gemm":   the other CholeskyQR2 shapes: SYRK or GEMM Gram matrix and a TN GEMM for Q1^T B;

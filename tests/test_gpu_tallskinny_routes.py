@@ -1,12 +1,12 @@
 """Every kernel route of the Gram, eigen-solver, SVD and tall-skinny QR entry points, at the shapes where the route changes.
 
 As on the QR and least-squares paths (``test_gpu_routes.py``), kernel choice here depends on the shape alone.  The
-functions below mirror the predicates of ``syrk_tn_supported`` / ``gram_ld`` (``syrk.cu``, ``tallskinny.cu``),
+functions below mirror the predicates of ``syrk_tn_supported`` / ``gram`` (``syrk.cu``, ``ops.cuh``),
 ``eigh_jacobi``, ``tsqr_local`` / ``tsqr_wide``, the completion QR of ``svd_complete_impl`` and the row chunking of
 ``gemm`` (``gemm.cu``), and derive every boundary from the device's ``max_smem`` and ``sm_count``.  Each case proves which
 route ran with an observable that differs between the routes, without any extra ABI:
 
-- Gram: the GEMM route is bitwise the TN GEMM that ``gram_ld`` calls; the SYRK route makes exactly two launches and, on
+- Gram: the GEMM route is bitwise the TN GEMM that ``gram`` calls; the SYRK route makes exactly two launches and, on
   Gaussian input, differs from that GEMM.
 - Eigen-solver: the one-sided route makes 4 launches, the two-sided route 3.  For n > 128 the ``JACOBI_TWO_SIDED`` option
   changes nothing (bitwise); for n <= 128 it selects the other kernel, which gives other bits on a generic matrix.
@@ -67,7 +67,7 @@ GEMM_ROW_CHUNK = 1 << 21                       # gemm: taller products run in ro
 
 
 def gram_route(m, n, aligned=True):
-    """gram_ld with lda = n: the symmetric rank-k kernel when syrk_tn_supported holds, else the TN GEMM."""
+    """gram with lda = n: the symmetric rank-k kernel when syrk_tn_supported holds, else the TN GEMM."""
     ok = 2 <= n <= 128 and n % 2 == 0 and aligned and m >= SYRK_MIN_ROWS
     return "syrk" if ok else "gemm"
 
@@ -218,7 +218,7 @@ def test_gram_routes(ctx, shape):
         dA, dG, dH = ctx.upload(buf), ctx.alloc(8 * n * n), ctx.alloc(8 * n * n)
         p = dA.ptr + 8 * off
         _, nl = counted(ctx, ctx.call, "lq_gram_dev", p, m, n, dG.ptr)
-        ctx.call("lq_gemm_dev", 1, 0, n, n, m, 1.0, p, n, p, n, 0.0, dH.ptr, n)   # the call gram_ld makes
+        ctx.call("lq_gemm_dev", 1, 0, n, n, m, 1.0, p, n, p, n, 0.0, dH.ptr, n)   # the call gram makes
         return ctx.download(dG, (n, n)), ctx.download(dH, (n, n)), nl
 
     Ai = rng.integers(-1024, 1025, size=(m, n)).astype(np.float64)
