@@ -95,7 +95,7 @@ int lq_lstsq_householder_batched(lq_ctx* ctx, const double* A, const double* B, 
                                  int nrhs, double* X);
 /* the same with a per-system singularity report: info[b] = 0, or 1 + the first column whose R[j][j] is exactly 0 -- the
  * case in which the reference's np.linalg.solve raises LinAlgError("Singular matrix") (linalg/qr.py:134); the shim raises the
- * same.  Filled by the warp-per-system kernel (n <= 64, nrhs <= 16), 0 for other shapes. */
+ * same.  Every route (warp-per-system, streaming, one-CTA and blocked) fills it; info may be NULL. */
 int lq_lstsq_householder_batched_info_dev(lq_ctx* ctx, const double* A, const double* B, int64_t batch, int m, int n,
                                           int nrhs, double* X, int32_t* info);
 int lq_lstsq_householder_batched_info(lq_ctx* ctx, const double* A, const double* B, int64_t batch, int m, int n,

@@ -814,23 +814,4 @@ int lq_householder_qr_dev(lq_ctx* h, const double* A, int m, int n, double* Q, d
     return blocked_householder_qr(c, A, m, n, Q, R);
 }
 
-int lq_householder_qr(lq_ctx* h, const double* A, int m, int n, double* Q, double* R) {
-    Ctx* c = as_ctx(h);
-    if (!c) return LQ_ERR_ARG;
-    LQ_REQUIRE(c, m >= 1 && n >= 1 && m >= n, LQ_ERR_SHAPE, "householder_qr needs m >= n >= 1 (got %d x %d)", m, n);
-    LQ_REQUIRE(c, A && Q && R, LQ_ERR_ARG, "null pointer");
-    LQ_CUDA(c, cudaSetDevice(c->device));
-    const size_t mn = sizeof(double) * (size_t)m * n, nn = sizeof(double) * (size_t)n * n;
-    DevBuf dA, dQ, dR;
-    LQ_TRY(dA.alloc(c, mn));
-    LQ_TRY(dQ.alloc(c, mn));
-    LQ_TRY(dR.alloc(c, nn));
-    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
-    LQ_TRY(lq_householder_qr_dev(h, dA.as<double>(), m, n, dQ.as<double>(), dR.as<double>()));
-    LQ_CUDA(c, cudaMemcpyAsync(Q, dQ.p, mn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(R, dR.p, nn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-    return LQ_OK;
-}
-
 }  // extern "C"

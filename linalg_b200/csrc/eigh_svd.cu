@@ -686,26 +686,6 @@ int lq_svd_gram_sharded_dev(lq_ctx* h, const double* A, int64_t m, int n, double
     LQ_CUDA(c, cudaSetDevice(c->device));
     return svd_gram_local(c, A, m, n, tol, U, s, Vt, rank_host, true);
 }
-int lq_svd_gram(lq_ctx* h, const double* A, int64_t m, int n, double tol, double* U, double* s, double* Vt,
-                int* rank_host) {
-    Ctx* c = as_ctx(h);
-    if (!c) return LQ_ERR_ARG;
-    LQ_REQUIRE(c, m >= n && n >= 1, LQ_ERR_SHAPE, "svd_gram needs m >= n >= 1");
-    LQ_CUDA(c, cudaSetDevice(c->device));
-    const size_t mn = sizeof(double) * (size_t)m * n, nn = sizeof(double) * (size_t)n * n;
-    DevBuf dA, dU, ds, dVt;
-    LQ_TRY(dA.alloc(c, mn));
-    LQ_TRY(dU.alloc(c, mn));
-    LQ_TRY(ds.alloc(c, sizeof(double) * n));
-    LQ_TRY(dVt.alloc(c, nn));
-    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
-    LQ_TRY(svd_gram_local(c, dA.as<double>(), m, n, tol, dU.as<double>(), ds.as<double>(), dVt.as<double>(), rank_host, false));
-    LQ_CUDA(c, cudaMemcpyAsync(U, dU.p, mn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(s, ds.p, sizeof(double) * n, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(Vt, dVt.p, nn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-    return LQ_OK;
-}
 // linalg/svd.py:67-76 on the device: orthonormal completion of U (host, m x n, first `rank` columns
 // valid) from the candidate directions Z: drawn by the caller (host, m x (n - rank): upstream draws them from the global
 // np.random) or, with a seed, generated on the device (no upload; deterministic -- SURVEY.md section 8f-1).

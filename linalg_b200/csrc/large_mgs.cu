@@ -113,24 +113,5 @@ extern "C" {
 int lq_mgs_qr_dev(lq_ctx* h, const double* A, int m, int n, int reorth, double* Q, double* R, int32_t* info) {
     return lq_mgs_qr_batched_dev(h, A, 1, m, n, reorth, Q, R, info);
 }
-int lq_mgs_qr(lq_ctx* h, const double* A, int m, int n, int reorth, double* Q, double* R, int32_t* info) {
-    Ctx* c = as_ctx(h);
-    if (!c) return LQ_ERR_ARG;
-    LQ_REQUIRE(c, m >= 1 && n >= 1 && A && Q && R, LQ_ERR_SHAPE, "mgs_qr: bad arguments");
-    LQ_CUDA(c, cudaSetDevice(c->device));
-    const size_t mn = sizeof(double) * (size_t)m * n, nn = sizeof(double) * (size_t)n * n;
-    DevBuf dA, dQ, dR, dI;
-    LQ_TRY(dA.alloc(c, mn));
-    LQ_TRY(dQ.alloc(c, mn));
-    LQ_TRY(dR.alloc(c, nn));
-    LQ_TRY(dI.alloc(c, 16));
-    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
-    LQ_TRY(lq_mgs_qr_batched_dev(h, dA.as<double>(), 1, m, n, reorth, dQ.as<double>(), dR.as<double>(), dI.as<int32_t>()));
-    LQ_CUDA(c, cudaMemcpyAsync(Q, dQ.p, mn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(R, dR.p, nn, cudaMemcpyDeviceToHost, c->stream));
-    if (info) LQ_CUDA(c, cudaMemcpyAsync(info, dI.p, 4, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-    return LQ_OK;
-}
 
 }  // extern "C"

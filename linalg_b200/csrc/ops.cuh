@@ -87,13 +87,35 @@ int tsqr_local(Ctx* c, const double* A, long long m, int n, double* Q, double* R
 // 0, or 1 + the first column whose R[j][j] is exactly 0
 int lstsq_tsqr_local(Ctx* c, const double* A, long long m, int n, const double* B, int nrhs, double* X, int* info, bool sharded);
 
-// ---- batched (api_batched.cu).  qr32: 32 x 32 matrices go to the batched 32 x 32 kernel; false keeps them on the
-// one-CTA kernel (the single-matrix entry point)
+// ---- batched dispatchers (api_batched.cu).  Each *_one_launch predicate says whether a shape takes one kernel launch
+// for the whole batch, on any stream `st`.  Otherwise the dispatcher runs the single-matrix path matrix by matrix, and
+// `st` must be the context stream.
+// qr32: 32 x 32 matrices go to the batched 32 x 32 kernel; false keeps them on the one-CTA kernel (the single-matrix
+// entry point)
+bool hh_qr_batched_one_launch(Ctx* c, int m, int n);
 int hh_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double* Q,
                          double* R, bool qr32);
+// info (device, may be null): per matrix 0, or 1 + the first column with R[j][j] < 1e-12 (linalg/qr.py:40-41)
+bool mgs_qr_batched_one_launch(Ctx* c, int m, int n);
+int mgs_qr_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, int reorth,
+                          double* Q, double* R, int* info);
 // info (device, may be null): per system 0, or 1 + the first column whose R[j][j] is exactly 0
+bool lstsq_hh_batched_one_launch(Ctx* c, int m, int n, int nrhs);
 int lstsq_hh_batched_stream(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
                             int nrhs, double* X, int* info = nullptr);
+bool lstsq_mgs_batched_one_launch(Ctx* c, int m, int n, int nrhs);
+int lstsq_mgs_batched_stream(Ctx* c, cudaStream_t st, const double* A, const double* B, long long batch, int m, int n,
+                             int nrhs, double* X, int* info);
+// one launch when svd_small_supported(m, n) (batched_svd_small.cuh)
+int svd_batched_stream(Ctx* c, cudaStream_t st, const double* A, long long batch, int m, int n, double tol, double* U,
+                       double* s, double* Vt, int* rank);
+
+// argument checks shared by the batched entry points (device and host pointers)
+#define LQ_ARGS_QR(c, A, batch, m, n)                                                                       \
+    LQ_REQUIRE(c, c != nullptr, LQ_ERR_ARG, "null context");                                               \
+    LQ_REQUIRE(c, batch >= 0 && m >= 1 && n >= 1, LQ_ERR_SHAPE, "bad shape batch=%lld m=%d n=%d",        \
+               (long long)batch, m, n);                                                                    \
+    LQ_REQUIRE(c, batch == 0 || A != nullptr, LQ_ERR_ARG, "null input pointer")
 
 // ---- kernel launches.  Every kernel of the linear-algebra entry points goes through launch<Kern> (launch_cluster<Kern>
 // for one cluster of CTAs), which in this order

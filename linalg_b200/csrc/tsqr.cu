@@ -592,23 +592,6 @@ int lq_tsqr_sharded_dev(lq_ctx* h, const double* A, int64_t m, int n, double* Q,
     LQ_CUDA(c, cudaSetDevice(c->device));
     return tsqr_local(c, A, m, n, Q, R, true);
 }
-int lq_tsqr(lq_ctx* h, const double* A, int64_t m, int n, double* Q, double* R) {
-    Ctx* c = as_ctx(h);
-    if (!c) return LQ_ERR_ARG;
-    LQ_REQUIRE(c, m >= n && n >= 1, LQ_ERR_SHAPE, "tsqr needs m >= n >= 1");
-    LQ_CUDA(c, cudaSetDevice(c->device));
-    const size_t mn = sizeof(double) * (size_t)m * n, nn = sizeof(double) * (size_t)n * n;
-    DevBuf dA, dQ, dR;
-    LQ_TRY(dA.alloc(c, mn));
-    LQ_TRY(dQ.alloc(c, mn));
-    LQ_TRY(dR.alloc(c, nn));
-    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
-    LQ_TRY(tsqr_local(c, dA.as<double>(), m, n, dQ.as<double>(), dR.as<double>(), false));
-    LQ_CUDA(c, cudaMemcpyAsync(Q, dQ.p, mn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(R, dR.p, nn, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-    return LQ_OK;
-}
 
 int lq_lstsq_tsqr_dev(lq_ctx* h, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info) {
     Ctx* c = as_ctx(h);
@@ -621,27 +604,6 @@ int lq_lstsq_tsqr_sharded_dev(lq_ctx* h, const double* A, int64_t m, int n, cons
     if (!c) return LQ_ERR_ARG;
     LQ_CUDA(c, cudaSetDevice(c->device));
     return lstsq_tsqr_local(c, A, m, n, B, nrhs, X, info, true);
-}
-int lq_lstsq_tsqr(lq_ctx* h, const double* A, int64_t m, int n, const double* B, int nrhs, double* X, int32_t* info) {
-    Ctx* c = as_ctx(h);
-    if (!c) return LQ_ERR_ARG;
-    LQ_REQUIRE(c, m >= n && n >= 1 && nrhs >= 1 && m < (1LL << 31), LQ_ERR_SHAPE,
-               "lstsq_tsqr needs 2^31 > m >= n >= 1 and nrhs >= 1 (got %lld x %d, %d rhs)", (long long)m, n, nrhs);
-    LQ_REQUIRE(c, A && B && X && info, LQ_ERR_ARG, "lstsq_tsqr: null pointer");
-    LQ_CUDA(c, cudaSetDevice(c->device));
-    const size_t mn = sizeof(double) * (size_t)m * n, mk = sizeof(double) * (size_t)m * nrhs, nk = sizeof(double) * (size_t)n * nrhs;
-    DevBuf dA, dB, dX, dI;
-    LQ_TRY(dA.alloc(c, mn));
-    LQ_TRY(dB.alloc(c, mk));
-    LQ_TRY(dX.alloc(c, nk));
-    LQ_TRY(dI.alloc(c, 16));
-    LQ_CUDA(c, cudaMemcpyAsync(dA.p, A, mn, cudaMemcpyHostToDevice, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(dB.p, B, mk, cudaMemcpyHostToDevice, c->stream));
-    LQ_TRY(lstsq_tsqr_local(c, dA.as<double>(), m, n, dB.as<double>(), nrhs, dX.as<double>(), dI.as<int>(), false));
-    LQ_CUDA(c, cudaMemcpyAsync(X, dX.p, nk, cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaMemcpyAsync(info, dI.p, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    LQ_CUDA(c, cudaStreamSynchronize(c->stream));
-    return LQ_OK;
 }
 
 }  // extern "C"

@@ -2,8 +2,8 @@
 
 Kernel selection depends on the shape alone: each entry point is a fixed table of routes picked by thresholds on
 (m, n, nrhs) and on the device's opt-in shared memory per block.  The functions below mirror those predicates
-(``batched_small.cuh``, ``lstsq_stream.cu``, ``lq_householder_qr_dev`` in ``blocked_qr.cu``, ``pick_chunk`` in
-``api_batched.cu``) and derive the boundary shapes from them, so a case sits on the last shape of a route or on the
+(``batched_small.cuh``, ``lstsq_stream.cu``, ``lq_householder_qr_dev`` in ``blocked_qr.cu``, ``stage_host`` in
+``api_host.cu``) and derive the boundary shapes from them, so a case sits on the last shape of a route or on the
 first shape of the next one.  Every call also counts kernel launches: a one-kernel route launches exactly once per call
 (once per chunk on the host pipelines), a blocked or large route more than once per matrix.  A mirror that drifts from
 the library fails there, instead of quietly turning a boundary case into a duplicate of its neighbour.

@@ -1,7 +1,8 @@
 """svd_batched: the A^T A economy SVD of every matrix of a batch.
 
-Matrix i of the result is ``svd(A[i], tol)``.  The route depends on the shape alone (``svd_batched_stream``,
-``api_batched.cu``): n <= 32 and m <= 4096 after transposition run the warp-per-matrix kernel (one launch per call), every
+Matrix i of the result is ``svd(A[i], tol)``.  The route depends on the shape alone (``svd_small_supported``, which
+``svd_batched_stream`` in ``api_batched.cu`` and the host-pointer entry point in ``api_host.cu`` both call): n <= 32 and
+m <= 4096 after transposition run the warp-per-matrix kernel (one launch per call or per host-pipeline chunk), every
 other shape runs the single-matrix pipeline matrix by matrix and is bitwise ``svd(A[i])``.  Each matrix is held to the
 bounds of ``svd`` against LAPACK (``svd_errors`` of ``test_gpu_tallskinny_routes``).
 """
