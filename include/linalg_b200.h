@@ -109,7 +109,10 @@ int lq_lstsq_mgs_batched(lq_ctx* ctx, const double* A, const double* B, int64_t 
 
 /* ---- a5: svd via the A^T A eigen-route  (linalg/svd.py:10-82), m >= n ------------------------- */
 /* U (m, n), s (n) descending, Vt (n, n); *rank = #(s > tol).  Columns of U beyond rank are
- * left ZERO here; the shim completes them (svd.py:67-76) with lq_svd_complete. */
+ * left ZERO here; the shim completes them (svd.py:67-76) with lq_svd_complete.
+ * Non-finite input: a NaN or Inf in A, or a finite A whose A^T A overflows, gives s = NaN throughout, Vt = I and rank 0
+ * (lq_eigh_dev's contract; sigma of a NaN eigenvalue is NaN, never 0), with no error: the reference raises for some such
+ * shapes and returns NaN singular values for the others, never an all-finite s.  This holds for lq_svd_gram_batched too. */
 int lq_svd_gram_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double tol, double* U, double* s, double* Vt,
                     int* rank_host);
 int lq_svd_gram(lq_ctx* ctx, const double* A, int64_t m, int n, double tol, double* U, double* s, double* Vt,
@@ -139,10 +142,14 @@ int lq_gram_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double* G);     
  * which cannot happen for PSD input); 128 < n <= 2048: two-sided Jacobi (any symmetric matrix).  Input range: any finite
  * G whose largest |diagonal| entry is normal (2^-1022 to 2^1024); both kernels work on G scaled by a power of two to a
  * largest diagonal entry in [1, 2), so the result scales with G, bit for bit, as long as no entry of the scaled G is
- * subnormal. */
+ * subnormal.  A G with a NaN or infinite entry returns NaN for every eigenvalue and V = I, and is not an error (the
+ * reference's eigh raises for some such n and returns n - 1 or n NaN values for the others); lambda_desc is sorted with NaN
+ * first, as np.argsort(lam)[::-1] puts it, and every element of lambda_desc and V is written for any input
+ * (tests/test_gpu_nonfinite.py). */
 int lq_eigh_dev(lq_ctx* ctx, const double* G, int n, double* lambda_desc, double* V);
+/* row-major C = a op(A) op(B) + b C.  With b = 0, C is not read: it may hold anything, NaN and Inf included. */
 int lq_gemm_dev(lq_ctx* ctx, int transa, int transb, int64_t m, int n, int k, double alpha, const double* A,
-                int lda, const double* B, int ldb, double beta, double* C, int ldc); /* row-major C = a op(A) op(B) + b C */
+                int lda, const double* B, int ldb, double beta, double* C, int ldc);
 
 /* ---- a7: TSQR for tall-skinny matrices, diag(R) > 0 (the MGS convention) ------------------------ */
 int lq_tsqr_dev(lq_ctx* ctx, const double* A, int64_t m, int n, double* Q, double* R);

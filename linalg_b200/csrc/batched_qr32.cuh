@@ -119,7 +119,9 @@ __global__ void __launch_bounds__(WARPS * 32, MINB)
             for (int s = so; s < C; ++s) d[s] = group_sum<P, C>(d[s] + d2[s]);
             const double ss = __shfl_sync(0xffffffffu, d[so], lo, L);  // ||v_j||^2
             double rinv;
-            const double nrm = sqrt_nr_t<2>(fmax(ss, 1e-300), rinv);  // MUFU seed + 2 Newton steps: 2.7e-16 (lq_probe 13..16)
+            // MUFU seed + 2 Newton steps: 2.7e-16 (lq_probe 13..16).  The floor keeps a NaN norm NaN (fmax would turn it
+            // into 1e-150 and report the column as dependent, where the reference's R[j, j] < 1e-12 is false and it goes on)
+            const double nrm = sqrt_nr_t<2>(ss < 1e-300 ? 1e-300 : ss, rinv);
             if (nrm < kEps && bad == 0) bad = j + 1;
             const double rinv2 = rinv * rinv;
             // R row j: r_jc = d_c / ||v_j|| (c > j), ||v_j|| on the diagonal, 0 left of it

@@ -11,7 +11,7 @@
 //          warp-private shared memory with an odd pitch: in the column phase lane i updates row i of G and V, in the
 //          row phase lane j updates column j of G (conflict-free both ways).  A round whose pair does not rotate is
 //          skipped by the whole warp.  A zero row and column never rotates, so its eigenvalue stays exactly 0.
-//   post   descending order by counting (NaN sorts last, ties by index, always a permutation), s = sqrt(max(lambda, 0)),
+//   post   descending order by counting (NaN sorts first, ties by index, always a permutation), s = sqrt(max(lambda, 0)) with NaN kept,
 //          rank = #(s > tol), Vt = V^T, U[:, j] = A (v_j / s_j) for s_j > tol and 0 otherwise: a second pass over A,
 //          which is still in L2 (the matrices of all resident warps take ~15 MB).  U and Vt are written with streaming
 //          stores so that they do not evict the A tiles of other warps.
@@ -87,8 +87,15 @@ __global__ void __launch_bounds__(WARPS * 32) svd_small_kernel(const double* __r
             }
             __syncwarp();
         }
+        bool bad = false;
 #pragma unroll
-        for (int i = 0; i < K::NMAX; ++i) G[i * K::LD + ln] = g[i];  // rows / columns >= n are exactly 0
+        for (int i = 0; i < K::NMAX; ++i) {
+            G[i * K::LD + ln] = g[i];  // rows / columns >= n are exactly 0 (for finite A)
+            bad |= i < n && !isfinite(g[i]);
+        }
+        // a NaN or infinite entry of G: no sweep and every eigenvalue NaN, as jacobi_kernel / jacobi1s_kernel do (so this
+        // route agrees with the single-matrix route on non-finite input)
+        const bool nonfinite = __any_sync(FULL, ln < n && bad);
         __syncwarp();
         // work on 2^-e G with max|diag| in [1, 2), exactly as jacobi_kernel does; lambda is scaled back by 2^e below
         double d = ln < n ? fabs(G[ln * K::LD + ln]) : 0.0;
@@ -106,7 +113,7 @@ __global__ void __launch_bounds__(WARPS * 32) svd_small_kernel(const double* __r
         const double floor_abs = 4.9303806576313238e-32 * scalbn(d, -e);  // eps^2 * max|diag|
         const double rel_tol = 4.0 * 1.1102230246251565e-16;
         const int ne = (n + 1) & ~1, half = ne / 2;
-        for (int sweep = 0; sweep < K::MAX_SWEEPS; ++sweep) {
+        for (int sweep = 0; sweep < (nonfinite ? 0 : K::MAX_SWEEPS); ++sweep) {
             bool rotated = false;
             for (int rd = 0; rd < ne - 1; ++rd) {
                 if (ln < half) {
@@ -156,14 +163,12 @@ __global__ void __launch_bounds__(WARPS * 32) svd_small_kernel(const double* __r
         }
 
         // ---- descending order, s, rank, Vt
-        const double lam = ln < n ? scalbn(G[ln * K::LD + ln], e) : 0.0;
-        const double key = isnan(lam) ? -INFINITY : lam;
+        // NaN first, as in eig_sort_kernel and the reference's argsort()[::-1], so both svd_batched routes agree; sigma of a
+        // NaN eigenvalue is NaN, not 0
+        const double lam = ln >= n ? 0.0 : (nonfinite ? eig_nan() : scalbn(G[ln * K::LD + ln], e));
         int rk = 0;
-        for (int j = 0; j < n; ++j) {
-            const double kj = __shfl_sync(FULL, key, j);
-            rk += (kj > key) || (kj == key && j < ln);
-        }
-        const double sv = sqrt(fmax(lam, 0.0));
+        for (int j = 0; j < n; ++j) rk += eig_desc_before(__shfl_sync(FULL, lam, j), j, lam, ln);
+        const double sv = sqrt_clip0(lam);
         if (ln < n) {
             src[rk] = ln;
             S[b * n + rk] = sv;

@@ -248,4 +248,21 @@ __device__ __forceinline__ void rr_pair(int n_even, int round, int k, int& p, in
     q = max(a, b);
 }
 
+// ------------------------------------------------------------------ descending eigenvalue order
+// Whether eigenvalue a (index ia) comes before b (index ib): NaN first (where the reference's np.argsort(lam)[::-1] puts it),
+// then descending, equal values by index.  A strict total order even with NaN, so ranking by counting is a permutation; a
+// bare (b > a) || (b == a && ib < ia) is false both ways for NaN and gives several eigenvalues the same rank.
+__device__ __forceinline__ bool eig_desc_before(double a, int ia, double b, int ib) {
+    const bool na = isnan(a), nb = isnan(b);
+    if (na != nb) return na;
+    return (!na && a > b) || ((na || a == b) && ia < ib);
+}
+
+// s = sqrt(max(lambda, 0)) that keeps a NaN eigenvalue NaN, as the reference's np.sqrt(np.clip(lam, 0, None)) does (fmax
+// alone drops the NaN operand and would report sigma = 0 for a non-finite matrix)
+__device__ __forceinline__ double sqrt_clip0(double lam) { return sqrt(isnan(lam) ? lam : fmax(lam, 0.0)); }
+
+// the eigenvalue of a matrix with a NaN or infinite entry (the default quiet NaN, one payload on every route)
+__device__ __forceinline__ double eig_nan() { return __longlong_as_double(0x7ff8000000000000LL); }
+
 }  // namespace lq

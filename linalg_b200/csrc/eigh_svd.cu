@@ -31,11 +31,17 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
     const int tid = threadIdx.x, nt = blockDim.x;
     const int half = ne / 2;
 
+    int bad = 0;
     for (int e = tid; e < ne * ne; e += nt) {
         const int i = e / ne, j = e - i * ne;
-        Am[(size_t)i * ld + j] = (i < n && j < n) ? G[(size_t)i * n + j] : 0.0;
+        const double v = (i < n && j < n) ? G[(size_t)i * n + j] : 0.0;
+        bad |= !isfinite(v);
+        Am[(size_t)i * ld + j] = v;
     }
-    __syncthreads();
+    // A NaN or infinite entry: no rotation test can be evaluated on it (an infinite diagonal makes floor_abs infinite and
+    // stops every rotation, a NaN pair never rotates), so the diagonal left behind would be finite values that are not
+    // eigenvalues.  Every eigenvalue is NaN instead and no sweep runs (V = I, written in full by the replay).
+    const int nonfinite = __syncthreads_or(bad);
     // work on 2^-e G with max|diag| in [1, 2): the rotation test forms app * aqq, which would overflow from max|diag| ~ 2^512.
     // The scaling is exact; lambda is scaled back by 2^e below.
     if (tid == 0) {
@@ -56,7 +62,7 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
     const double floor_abs = 4.9303806576313238e-32 * s_scale;  // eps^2 * max|diag|
 
     int rounds = 0;
-    for (int sweep = 0; sweep < max_sweeps; ++sweep) {
+    for (int sweep = 0; sweep < (nonfinite ? 0 : max_sweeps); ++sweep) {
         if (tid == 0) s_rot = 0;
         __syncthreads();
         for (int rd = 0; rd < ne - 1; ++rd, ++rounds) {
@@ -144,7 +150,7 @@ __global__ void __launch_bounds__(1024) jacobi_kernel(const double* __restrict__
         if (nrot == 0) break;
     }
     if (tid == 0) *nrounds_out = rounds;
-    for (int i = tid; i < n; i += nt) lambda[i] = scalbn(Am[(size_t)i * ld + i], gexp);
+    for (int i = tid; i < n; i += nt) lambda[i] = nonfinite ? eig_nan() : scalbn(Am[(size_t)i * ld + i], gexp);
 }
 
 
@@ -243,11 +249,17 @@ __global__ void __launch_bounds__(512) jacobi1s_kernel(const double* __restrict_
     const int NU = NU_T ? NU_T : ne / 16, nblk = ne / 4;
     const int slot = 4 * wid + g;
 
+    int bad = 0;
     for (int e = tid; e < ne * ne; e += nt) {
         const int j = e / ne, i = e - j * ne;
-        Bm[e] = (i < n && j < n) ? G[(size_t)j * n + i] : 0.0;  // G is symmetric: read it row-wise
+        const double v = (i < n && j < n) ? G[(size_t)j * n + i] : 0.0;  // G is symmetric: read it row-wise
+        bad |= !isfinite(v);
+        Bm[e] = v;
     }
-    __syncthreads();
+    // a NaN or infinite entry: no sweep, the replay gives V = I and eig_rayleigh_kernel writes NaN for every eigenvalue
+    // (nsteps_out[3]); see jacobi_kernel
+    const int nonfinite = __syncthreads_or(bad);
+    if (tid == 0) nsteps_out[3] = nonfinite;
     // B = 2^-e G with max|diag| in [1, 2): the rotation test multiplies four entries (alpha beta, gamma^2), which would
     // overflow from max|diag| ~ 2^256 and underflow below ~ 2^-256.  The scaling is exact; eig_rayleigh_kernel scales
     // lambda back by 2^e (nsteps_out[2]).
@@ -289,7 +301,7 @@ __global__ void __launch_bounds__(512) jacobi1s_kernel(const double* __restrict_
     int step_base = 0;
     const int sps = jacobi1s_steps_per_sweep(ne);
     int rotated = 0;
-    for (int sweep = 0; sweep < max_sweeps; ++sweep, step_base += sps) {
+    for (int sweep = 0; sweep < (nonfinite ? 0 : max_sweeps); ++sweep, step_base += sps) {
         if (tid == 0) s_rot = 0;
         rotated = 0;
         // ---- the pairs inside the blocks
@@ -369,7 +381,7 @@ __global__ void __launch_bounds__(512) jacobi1s_kernel(const double* __restrict_
     if (tid == 0) {
         double mn = 1e300, mx = 0.0;
         for (int i = 0; i < n; ++i) mn = fmin(mn, s_cn[i]), mx = fmax(mx, s_cn[i]);
-        nsteps_out[1] = (allow_direct && mx > 0.0 && mn > 1e-2 * mx) ? 1 : 0;
+        nsteps_out[1] = (allow_direct && !nonfinite && mx > 0.0 && mn > 1e-2 * mx) ? 1 : 0;
     }
 }
 
@@ -440,16 +452,16 @@ __global__ void __launch_bounds__(128) jacobi1s_apply_kernel(const double2* __re
 }
 
 // lambda_i = 2^e v_i^T (2^-e G v_i) = 2^e v_i . b_i   (B = 2^-e G V column-major with pitch ne, e = flags[2]; V row-major
-// n x n, eigenvectors in columns)
+// n x n, eigenvectors in columns); NaN for a non-finite G (flags[3])
 __global__ void __launch_bounds__(256) eig_rayleigh_kernel(const double* __restrict__ B, int ne, const double* __restrict__ V, int n,
                                                            const int* __restrict__ flags, double* __restrict__ lambda) {
     const int wid = threadIdx.x >> 5, ln = threadIdx.x & 31;
-    const int e = flags[2];
+    const int e = flags[2], nonfinite = flags[3];
     for (int i = blockIdx.x * (blockDim.x >> 5) + wid; i < n; i += gridDim.x * (blockDim.x >> 5)) {
         double acc = 0.0;
         for (int j = ln; j < n; j += 32) acc = fma(V[(size_t)j * n + i], B[(size_t)i * ne + j], acc);
         acc = warp_sum(acc);
-        if (ln == 0) lambda[i] = scalbn(acc, e);
+        if (ln == 0) lambda[i] = nonfinite ? eig_nan() : scalbn(acc, e);
     }
 }
 
@@ -480,17 +492,15 @@ __global__ void __launch_bounds__(256) jacobi_apply_kernel(const double2* __rest
 }
 
 // sort eigenvalues descending (rank by counting), permute the columns of V accordingly.  Any number of CTAs: every CTA
-// ranks all eigenvalues itself (n^2 compares) and moves its slice of V (one CTA took 35 us at n = 128).
+// ranks all eigenvalues itself (n^2 compares) and moves its slice of V (one CTA took 35 us at n = 128).  The order is
+// eig_desc_before's (NaN first), so the ranks are a permutation and every slot of lam_out and of V is written for any input.
 __global__ void __launch_bounds__(256) eig_sort_kernel(const double* __restrict__ lam_in, const double* __restrict__ Vin, int n,
                                                        double* __restrict__ lam_out, double* __restrict__ Vout) {
     extern __shared__ int rank_of[];
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         const double li = lam_in[i];
         int rk = 0;
-        for (int j = 0; j < n; ++j) {
-            const double lj = lam_in[j];
-            rk += (lj > li) || (lj == li && j < i);
-        }
+        for (int j = 0; j < n; ++j) rk += eig_desc_before(lam_in[j], j, li, i);
         rank_of[i] = rk;
         if (blockIdx.x == 0) lam_out[rk] = li;
     }
@@ -501,8 +511,9 @@ __global__ void __launch_bounds__(256) eig_sort_kernel(const double* __restrict_
     }
 }
 
-// s = sqrt(max(lambda, 0)); M2 = V diag(1/s for s > tol else 0); Vt = V^T; rank = #(s > tol).  Any number of CTAs (one CTA
-// spent 48 us on 16 384 square roots and divisions at n = 128): the singular values are formed once per CTA in shared memory.
+// s = sqrt(max(lambda, 0)) (NaN stays NaN); M2 = V diag(1/s for s > tol else 0); Vt = V^T; rank = #(s > tol).  Any number
+// of CTAs (one CTA spent 48 us on 16 384 square roots and divisions at n = 128): the singular values are formed once per CTA
+// in shared memory.
 __global__ void __launch_bounds__(256) svd_post_kernel(const double* __restrict__ lam, const double* __restrict__ V, int n,
                                                        double tol, double* __restrict__ s, double* __restrict__ M2,
                                                        double* __restrict__ Vt, int* __restrict__ rank) {
@@ -511,7 +522,7 @@ __global__ void __launch_bounds__(256) svd_post_kernel(const double* __restrict_
     if (threadIdx.x == 0) cnt = 0;
     __syncthreads();
     for (int j = threadIdx.x; j < n; j += blockDim.x) {
-        const double sj = sqrt(fmax(lam[j], 0.0));
+        const double sj = sqrt_clip0(lam[j]);
         sv[j] = sj;
         if (blockIdx.x == 0) {
             s[j] = sj;
